@@ -15,6 +15,7 @@ Run in the build container (where /root/reference exists): `python baseline/inst
 calls it when /root/reference is present.
 """
 import hashlib
+import os
 import shutil
 import subprocess
 import sys
@@ -26,8 +27,17 @@ REF = Path("/root/reference")
 DST = ROOT / "baseline" / "_ref"
 
 
+def reference_readable():
+    """A reference this user may not read counts as absent: on a directory it cannot search, Path.exists() raises
+    PermissionError rather than returning False."""
+    try:
+        return REF.exists() and os.access(REF, os.R_OK | os.X_OK)
+    except PermissionError:
+        return False
+
+
 def main():
-    if not REF.exists():
+    if not reference_readable():
         print("baseline/install_ref.py: /root/reference is not present; keeping whatever baseline/_ref holds")
         return 0
     if DST.exists():

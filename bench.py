@@ -7,6 +7,7 @@ configs[2]: 600 synthetic 1920x1080 frames, frame pairs sharded across the GPUs 
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the UNMODIFIED reference module (baseline/_ref) on the host cores
     python bench.py --workload 4k_eval | train | api256      # the other BASELINE configs, same JSON schema
+    python bench.py --dump-outputs DIR ...    # also writes the last timed step's outputs as DIR/<name>.npy
 
 Default workload (`video1080p`). A step = one forward of `--pairs` consecutive frame pairs (u8 frames resident in HBM
 -> u8 interpolated frames in HBM).
@@ -162,7 +163,7 @@ def cpu_step_fn(threads, bilinear=False):
 
 def run_reference(args):
     """Reference arm: same workload / config keys as the b200 arm, each step = one forward of `--pairs` 1080p frame
-    pairs through the reference module on all host cores; the number of steps is bounded by a wall-clock budget."""
+    pairs through the reference module on all host cores, exactly `--steps` timed steps."""
     if int(os.environ.get("RANK", "0")) != 0:
         return
     if args.workload != "video1080p":
@@ -174,17 +175,14 @@ def run_reference(args):
     fn, kind, what = cpu_step_fn(threads, args.bilinear)
     fr = synthetic_frames(B + 1)
     fn(fr[:2, :, :64, :64])  # thread pool / allocator warm-up on a tiny crop
-    budget_s, times = 240.0, []
+    times = []
     warmup, steps = min(args.warmup, 1), args.steps
-    t_start = time.perf_counter()
     for i in range(warmup + steps):
         t0 = time.perf_counter()
         fn(fr)
         dt = time.perf_counter() - t0
         if i >= warmup:
             times.append(dt)
-        if time.perf_counter() - t_start + dt > budget_s and times:
-            break       # a 4-pair 1080p CPU step takes ~10 s: keep the whole run inside a few minutes
     total = sum(times)
     fps = B * len(times) / total
     line = {
@@ -253,7 +251,8 @@ class Ranks:
 
 
 def timed_steps(R, step, steps, warmup, sampler_index=None):
-    """W untimed steps, then exactly K steps between CUDA events, barrier + synchronize on both sides, max over ranks."""
+    """W untimed steps, then exactly K steps between CUDA events, barrier + synchronize on both sides, max over ranks.
+    Returns (ms, clock samples, what the last timed step returned)."""
     torch = R.torch
     for i in range(warmup):
         step(i)
@@ -264,12 +263,33 @@ def timed_steps(R, step, steps, warmup, sampler_index=None):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     R.barrier()
     ev0.record()
-    for i in range(steps):
+    for i in range(steps - 1):
         step(i)
+    last = step(steps - 1)
     ev1.record()
     R.barrier()
     ms = R.max(ev0.elapsed_time(ev1))
-    return ms, (sampler.stop() if R.rank == 0 else None)
+    return ms, (sampler.stop() if R.rank == 0 else None), last
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array (torch tensor or numpy) as out_dir/<name>.npy, float64 kept, any other dtype as float32. An
+    array larger than its share of DUMP_BYTES is replaced by a fixed seeded sample of its flattened elements, in index
+    order, so that runs with the same arguments write the same elements."""
+    import numpy as np
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 4096                 # room for each .npy header
+    for name, a in arrays.items():
+        a = np.asarray(a.detach().cpu() if hasattr(a, "detach") else a)
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        if a.nbytes > share:
+            keep = np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False)
+            a = a.reshape(-1)[np.sort(keep)]
+        np.save(out_dir / f"{name}.npy", a)
 
 
 def cpu_baseline(pairs_hw, sample_steps, what, bilinear=False):
@@ -316,7 +336,8 @@ def run_video1080p(args):
         return net.forward(frames[s:s + B], frames[s + 1:s + B + 1], want_f32=False, want_u8=True)[1]
 
     flops_step, launches_step = net.cost(B, H, W)
-    ms, clocks = timed_steps(R, step, args.steps, args.warmup)
+    ms, clocks, last = timed_steps(R, step, args.steps, args.warmup)
+    last = last.cpu() if args.dump_outputs and R.rank == 0 else None
     value = R.world * B * args.steps / (ms / 1e3)
 
     # ---- separate profiled pass (per-launch CUDA events perturb the step, so `value` above is timed without them)
@@ -411,6 +432,8 @@ def run_video1080p(args):
                 "whole_step_tflops": flops_step * args.steps / (ms / 1e3) / 1e12}
     if args.profile_out:
         Path(args.profile_out).write_text(json.dumps(prof, indent=1))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"interpolated_u8": last})
 
     cpu = None if args.no_cpu_baseline else cpu_baseline((B, H, W), 1, "of the clip's 599", args.bilinear)
     line = {
@@ -456,10 +479,13 @@ def run_4k_eval(args):
         mid = net.forward(a, b, want_f32=False, want_u8=True)[1]
         q1 = net.forward(a, mid, want_f32=False, want_u8=True)[1]
         q3 = net.forward(mid, b, want_f32=False, want_u8=True)[1]
-        return E.ssim_psnr_u8(torch.cat([q1[:, 0], mid[:, 0], q3[:, 0]]), gt)
+        new = torch.cat([q1[:, 0], mid[:, 0], q3[:, 0]])
+        return new, E.ssim_psnr_u8(new, gt)
 
     flops_fwd, launches_fwd = net.cost(B, h, w)
-    ms, clocks = timed_steps(R, step, args.steps, args.warmup)
+    ms, clocks, last = timed_steps(R, step, args.steps, args.warmup)
+    if args.dump_outputs and R.rank == 0:
+        dump_outputs(args.dump_outputs, {"interpolated_u8": last[0], "psnr_ssim": last[1]})   # frames: q1, mid, q3
     value = R.world * 3 * B * args.steps / (ms / 1e3)
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
     out = torch.cat([gt[:B]] * 3)
@@ -543,7 +569,9 @@ def run_train(args):
     def step(i):
         return step_obj(f0, f1, gt)
 
-    ms, clocks = timed_steps(R, step, args.steps, max(args.warmup, 4))
+    ms, clocks, last = timed_steps(R, step, args.steps, max(args.warmup, 4))
+    if args.dump_outputs and R.rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": last})
     value = R.world * batch * args.steps / (ms / 1e3)
     # end to end: the batch comes from pinned host memory every step and the loss is read back every step
     dbuf = torch.empty_like(host0, device=dev)
@@ -600,19 +628,21 @@ def run_api256(args):
     def step(i):
         return net.forward(d[:1], d[1:], want_f32=False, want_u8=True)[1]
 
-    ms, clocks = timed_steps(R, step, args.steps * 10, args.warmup)
-    per_call = ms / (args.steps * 10)
+    ms, clocks, last = timed_steps(R, step, args.steps, args.warmup)
+    if args.dump_outputs and R.rank == 0:
+        dump_outputs(args.dump_outputs, {"interpolated_u8": last})
+    per_call = ms / args.steps
     net.interpolate_host_u8(fr[:1], fr[1:])
     t0 = time.perf_counter()
-    for _ in range(args.steps * 10):
+    for _ in range(args.steps):
         net.interpolate_host_u8(fr[:1], fr[1:])
-    wall = (time.perf_counter() - t0) / (args.steps * 10)
+    wall = (time.perf_counter() - t0) / args.steps
     flops, launches = net.cost(1, 256, 256)
     if R.rank == 0:
         pk, pk_src = peaks()
         tfl = flops / (per_call / 1e3) / 1e12
         print(json.dumps({"metric": "interpolated frames/sec, one 256x256 pair per call", "value": R.world * 1e3 / per_call,
-                          "unit": "frames/s", "n_gpus": R.world, "steps": args.steps * 10, "warmup": args.warmup,
+                          "unit": "frames/s", "n_gpus": R.world, "steps": args.steps, "warmup": args.warmup,
                           "ms_per_step": per_call, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                           "dtype": "bf16", "data": "synthetic",
                           "config": {"workload": "API operating point: UNet(2,1,bilinear=True) forward, 1 pair 256x256 per call",
@@ -621,7 +651,7 @@ def run_api256(args):
                           "e2e": {"value": R.world / wall, "unit": "frames/s", "h2d_bytes_per_step": 2 * 65536,
                                   "d2h_bytes_per_step": 65536, "ms_per_call": wall * 1e3,
                                   "api": "fiNetInterpolateHostU8 (synchronous host u8 pair -> host u8 frame)"},
-                          "gpu_launches": launches * args.steps * 10,
+                          "gpu_launches": launches * args.steps,
                           "roofline": {"bound": "tensor", "achieved": tfl, "peak": pk["bf16_tflops"], "unit": "TFLOP/s",
                                        "frac": tfl / pk["bf16_tflops"], "traffic": None, "kernel": "whole forward",
                                        "peak_source": pk_src},
@@ -632,7 +662,7 @@ def run_api256(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps (api256: one 256x256 call per step)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="video1080p", choices=["video1080p", "4k_eval", "train", "api256"])
@@ -642,7 +672,14 @@ def main():
                     help="bf16 (headline) or the hi/lo-split fp32-grade path (3x the tensor work)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-out", default=None, help="write the per-launch table (JSON) here")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step returned (rank 0's shard) as DIR/<name>.npy, float32 or "
+                         "float64, at most 64 MB in all (a fixed seeded sample of a larger output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the b200 arm only")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)

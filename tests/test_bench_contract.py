@@ -32,6 +32,69 @@ def test_reference_arm_prints_one_json_line_on_the_b200_arms_config():
         assert d["cpu_baseline"]["kind"] == "reference"
 
 
+def test_dump_outputs_writes_float_arrays_within_64_mb(tmp_path):
+    import numpy as np
+    import torch
+    sys.path.insert(0, str(ROOT))
+    import bench
+    ramp = np.arange(16_000_000, dtype=np.int32)          # 64 MB as float32: more than its half of the budget
+    frame = torch.arange(256, dtype=torch.uint8).view(1, 1, 16, 16)
+    metrics = torch.rand(6, 2, dtype=torch.float64)
+    for d in ("a", "b"):
+        bench.dump_outputs(tmp_path / d, {"ramp": ramp, "frame": frame, "metrics": metrics})
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 64_000_000
+    a = np.load(tmp_path / "a" / "ramp.npy")
+    assert a.dtype == np.float32 and a.ndim == 1 and 0 < a.size < ramp.size
+    assert np.all(np.diff(a) > 0) and a[-1] < ramp.size                  # distinct elements, in index order
+    assert np.array_equal(a, np.load(tmp_path / "b" / "ramp.npy"))       # the same sample every run
+    f = np.load(tmp_path / "a" / "frame.npy")
+    assert f.dtype == np.float32 and np.array_equal(f, frame.numpy())
+    m = np.load(tmp_path / "a" / "metrics.npy")
+    assert m.dtype == np.float64 and np.array_equal(m, metrics.numpy())
+
+
+def test_timed_steps_runs_exactly_k_steps_and_returns_the_last():
+    import types
+    sys.path.insert(0, str(ROOT))
+    import bench
+
+    class Event:
+        def __init__(self, enable_timing=False):
+            pass
+
+        def record(self):
+            pass
+
+        def elapsed_time(self, other):
+            return 12.5
+
+    class OneRank:              # not rank 0, so no clock sampler is started
+        rank, local = 1, 0
+        torch = types.SimpleNamespace(cuda=types.SimpleNamespace(Event=Event))
+
+        def barrier(self):
+            pass
+
+        def max(self, v):
+            return v
+
+    calls = []
+
+    def step(i):
+        calls.append(i)
+        return len(calls)
+
+    ms, clocks, last = bench.timed_steps(OneRank(), step, 5, 3)
+    assert calls == [0, 1, 2, 0, 1, 2, 3, 4]
+    assert (ms, clocks, last) == (12.5, None, 8)
+
+
+def test_steps_below_one_are_rejected():
+    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=120)
+    assert r.returncode == 2 and "--steps" in r.stderr
+
+
 def test_other_workloads_of_the_reference_arm_say_unavailable():
     r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--workload", "train"],
                        capture_output=True, text=True, timeout=120)
