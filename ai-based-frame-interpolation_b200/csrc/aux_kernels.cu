@@ -1,5 +1,6 @@
 // CUDA-core kernels of the frame-synthesis path (the stem convolution lives in stem_mma.cu): the bilinear
-// decoder upsample, frame-pair packing, output post-processing and the fused SSIM+PSNR metric kernel.
+// decoder upsample, frame-pair packing, output post-processing, the fused SSIM+PSNR metric kernel and the
+// frame-pair SAD of scene-cut detection.
 #include "aux_kernels.cuh"
 #include "ptx.cuh"
 
@@ -383,6 +384,67 @@ ssim_psnr_finalize_kernel(const double* __restrict__ part_ssim, const unsigned l
     }
 }
 
+// ------------------------------------------------------------------------------------------------ pair SAD
+// sad[p] = sum_k |f[p+1][k] - f[p][k]| over all frame_bytes bytes of every consecutive frame pair (scene-cut statistic).
+// blockIdx.y = group of PS_GROUP consecutive pairs; a thread walks its 16-byte chunks through the group's frames with
+// the previous frame's chunk in registers, so each frame is read once per group (group edges twice: +1/PS_GROUP).
+// Per-pair sums stay in 32-bit registers (a chunk adds at most 16*255; the launcher keeps <= 2^20 chunks per thread)
+// and are reduced in 64 bit: one integer atomic per block and pair, exact and independent of the launch shape.
+constexpr int PS_THREADS = 256;
+constexpr int PS_GROUP = 8;
+
+__global__ void __launch_bounds__(PS_THREADS)
+pair_sad_kernel(const uint8_t* __restrict__ frames, long long frame_stride, long long frame_bytes, int n_pairs, int vec,
+                unsigned long long* __restrict__ sad) {
+    const int p0 = blockIdx.y * PS_GROUP;
+    const int cnt = min(PS_GROUP, n_pairs - p0);
+    const uint8_t* base = frames + p0 * frame_stride;
+    uint32_t acc[PS_GROUP];
+#pragma unroll
+    for (int k = 0; k < PS_GROUP; ++k) acc[k] = 0;
+    const long long tid = static_cast<long long>(blockIdx.x) * PS_THREADS + threadIdx.x;
+    const long long nthr = static_cast<long long>(gridDim.x) * PS_THREADS;
+    const long long n16 = vec ? frame_bytes / 16 : 0;
+    for (long long c = tid; c < n16; c += nthr) {
+        uint4 prev = __ldg(reinterpret_cast<const uint4*>(base) + c);
+#pragma unroll
+        for (int k = 0; k < PS_GROUP; ++k) {
+            // past the group's last frame the same chunk is loaded again (an L1 hit) and adds 0: no predicated loads
+            const int f = k + 1 < cnt ? k + 1 : cnt;
+            const uint4 cur = __ldg(reinterpret_cast<const uint4*>(base + f * frame_stride) + c);
+            acc[k] += __vsadu4(prev.x, cur.x) + __vsadu4(prev.y, cur.y) + __vsadu4(prev.z, cur.z) +
+                      __vsadu4(prev.w, cur.w);
+            prev = cur;
+        }
+    }
+    // bytes not covered by 16-byte chunks: the tail of an aligned frame, or every byte of an unaligned one
+    for (long long i = n16 * 16 + tid; i < frame_bytes; i += nthr) {
+        int prev = __ldg(base + i);
+#pragma unroll
+        for (int k = 0; k < PS_GROUP; ++k) {
+            const int f = k + 1 < cnt ? k + 1 : cnt;
+            const int cur = __ldg(base + f * frame_stride + i);
+            acc[k] += static_cast<uint32_t>(abs(cur - prev));
+            prev = cur;
+        }
+    }
+    __shared__ unsigned long long part[PS_THREADS / 32][PS_GROUP];
+#pragma unroll
+    for (int k = 0; k < PS_GROUP; ++k) {
+        unsigned long long v = acc[k];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+        if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5][k] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x < cnt) {
+        unsigned long long s = 0;
+#pragma unroll
+        for (int w = 0; w < PS_THREADS / 32; ++w) s += part[w][threadIdx.x];
+        if (s) atomicAdd(sad + p0 + threadIdx.x, s);
+    }
+}
+
 int grid_for(size_t work_items, int threads) {
     size_t g = (work_items + threads - 1) / threads;
     const size_t cap = 148 * 16;  // grid-stride loops: a few waves of the 148 SMs is enough
@@ -466,6 +528,31 @@ const char* ssim_psnr_launch(const uint8_t* a, const uint8_t* b, int N, int H, i
     const char* e = last_launch_error();
     if (e) return e;
     ssim_psnr_finalize_kernel<<<N, 256, 0, stream>>>(part_ssim, part_ssd, nblk, H, W, out);
+    return last_launch_error();
+}
+
+const char* pair_sad_launch(const uint8_t* frames, int64_t frame_stride, int64_t frame_bytes, int n_frames,
+                            uint64_t* sad, cudaStream_t stream) {
+    if (!frames || !sad) return "pair_sad: null operand";
+    if (n_frames < 2 || frame_bytes < 1 || frame_stride < frame_bytes)
+        return "pair_sad: needs >= 2 frames of >= 1 byte, frame_stride >= frame_bytes";
+    const int n_pairs = n_frames - 1;
+    const int gy = (n_pairs + PS_GROUP - 1) / PS_GROUP;
+    if (gy > 65535) return "pair_sad: at most 524280 pairs per call";
+    const int vec = (reinterpret_cast<uintptr_t>(frames) % 16 == 0) && (frame_stride % 16 == 0);
+    const long long units = vec ? frame_bytes / 16 : frame_bytes;
+    long long gx = (units + PS_THREADS - 1) / PS_THREADS;
+    const long long fill = (148 * 8 + gy - 1) / gy;  // about one wave of 8 blocks per SM over all groups
+    if (gx > fill) gx = fill;
+    // 32-bit per-thread sums: at most 2^20 units (16*255 each) per thread, plus < 16 tail bytes of 255
+    const long long min_gx = (units + (static_cast<long long>(PS_THREADS) << 20) - 1) / (static_cast<long long>(PS_THREADS) << 20);
+    if (gx < min_gx) gx = min_gx;
+    if (gx < 1) gx = 1;
+    if (gx > 0x7fffffffLL) return "pair_sad: frame too large";
+    const cudaError_t e = cudaMemsetAsync(sad, 0, static_cast<size_t>(n_pairs) * sizeof(uint64_t), stream);
+    if (e != cudaSuccess) return cudaGetErrorString(e);
+    pair_sad_kernel<<<dim3(static_cast<unsigned>(gx), gy), PS_THREADS, 0, stream>>>(
+        frames, frame_stride, frame_bytes, n_pairs, vec, reinterpret_cast<unsigned long long*>(sad));
     return last_launch_error();
 }
 

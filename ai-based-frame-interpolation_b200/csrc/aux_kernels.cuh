@@ -47,4 +47,9 @@ size_t ssim_psnr_workspace_bytes(int N, int H, int W);
 const char* ssim_psnr_launch(const uint8_t* a, const uint8_t* b, int N, int H, int W, double* out /*[N][2]*/,
                              void* workspace, cudaStream_t stream);
 
+// Scene-cut statistic: sad[p] = sum |f[p+1] - f[p]| over the frame_bytes bytes of each of the n_frames-1 consecutive
+// pairs of u8 frames frame_stride bytes apart (exact; zeroes sad on `stream` first).
+const char* pair_sad_launch(const uint8_t* frames, int64_t frame_stride, int64_t frame_bytes, int n_frames,
+                            uint64_t* sad, cudaStream_t stream);
+
 }  // namespace fi

@@ -156,8 +156,11 @@ struct fiNet {
         void* dev_in = nullptr;
         void* dev_out = nullptr;
         cudaEvent_t in_ready = nullptr, done = nullptr, out_ready = nullptr;
+        uint64_t* pin_sad = nullptr;  // per-pair SAD of the batch (fiNetInterpolateClipHostU8Sad only)
+        uint64_t* dev_sad = nullptr;
     } clip[2];
     size_t clip_in_bytes = 0, clip_out_bytes = 0;
+    int clip_sad_pairs = 0;  // capacity of pin_sad / dev_sad
     cudaStream_t clip_h2d = nullptr, clip_d2h = nullptr;
     // pinned staging for the host-buffer convenience call
     void* pin_in = nullptr;
@@ -746,6 +749,8 @@ int fiNetDestroy(fiNet* net) {
         if (c.pin_out) cudaFreeHost(c.pin_out);
         if (c.dev_in) cudaFree(c.dev_in);
         if (c.dev_out) cudaFree(c.dev_out);
+        if (c.pin_sad) cudaFreeHost(c.pin_sad);
+        if (c.dev_sad) cudaFree(c.dev_sad);
         if (c.in_ready) cudaEventDestroy(c.in_ready);
         if (c.done) cudaEventDestroy(c.done);
         if (c.out_ready) cudaEventDestroy(c.out_ready);
@@ -1006,6 +1011,13 @@ int fiNetInterpolateClipHostU8(fiNet* net, const uint8_t* frames_host, int n_fra
 int fiNetInterpolateClipHostU8Strided(fiNet* net, const uint8_t* frames_host, int64_t frame_stride, int n_frames,
                                       int channels_per_frame, uint8_t* out_host, int64_t out_stride, int H, int W,
                                       int pairs_per_batch, void* stream) {
+    return fiNetInterpolateClipHostU8Sad(net, frames_host, frame_stride, n_frames, channels_per_frame, out_host,
+                                         out_stride, H, W, pairs_per_batch, stream, nullptr);
+}
+
+int fiNetInterpolateClipHostU8Sad(fiNet* net, const uint8_t* frames_host, int64_t frame_stride, int n_frames,
+                                  int channels_per_frame, uint8_t* out_host, int64_t out_stride, int H, int W,
+                                  int pairs_per_batch, void* stream, uint64_t* pair_sad_host) {
     if (!net || !frames_host || !out_host) return fail(FI_ERR_INVALID, "null argument");
     if (2 * channels_per_frame != net->n_channels)
         return fail(FI_ERR_INVALID, "2 x %d channels per frame != n_channels %d", channels_per_frame, net->n_channels);
@@ -1047,6 +1059,20 @@ int fiNetInterpolateClipHostU8Strided(fiNet* net, const uint8_t* frames_host, in
         net->clip_in_bytes = in_bytes;
         net->clip_out_bytes = out_bytes;
     }
+    if (pair_sad_host && net->clip_sad_pairs < B) {
+        CUDA_TRY(cudaDeviceSynchronize());
+        for (auto& c : net->clip) {
+            if (c.pin_sad) cudaFreeHost(c.pin_sad);
+            if (c.dev_sad) cudaFree(c.dev_sad);
+            c.pin_sad = c.dev_sad = nullptr;
+        }
+        net->clip_sad_pairs = 0;
+        for (auto& c : net->clip) {
+            CUDA_TRY(cudaMallocHost(reinterpret_cast<void**>(&c.pin_sad), B * sizeof(uint64_t)));
+            CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&c.dev_sad), B * sizeof(uint64_t)));
+        }
+        net->clip_sad_pairs = B;
+    }
     const int n_pairs = n_frames - 1;
     const int n_batches = (n_pairs + B - 1) / B;
     auto collect = [&](int b) -> int {  // wait for batch b's D2H and hand its frames to the caller
@@ -1061,6 +1087,7 @@ int fiNetInterpolateClipHostU8Strided(fiNet* net, const uint8_t* frames_host, in
                 memcpy(out_host + static_cast<int64_t>(first + i) * out_stride,
                        static_cast<const char*>(c.pin_out) + i * outf_bytes, outf_bytes);
         }
+        if (pair_sad_host) memcpy(pair_sad_host + first, c.pin_sad, cnt * sizeof(uint64_t));
         return FI_OK;
     };
     for (int b = 0; b < n_batches; ++b) {
@@ -1078,6 +1105,9 @@ int fiNetInterpolateClipHostU8Strided(fiNet* net, const uint8_t* frames_host, in
         CUDA_TRY(cudaMemcpyAsync(c.dev_in, c.pin_in, (cnt + 1) * frame_bytes, cudaMemcpyHostToDevice, net->clip_h2d));
         CUDA_TRY(cudaEventRecord(c.in_ready, net->clip_h2d));
         CUDA_TRY(cudaStreamWaitEvent(st, c.in_ready, 0));
+        if (pair_sad_host)  // the batch's cnt+1 frames were just uploaded: the SAD reads them from L2, not the host
+            KERNEL_TRY(fi::pair_sad_launch(static_cast<const uint8_t*>(c.dev_in), static_cast<int64_t>(frame_bytes),
+                                           static_cast<int64_t>(frame_bytes), cnt + 1, c.dev_sad, st));
         fiPlanes p0, p1;
         p0.ptr = c.dev_in;
         p0.channels = channels_per_frame;
@@ -1092,6 +1122,8 @@ int fiNetInterpolateClipHostU8Strided(fiNet* net, const uint8_t* frames_host, in
         CUDA_TRY(cudaEventRecord(c.done, st));
         CUDA_TRY(cudaStreamWaitEvent(net->clip_d2h, c.done, 0));
         CUDA_TRY(cudaMemcpyAsync(c.pin_out, c.dev_out, cnt * outf_bytes, cudaMemcpyDeviceToHost, net->clip_d2h));
+        if (pair_sad_host)
+            CUDA_TRY(cudaMemcpyAsync(c.pin_sad, c.dev_sad, cnt * sizeof(uint64_t), cudaMemcpyDeviceToHost, net->clip_d2h));
         CUDA_TRY(cudaEventRecord(c.out_ready, net->clip_d2h));
         if (b > 0 && (rc = collect(b - 1))) return rc;
     }
@@ -1289,6 +1321,16 @@ int fiSsimPsnrU8(const uint8_t* pred, const uint8_t* target, int N, int H, int W
                  void* stream) {
     const char* e = fi::ssim_psnr_launch(pred, target, N, H, W, out, workspace, static_cast<cudaStream_t>(stream));
     if (e) return fail(FI_ERR_INVALID, "%s", e);
+    return FI_OK;
+}
+
+int fiPairSadU8(const uint8_t* frames, int64_t frame_stride, int64_t frame_bytes, int n_frames, uint64_t* sad,
+                void* stream) {
+    if (!frames || !sad) return fail(FI_ERR_INVALID, "null argument");
+    if (n_frames < 2 || frame_bytes < 1 || frame_stride < frame_bytes)
+        return fail(FI_ERR_INVALID, "needs >= 2 frames of >= 1 byte and frame_stride >= frame_bytes");
+    const char* e = fi::pair_sad_launch(frames, frame_stride, frame_bytes, n_frames, sad, static_cast<cudaStream_t>(stream));
+    if (e) return fail(FI_ERR_CUDA, "%s", e);
     return FI_OK;
 }
 

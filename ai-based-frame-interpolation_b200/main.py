@@ -9,10 +9,18 @@ import sys
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 
+def _scene_threshold(text):
+    from model.scene import check_threshold
+    try:
+        return check_threshold(text)
+    except ValueError as e:
+        raise argparse.ArgumentTypeError(str(e)) from None
+
+
 def build_parser():
     p = argparse.ArgumentParser(description="AI-Based Frame Interpolation (B200-native path)")
     sub = p.add_subparsers(dest="command", help="Available commands")
-    # flags, defaults and required-ness as reference main.py:40-72; --gpus is the only addition
+    # flags, defaults and required-ness as reference main.py:40-72; --gpus and --scene-threshold are the only additions
     t = sub.add_parser("train", help="Train the frame interpolation model")
     t.add_argument("--data-dir", required=True, help="Directory containing training data")
     t.add_argument("--epochs", type=int, default=100, help="Number of training epochs")
@@ -33,6 +41,9 @@ def build_parser():
     v.add_argument("--device", default="auto", help="Device to use (cuda/auto)")
     v.add_argument("--gpus", type=int, default=None,
                    help="Shard the frame pairs over this many GPUs of the box (default: $FI_GPUS, else 1)")
+    v.add_argument("--scene-threshold", type=_scene_threshold, default=None, metavar="T",
+                   help="Detect scene cuts (score in (0, 100], try 10) and repeat the frame before a cut instead of "
+                        "blending two shots (default: off)")
     s = sub.add_parser("serve", help="Start the web API server")
     s.add_argument("--host", default="0.0.0.0", help="Host to bind to")
     s.add_argument("--port", type=int, default=8000, help="Port to bind to")
@@ -76,10 +87,12 @@ def main(argv=None):
             print(f"Interpolated frame saved to: {args.output}")
         elif args.command == "video":
             from model.inference import FrameInterpolator
-            interpolator = FrameInterpolator(args.model, device, gpus=args.gpus)
+            interpolator = FrameInterpolator(args.model, device, gpus=args.gpus, scene_threshold=args.scene_threshold)
             print(f"Interpolating video: {args.input}\nOutput: {args.output}\nFactor: {args.factor}x")
             n = interpolator.interpolate_video(args.input, args.output, args.factor)
             print(f"Video interpolation completed! ({n} frames written)")
+            if args.scene_threshold is not None:
+                print(f"Scene cuts found: {len(interpolator.last_scene_cuts)} (threshold {args.scene_threshold:g})")
         elif args.command == "serve":
             import uvicorn
             print(f"Starting API server on {args.host}:{args.port}")

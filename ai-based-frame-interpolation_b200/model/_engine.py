@@ -64,6 +64,8 @@ _SIGNATURES = {
                                              C.c_int, C.c_void_p]),
     "fiNetInterpolateClipHostU8Strided": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p,
                                                     C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "fiNetInterpolateClipHostU8Sad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p,
+                                                C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "fiNetForwardCost": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_int)]),
     "fiNetPlanStats": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_longlong), C.POINTER(C.c_size_t)]),
     "fiNetReadActivation": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int),
@@ -82,6 +84,7 @@ _SIGNATURES = {
     "fiSsimPsnrWorkspaceBytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "fiSsimPsnrU8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                C.c_void_p]),
+    "fiPairSadU8": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_void_p]),
     # training-step kernels
     "fiBnStats": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "fiBnApplyRelu": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -233,11 +236,13 @@ class Net:
                                                current_stream()))
         return out
 
-    def interpolate_clip_host_u8(self, frames, pairs_per_batch=4, out=None):
+    def interpolate_clip_host_u8(self, frames, pairs_per_batch=4, out=None, sad_out=None):
         """numpy uint8 [F,C,H,W] host clip in, numpy uint8 [F-1,n_classes,H,W] midpoints out; copies and compute are
         pipelined inside the library. `out`: optional preallocated result array (e.g. this GPU's slice of a clip-wide
         buffer when the pairs are sharded across GPUs). Both arrays may be strided along the frame axis (every frame
-        itself contiguous), e.g. `seq[0::2]` in and `seq[1::2]` out of one interleaved sequence."""
+        itself contiguous), e.g. `seq[0::2]` in and `seq[1::2]` out of one interleaved sequence. `sad_out`: optional
+        contiguous uint64 [F-1] array that receives the scene-cut statistic of every pair, sum |f[i+1] - f[i]| over
+        all C*H*W bytes, computed on the GPU from the uploaded frames (fiNetInterpolateClipHostU8Sad)."""
         import numpy as np
         frames = np.asarray(frames)
         if frames.dtype != np.uint8 or frames.ndim != 4:
@@ -257,10 +262,14 @@ class Net:
               or (f > 1 and not frame_contiguous(out))):
             raise FiError(f"out must be a writable uint8 array of shape {(f - 1, self.n_classes, h, w)} whose frames "
                           "are contiguous")
+        if sad_out is not None and (sad_out.dtype != np.uint64 or sad_out.shape != (f - 1,) or not sad_out.flags.writeable
+                                    or not sad_out.flags.c_contiguous):
+            raise FiError(f"sad_out must be a writable contiguous uint64 array of shape {(f - 1,)}")
         with torch.cuda.device(self.device):
-            check(lib().fiNetInterpolateClipHostU8Strided(self._h, frames.ctypes.data, frames.strides[0], f, c,
-                                                          out.ctypes.data, out.strides[0] if f > 1 else 0, h, w,
-                                                          pairs_per_batch, current_stream()))
+            check(lib().fiNetInterpolateClipHostU8Sad(self._h, frames.ctypes.data, frames.strides[0], f, c,
+                                                      out.ctypes.data, out.strides[0] if f > 1 else 0, h, w,
+                                                      pairs_per_batch, current_stream(),
+                                                      sad_out.ctypes.data if sad_out is not None else None))
         return out
 
     def set_profiling(self, on):
@@ -309,6 +318,22 @@ def ssim_psnr_u8(pred: torch.Tensor, target: torch.Tensor) -> torch.Tensor:
     with torch.cuda.device(pred.device):
         check(lib().fiSsimPsnrU8(pred.data_ptr(), target.data_ptr(), n, h, w, out.data_ptr(), ws.data_ptr(),
                                  current_stream()))
+    return out
+
+
+def pair_sad_u8(frames: torch.Tensor) -> torch.Tensor:
+    """frames: uint8 CUDA tensor [F, ...], each frame contiguous, any stride along dim 0. Returns int64 CUDA tensor
+    [F-1]: sum |frames[i+1] - frames[i]| over every byte of the frame (fiPairSadU8; uint64 in the library, and every
+    value fits int64)."""
+    require_cuda(frames.device)
+    if frames.dtype != torch.uint8 or frames.dim() < 2 or frames.shape[0] < 2:
+        raise FiError("frames must be a uint8 tensor [F, ...] with at least two frames")
+    if not frames[0].is_contiguous():
+        frames = frames.contiguous()
+    out = torch.empty(frames.shape[0] - 1, dtype=torch.int64, device=frames.device)
+    with torch.cuda.device(frames.device):
+        check(lib().fiPairSadU8(frames.data_ptr(), frames.stride(0), frames[0].numel(), frames.shape[0], out.data_ptr(),
+                                current_stream()))
     return out
 
 

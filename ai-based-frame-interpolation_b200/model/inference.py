@@ -17,10 +17,12 @@ import torch
 try:
     from . import _engine as _E
     from .multigpu import GpuPool
+    from .scene import check_threshold, scene_cuts, scene_scores
     from .unet import FrameInterpolationUNet, UNet
 except ImportError:  # `python model/inference.py` / model/ on sys.path, like the reference's scripts
     import _engine as _E
     from multigpu import GpuPool
+    from scene import check_threshold, scene_cuts, scene_scores
     from unet import FrameInterpolationUNet, UNet
 
 
@@ -147,9 +149,17 @@ class FrameInterpolator:
     and postprocess_image are fused into the first and last kernels.
     """
 
-    def __init__(self, model_path, device="cuda", pairs_per_batch=4, gpus=None):
+    def __init__(self, model_path, device="cuda", pairs_per_batch=4, gpus=None, scene_threshold=None):
         """gpus: number of GPUs (device indices device.index .. +gpus-1) or an explicit list of device indices that
-        `interpolate_sequence` / `interpolate_video` shard the frame pairs over (default: $FI_GPUS, else 1)."""
+        `interpolate_sequence` / `interpolate_video` shard the frame pairs over (default: $FI_GPUS, else 1).
+
+        scene_threshold: None (default) interpolates every pair. A value in (0, 100] turns on scene-cut detection in
+        `interpolate_clip`, `interpolate_sequence` and `interpolate_video` (rule: model/scene.py; 10 is a good start):
+        every new frame of a pair detected as a cut is a copy of the pair's first frame instead of a ghosted blend of
+        two shots, and `last_scene_cuts` lists the cut pairs of the last call. `interpolate_frames` (one pair, no
+        neighbours to compare with) ignores it."""
+        self.scene_threshold = None if scene_threshold is None else check_threshold(scene_threshold)
+        self.last_scene_cuts = None
         self.device = _resolve_device(device)
         state, _ = _read_checkpoint(model_path, self.device)
         keys = list(state.keys())
@@ -215,7 +225,8 @@ class FrameInterpolator:
         return [o[..., 0] if grey_in and o.shape[-1] == 1 else o for o in out]
 
     def interpolate_frames(self, frame1, frame2):
-        """Midpoint frame of one pair; same dtype/shape family as the inputs (BGR in -> BGR out)."""
+        """Midpoint frame of one pair; same dtype/shape family as the inputs (BGR in -> BGR out). `scene_threshold`
+        does not apply: a single pair always gets the network's midpoint."""
         frame1, frame2 = np.asarray(frame1), np.asarray(frame2)
         if frame1.shape != frame2.shape or frame1.dtype != np.uint8:
             raise ValueError("frames must be uint8 arrays of identical shape")
@@ -227,18 +238,30 @@ class FrameInterpolator:
             out += self._forward_pairs(firsts[i:i + self.pairs_per_batch], seconds[i:i + self.pairs_per_batch])
         return out
 
-    def _clip_call(self, frames, out):
+    def _clip_call(self, frames, out, sad=None):
         """[F,C,H,W] u8 host clip -> out [F-1,n_classes,H,W]: one GPU = the library's pipelined clip call (pinned
-        double-buffered staging, copies overlapped with compute); several GPUs = contiguous pair ranges, one per GPU."""
+        double-buffered staging, copies overlapped with compute); several GPUs = contiguous pair ranges, one per GPU.
+        sad: optional uint64 [F-1] that receives each pair's sum of absolute differences, computed on the GPU."""
         if self._single_device:
-            return self.model._engine(self.device).interpolate_clip_host_u8(frames, self.pairs_per_batch, out=out)
-        return self._gpu_pool().clip_midpoints(frames, self.pairs_per_batch, out)
+            return self.model._engine(self.device).interpolate_clip_host_u8(frames, self.pairs_per_batch, out=out,
+                                                                            sad_out=sad)
+        return self._gpu_pool().clip_midpoints(frames, self.pairs_per_batch, out, sad_out=sad)
 
     def interpolate_clip(self, frames, out=None):
         """Midpoint of every consecutive pair of a clip held in ONE uint8 array: [F,H,W] grey or [F,H,W,3] BGR ->
         [F-1,H,W] / [F-1,H,W,3]. `out` may be a preallocated result array (re-used across calls by the video loop and by
         bench.py; a fresh 1 GB result array costs page faults comparable to the GPU time of a short clip). Grey clips
-        and their `out` may be strided along the frame axis (`seq[0::2]` -> `seq[1::2]`)."""
+        and their `out` may be strided along the frame axis (`seq[0::2]` -> `seq[1::2]`). With `scene_threshold` set,
+        the result of a cut pair i is a copy of frames[i] and `last_scene_cuts` lists those i."""
+        out, cuts, _ = self._clip(frames, out, 0.0)
+        if cuts is not None:
+            self.last_scene_cuts = cuts
+        return out
+
+    def _clip(self, frames, out, prev_mafd):
+        """interpolate_clip. prev_mafd: mafd of the pair before the clip's first pair (0.0 at the start of a clip or
+        video), or None to skip scene detection. Returns (out, cut pair indices or None, mafd of the clip's last pair)."""
+        detect = self.scene_threshold is not None and prev_mafd is not None
         arr = np.asarray(frames)
         if arr.dtype != np.uint8 or arr.ndim not in (3, 4) or arr.shape[0] < 2:
             raise ValueError("expected a uint8 clip [F,H,W] or [F,H,W,C] with at least two frames")
@@ -246,38 +269,49 @@ class FrameInterpolator:
             out = np.empty((arr.shape[0] - 1,) + arr.shape[1:], dtype=np.uint8)
         elif out.shape != (arr.shape[0] - 1,) + arr.shape[1:] or out.dtype != np.uint8:
             raise ValueError("out must be a uint8 array with one frame less than the clip")
+        sad = np.zeros(arr.shape[0] - 1, dtype=np.uint64) if detect else None
         if arr.ndim == 3:                                   # grey frames: may be strided along the frame axis
             if self.n_channels != 2:
                 raise _E.FiError(f"model expects {self.n_channels} input channels, frames are grey")
-            self._clip_call(arr[:, None], out[:, None])
-            return out
-        c = arr.shape[3]
-        if self.n_channels == 2:                            # grey model: every colour plane is its own clip
+            self._clip_call(arr[:, None], out[:, None], sad)
+        elif self.n_channels == 2:                          # grey model: every colour plane is its own clip
             plane = np.empty(out.shape[:3], dtype=np.uint8)
-            for k in range(c):
-                self._clip_call(np.ascontiguousarray(arr[..., k])[:, None], plane[:, None])
+            plane_sad = np.empty_like(sad) if detect else None
+            for k in range(arr.shape[3]):
+                self._clip_call(np.ascontiguousarray(arr[..., k])[:, None], plane[:, None], plane_sad)
                 out[..., k] = plane
-            return out
-        if self.n_channels == 2 * c:                        # colour model: planar frames
-            mids = np.empty((out.shape[0], c) + out.shape[1:3], dtype=np.uint8)
-            self._clip_call(np.ascontiguousarray(arr.transpose(0, 3, 1, 2)), mids)
+                if detect:
+                    sad += plane_sad                        # the SAD of a BGR pair is that of its three planes
+        elif self.n_channels == 2 * arr.shape[3]:           # colour model: planar frames
+            mids = np.empty((out.shape[0], arr.shape[3]) + out.shape[1:3], dtype=np.uint8)
+            self._clip_call(np.ascontiguousarray(arr.transpose(0, 3, 1, 2)), mids, sad)
             out[...] = mids.transpose(0, 2, 3, 1)
-            return out
-        raise _E.FiError(f"model expects {self.n_channels} input channels, frames have {c} per frame")
-
-    def _sequence_midpoints(self, seq):
-        """Midpoint of every consecutive pair of a frame list / array: the video loop's inner step."""
-        arr = seq if isinstance(seq, np.ndarray) else np.stack(seq)
-        return list(self.interpolate_clip(arr))
+        else:
+            raise _E.FiError(f"model expects {self.n_channels} input channels, frames have {arr.shape[3]} per frame")
+        if not detect:
+            return out, None, prev_mafd
+        scores, last_mafd = scene_scores(sad, arr[0].size, prev_mafd)
+        cuts = scene_cuts(scores, self.scene_threshold)
+        for i in cuts:
+            out[i] = arr[i]
+        return out, cuts, last_mafd
 
     def interpolate_sequence(self, frames, factor=2, out=None):
         """factor-1 new frames between every consecutive pair. factor = 2^k: recursive bisection (every new frame is
         a real forward of its two neighbours); any other factor repeats the midpoint, which is what the reference's
         only precedent does (model/inference.py:141-145). `out` (factor 2^k only): a caller-owned uint8 array
         [(F-1)*factor+1, ...frame shape] that receives the whole sequence — a video loop re-uses a few of them instead of
-        faulting in gigabytes of fresh pages per chunk (a 4K chunk is ~5 GB)."""
+        faulting in gigabytes of fresh pages per chunk (a 4K chunk is ~5 GB). With `scene_threshold` set, all factor-1
+        new frames of a cut pair are copies of its first frame and `last_scene_cuts` lists the cut pairs."""
+        seq, cuts, _ = self._sequence(frames, factor, out, 0.0)
+        if cuts is not None:
+            self.last_scene_cuts = cuts
+        return seq
+
+    def _sequence(self, frames, factor, out, prev_mafd):
+        """interpolate_sequence with the scene state of `_clip`: returns (sequence, cuts or None, last mafd)."""
         if factor < 2 or len(frames) < 2:
-            return list(frames)
+            return list(frames), ([] if self.scene_threshold is not None else None), prev_mafd
         if factor & (factor - 1) == 0:
             # Bisection in place: the source frames go to every `factor`-th slot of one result array; each level reads
             # the frames already present (stride `step`) and writes their midpoints between them (the library takes
@@ -303,22 +337,29 @@ class FrameInterpolator:
                     list(ex.map(place, bounds[:-1], bounds[1:]))
             else:
                 place(0, n_src)
-            step = factor
+            # only the first level reads exactly the source pairs: it alone is scored
+            _, cuts, last_mafd = self._clip(seq[::factor], seq[factor // 2::factor], prev_mafd)
+            step = factor // 2
             while step > 1:
-                self.interpolate_clip(seq[::step], out=seq[step // 2::step])
+                self._clip(seq[::step], seq[step // 2::step], None)
                 step //= 2
-            return list(seq)
-        mids = self._sequence_midpoints(frames)
+            for i in cuts or ():
+                seq[i * factor + 1:(i + 1) * factor] = seq[i * factor]
+            return list(seq), cuts, last_mafd
+        arr = frames if isinstance(frames, np.ndarray) else np.stack(frames)
+        mids, cuts, last_mafd = self._clip(arr, None, prev_mafd)    # a cut pair's midpoint is already its first frame
         frames = list(frames)
         out = []
         for f, m in zip(frames[:-1], mids):
             out += [f] + [m] * (factor - 1)
-        return out + [frames[-1]]
+        return out + [frames[-1]], cuts, last_mafd
 
     def interpolate_video(self, input_path, output_path, factor=2, chunk=64):
         """Read `input_path` with cv2, write `output_path` (mp4v) at factor x the frame rate. Three stages run
         concurrently — a decoder thread, the GPU stage (this thread) and an encoder thread — joined by bounded queues,
-        so decode / encode (cv2 releases the GIL) overlap the forwards of the neighbouring chunks."""
+        so decode / encode (cv2 releases the GIL) overlap the forwards of the neighbouring chunks. With
+        `scene_threshold` set, the scene state crosses chunk edges and `last_scene_cuts` numbers the cut pairs of the
+        input video (pair i = frames i, i+1), so the cuts found do not depend on `chunk` or on the number of GPUs."""
         import queue
         import threading
         cap = cv2.VideoCapture(input_path)
@@ -389,12 +430,16 @@ class FrameInterpolator:
                 buf = ring[slot] = np.empty(shape, dtype=np.uint8)
             return buf
 
+        prev_mafd, first_pair, cuts = 0.0, 0, []
         try:
             while not failure:
                 new = decoded.get()
                 frames = new if prev is None else [prev] + new
                 if len(frames) >= 2:
-                    seq = self.interpolate_sequence(frames, factor, out=result_buffer(len(frames), frames[0].shape))
+                    seq, chunk_cuts, prev_mafd = self._sequence(frames, factor, result_buffer(len(frames), frames[0].shape),
+                                                                prev_mafd)
+                    cuts += [first_pair + i for i in chunk_cuts or ()]
+                    first_pair += len(frames) - 1
                     encoded.put(seq if prev is None else seq[1:])
                 elif frames and prev is None:
                     encoded.put(frames)          # a one-frame video is copied through
@@ -415,6 +460,8 @@ class FrameInterpolator:
             cap.release()
         if failure:
             raise failure[0]
+        if self.scene_threshold is not None:
+            self.last_scene_cuts = cuts
         return written[0]
 
 

@@ -24,8 +24,8 @@ except ImportError:  # model/ on sys.path, like the reference's scripts
 
 
 class GpuPool:
-    """`runners`: one object per GPU with `.interpolate_clip_host_u8(frames, pairs_per_batch, out=...)` (an
-    `_engine.Net`, or a stand-in in the CPU tests of the scheduling logic)."""
+    """`runners`: one object per GPU with `.interpolate_clip_host_u8(frames, pairs_per_batch, out=..., sad_out=...)`
+    (an `_engine.Net`, or a stand-in in the CPU tests of the scheduling logic)."""
 
     def __init__(self, runners):
         if not runners:
@@ -74,9 +74,10 @@ class GpuPool:
     def n_alive(self):
         return sum(self.alive)
 
-    def clip_midpoints(self, frames, pairs_per_batch, out):
+    def clip_midpoints(self, frames, pairs_per_batch, out, sad_out=None):
         """frames: uint8 [F,C,H,W] C-contiguous host array; out: uint8 [F-1,n_classes,H,W] C-contiguous. Pair i of the
-        clip lands in out[i] whichever GPU computed it."""
+        clip lands in out[i] whichever GPU computed it. sad_out: optional uint64 [F-1] array; the worker of pair i
+        writes its scene-cut statistic to sad_out[i] (a re-queued range rewrites the same slots)."""
         n_frames = frames.shape[0]
         if n_frames < 2:
             return out
@@ -103,8 +104,9 @@ class GpuPool:
                     try:
                         if self.fault_hook is not None:
                             self.fault_hook(widx, first, n)
+                        extra = {} if sad_out is None else {"sad_out": sad_out[first:first + n]}
                         self.runners[widx].interpolate_clip_host_u8(frames[first:first + n + 1], pairs_per_batch,
-                                                                     out=out[first:first + n])
+                                                                     out=out[first:first + n], **extra)
                     except Exception as e:  # noqa: BLE001 - retire this worker, re-queue what it had left
                         if getattr(e, "code", None) == -1:   # FI_ERR_INVALID: the request is bad, not the GPU
                             with lock:

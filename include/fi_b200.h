@@ -100,6 +100,15 @@ int fiNetInterpolateClipHostU8Strided(fiNet* net, const uint8_t* frames_host, in
                                       int channels_per_frame, uint8_t* out_host, int64_t out_stride, int H, int W,
                                       int pairs_per_batch, void* stream);
 
+/* The same, plus the scene-cut statistic of every pair (the reference has no scene detection): when pair_sad_host is
+ * not NULL it receives n_frames-1 uint64 values, pair_sad_host[i] = sum |f[i+1] - f[i]| over all C*H*W bytes (exact).
+ * Each batch's SAD runs on the frames the call has just uploaded (fiPairSadU8 on `stream`, before the forward) and is
+ * copied back with the batch's midpoints; the host frames are not read again. With NULL this is exactly the strided
+ * call above (which wraps it). */
+int fiNetInterpolateClipHostU8Sad(fiNet* net, const uint8_t* frames_host, int64_t frame_stride, int n_frames,
+                                  int channels_per_frame, uint8_t* out_host, int64_t out_stride, int H, int W,
+                                  int pairs_per_batch, void* stream, uint64_t* pair_sad_host);
+
 /* Algorithmic FLOPs (2*MACs, no padding) of one forward at this shape, and the number of kernel launches it makes. */
 int fiNetForwardCost(fiNet* net, int N, int H, int W, double* flops, int* launches);
 /* Measurement hook for bench.py: when enabled, every launch of the following forwards is bracketed by a CUDA event
@@ -194,6 +203,13 @@ int fiHeadPostU8(const float* logits, uint8_t* out, size_t n, void* stream);
 size_t fiSsimPsnrWorkspaceBytes(int N, int H, int W);
 int fiSsimPsnrU8(const uint8_t* pred, const uint8_t* target, int N, int H, int W, double* out, void* workspace,
                  void* stream);
+/* Scene-cut statistic (what ffmpeg's scdet and RIFE's video script compute on the host; the reference has none):
+ * sad[i] = sum over k < frame_bytes of |frames[(i+1)*frame_stride + k] - frames[i*frame_stride + k]| for the n_frames-1
+ * consecutive pairs of u8 frames, exact in 64 bit. sad is zeroed on `stream` first. Any alignment and stride work;
+ * 16-byte aligned frames take the vector path. FI_ERR_INVALID on NULL pointers, n_frames < 2, frame_bytes < 1 or
+ * frame_stride < frame_bytes. */
+int fiPairSadU8(const uint8_t* frames, int64_t frame_stride, int64_t frame_bytes, int n_frames, uint64_t* sad,
+                void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------
  * Training step (model/train.py:153-249; SURVEY.md §8f row 2): the kernels around the tensor-core convolutions.
