@@ -1345,7 +1345,11 @@ int fiPairSadU8(const uint8_t* frames, int64_t frame_stride, int64_t frame_bytes
 #define ST static_cast<cudaStream_t>(stream)
 
 int fiBnStats(const void* z, int64_t P, int C, float* sum, float* sumsq, void* stream) {
-    TRAIN_CALL(fi::bn_stats_launch(z, P, C, sum, sumsq, ST));
+    TRAIN_CALL(fi::bn_stats_launch(z, P, C, sum, sumsq, nullptr, ST));
+}
+int fiBnStatsShifted(const void* z, int64_t P, int C, float* pivot, float* sum, float* sumsq, void* stream) {
+    if (!pivot) return fail(FI_ERR_INVALID, "bn_stats: null pivot");
+    TRAIN_CALL(fi::bn_stats_launch(z, P, C, sum, sumsq, pivot, ST));
 }
 int fiBnApplyRelu(const void* z, int64_t P, int C, const float* scale, const float* shift, void* a, void* stream) {
     TRAIN_CALL(fi::bn_apply_relu_launch(z, P, C, scale, shift, a, ST));
@@ -1399,7 +1403,14 @@ int fiWgradPointwise(const void* dz, const void* x, int cin, int N, int H, int W
 int fiBnFinalize(const float* sum, const float* sumsq, int C, int64_t P, float eps, float momentum, const float* gamma,
                  const float* beta, float* mean, float* rstd, float* scale, float* shift, float* running_mean,
                  float* running_var, void* stream) {
-    TRAIN_CALL(fi::bn_finalize_launch(sum, sumsq, C, P, eps, momentum, gamma, beta, mean, rstd, scale, shift, running_mean,
+    TRAIN_CALL(fi::bn_finalize_launch(sum, sumsq, nullptr, C, P, eps, momentum, gamma, beta, mean, rstd, scale, shift,
+                                      running_mean, running_var, ST));
+}
+int fiBnFinalizeShifted(const float* sum, const float* sumsq, const float* pivot, int C, int64_t P, float eps,
+                        float momentum, const float* gamma, const float* beta, float* mean, float* rstd, float* scale,
+                        float* shift, float* running_mean, float* running_var, void* stream) {
+    if (!pivot) return fail(FI_ERR_INVALID, "bn_finalize: null pivot");
+    TRAIN_CALL(fi::bn_finalize_launch(sum, sumsq, pivot, C, P, eps, momentum, gamma, beta, mean, rstd, scale, shift, running_mean,
                                       running_var, ST));
 }
 int fiUnpackConvGrad(const float* dW, int cout, int cin, float* grad, void* stream) {

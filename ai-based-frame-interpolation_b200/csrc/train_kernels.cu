@@ -25,6 +25,9 @@ int blocks_for(long long items, int threads, int cap = 148 * 8) {
 // Per-channel reductions over z: bf16 [P][C]. A thread owns one 8-channel group (16-byte loads) and walks pixels with a
 // block-wide stride, four independent loads in flight; when C/8 divides 256 the 256/(C/8) pixel lanes of a block are
 // combined with shared-memory atomics so that a block issues one global atomic per channel and quantity.
+// With a pivot the sums are shifted, S = sum (z - k) and Q = sum (z - k)^2 with k = z[0][c] (every thread can load it),
+// so that var = Q/P - (S/P)^2 does not cancel when a channel's mean is large against its spread: a constant channel is
+// exact, and a flat one (dark frame, letterbox bar, the bias-free stem output) keeps its variance.
 constexpr int RED_MAX_C = 2048;
 
 template <typename Acc>
@@ -58,21 +61,33 @@ __device__ __forceinline__ void unpack8(const uint4& v, float (&f)[8]) {
 }
 
 __global__ void __launch_bounds__(256, 4)
-bn_stats_kernel(const uint4* __restrict__ z, long long P, int c8, float* __restrict__ sum, float* __restrict__ sumsq) {
+bn_stats_kernel(const uint4* __restrict__ z, long long P, int c8, float* __restrict__ sum, float* __restrict__ sumsq,
+                float* __restrict__ pivot) {
     __shared__ float sh[2][RED_MAX_C];
     const int C = 8 * c8;
     for (int i = threadIdx.x; i < C; i += 256) sh[0][i] = sh[1][i] = 0.f;
     __syncthreads();
     bool any_smem = false;
     channel_reduce_walk(P, c8, [&](int g, long long p, long long step, bool via_smem) {
-        float s[8], q[8];
+        float s[8], q[8], k[8];
 #pragma unroll
-        for (int j = 0; j < 8; ++j) s[j] = q[j] = 0.f;
+        for (int j = 0; j < 8; ++j) s[j] = q[j] = k[j] = 0.f;
+        if (pivot) {
+            unpack8(__ldg(z + g), k);   // pixel 0 of the group's channels
+            if (p == 0) {               // the one lane that starts at pixel 0 publishes the pivot for bn_finalize
+#pragma unroll
+                for (int j = 0; j < 8; ++j) pivot[8 * g + j] = k[j];
+            }
+        }
         auto add = [&](const uint4& v) {
             float f[8];
             unpack8(v, f);
 #pragma unroll
-            for (int j = 0; j < 8; ++j) { s[j] += f[j]; q[j] = fmaf(f[j], f[j], q[j]); }
+            for (int j = 0; j < 8; ++j) {
+                const float d = f[j] - k[j];   // exact for bf16 values within a factor 2^16 of each other
+                s[j] += d;
+                q[j] = fmaf(d, d, q[j]);
+            }
         };
         for (; p + 3 * step < P; p += 4 * step) {
             const uint4 v0 = __ldg(z + p * c8 + g), v1 = __ldg(z + (p + step) * c8 + g);
@@ -91,15 +106,18 @@ bn_stats_kernel(const uint4* __restrict__ z, long long P, int c8, float* __restr
 }
 
 // Batch statistics -> per-channel affine + the nn.BatchNorm2d running estimates (momentum update, unbiased variance).
+// sum / sumsq are taken about pivot[c] (NULL: about 0).
 __global__ void __launch_bounds__(256)
-bn_finalize_kernel(const float* __restrict__ sum, const float* __restrict__ sumsq, int C, float inv_p, float unbias,
+bn_finalize_kernel(const float* __restrict__ sum, const float* __restrict__ sumsq, const float* __restrict__ pivot,
+                   int C, float inv_p, float unbias,
                    float eps, float momentum, const float* __restrict__ gamma, const float* __restrict__ beta,
                    float* __restrict__ mean_out, float* __restrict__ rstd_out, float* __restrict__ scale,
                    float* __restrict__ shift, float* __restrict__ running_mean, float* __restrict__ running_var) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= C) return;
-    const float mean = sum[c] * inv_p;
-    const float var = fmaxf(sumsq[c] * inv_p - mean * mean, 0.f);
+    const float ms = sum[c] * inv_p;   // mean - pivot
+    const float mean = (pivot ? pivot[c] : 0.f) + ms;
+    const float var = fmaxf(sumsq[c] * inv_p - ms * ms, 0.f);
     const float rstd = rsqrtf(var + eps);
     const float sc = gamma[c] * rstd;
     mean_out[c] = mean;
@@ -670,15 +688,16 @@ unpack_conv_grad_kernel(const float* __restrict__ dW, long long n, float* __rest
 // ------------------------------------------------------------------------------------------------ optimizer / packing
 // torch.optim.Adam defaults (reference model/train.py:160): p -= lr * mhat / (sqrt(vhat) + eps)
 // hyper (optional, device): {lr, step} read at run time, so a captured CUDA graph of the step can be replayed while
-// the learning-rate schedule and the step count advance.
+// the learning-rate schedule and the step count advance. The bias corrections are computed here on both paths, so that
+// the two give the same bits.
 __global__ void __launch_bounds__(256)
 adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, long long n,
-            float lr, float b1, float b2, float eps, float bc1, float bc2, const float* __restrict__ hyper) {
+            float lr, float b1, float b2, float eps, float step, const float* __restrict__ hyper) {
     if (hyper) {
         lr = hyper[0];
-        bc1 = 1.f - powf(b1, hyper[1]);
-        bc2 = 1.f - powf(b2, hyper[1]);
+        step = hyper[1];
     }
+    const float bc1 = 1.f - powf(b1, step), bc2 = 1.f - powf(b2, step);
     for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n;
          i += static_cast<long long>(gridDim.x) * blockDim.x) {
         const float gi = g[i];
@@ -758,16 +777,16 @@ int apply_blocks(long long n8, int c8) {
 }
 }  // namespace
 
-const char* bn_stats_launch(const void* z, long long P, int C, float* sum, float* sumsq, cudaStream_t st) {
+const char* bn_stats_launch(const void* z, long long P, int C, float* sum, float* sumsq, float* pivot, cudaStream_t st) {
     FI_REQUIRE(z && sum && sumsq && P > 0 && C > 0 && C % 8 == 0 && C <= RED_MAX_C, "bn_stats: bad arguments");
-    bn_stats_kernel<<<reduce_blocks(P, C / 8), 256, 0, st>>>(static_cast<const uint4*>(z), P, C / 8, sum, sumsq);
+    bn_stats_kernel<<<reduce_blocks(P, C / 8), 256, 0, st>>>(static_cast<const uint4*>(z), P, C / 8, sum, sumsq, pivot);
     return last_error();
 }
-const char* bn_finalize_launch(const float* sum, const float* sumsq, int C, long long P, float eps, float momentum,
-                               const float* gamma, const float* beta, float* mean, float* rstd, float* scale, float* shift,
-                               float* running_mean, float* running_var, cudaStream_t st) {
+const char* bn_finalize_launch(const float* sum, const float* sumsq, const float* pivot, int C, long long P, float eps,
+                               float momentum, const float* gamma, const float* beta, float* mean, float* rstd,
+                               float* scale, float* shift, float* running_mean, float* running_var, cudaStream_t st) {
     FI_REQUIRE(sum && sumsq && gamma && beta && mean && rstd && scale && shift && C > 0 && P > 0, "bn_finalize: bad arguments");
-    bn_finalize_kernel<<<(C + 255) / 256, 256, 0, st>>>(sum, sumsq, C, 1.0f / static_cast<float>(P),
+    bn_finalize_kernel<<<(C + 255) / 256, 256, 0, st>>>(sum, sumsq, pivot, C, 1.0f / static_cast<float>(P),
                                                         P > 1 ? static_cast<float>(P) / static_cast<float>(P - 1) : 1.f, eps,
                                                         momentum, gamma, beta, mean, rstd, scale, shift, running_mean,
                                                         running_var);
@@ -889,8 +908,7 @@ const char* unpack_conv_grad_launch(const float* dW, int cout, int cin, float* g
 const char* adam_launch(float* p, const float* g, float* m, float* v, long long n, float lr, float b1, float b2, float eps,
                         int step, const float* hyper, cudaStream_t st) {
     FI_REQUIRE(p && g && m && v && n > 0 && (step >= 1 || hyper), "adam: bad arguments");
-    adam_kernel<<<blocks_for(n, 256), 256, 0, st>>>(p, g, m, v, n, lr, b1, b2, eps, 1.f - powf(b1, static_cast<float>(step)),
-                                                   1.f - powf(b2, static_cast<float>(step)), hyper);
+    adam_kernel<<<blocks_for(n, 256), 256, 0, st>>>(p, g, m, v, n, lr, b1, b2, eps, static_cast<float>(step), hyper);
     return last_error();
 }
 const char* stem_pack_device_launch(const float* w, int cin, void* out, cudaStream_t st) {

@@ -7,10 +7,11 @@
 
 namespace fi {
 
-const char* bn_stats_launch(const void* z, long long P, int C, float* sum, float* sumsq, cudaStream_t st);
-const char* bn_finalize_launch(const float* sum, const float* sumsq, int C, long long P, float eps, float momentum,
-                               const float* gamma, const float* beta, float* mean, float* rstd, float* scale, float* shift,
-                               float* running_mean, float* running_var, cudaStream_t st);
+// pivot: NULL = plain sums; else pivot[c] = z[0][c] is written and the sums are taken about it
+const char* bn_stats_launch(const void* z, long long P, int C, float* sum, float* sumsq, float* pivot, cudaStream_t st);
+const char* bn_finalize_launch(const float* sum, const float* sumsq, const float* pivot, int C, long long P, float eps,
+                               float momentum, const float* gamma, const float* beta, float* mean, float* rstd,
+                               float* scale, float* shift, float* running_mean, float* running_var, cudaStream_t st);
 const char* bn_apply_relu_launch(const void* z, long long P, int C, const float* scale, const float* shift, void* a,
                                  cudaStream_t st);
 const char* head_forward_launch(const void* a, int N, long long HW, const float* w, const float* b, int ncls, float* y,

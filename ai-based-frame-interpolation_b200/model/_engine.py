@@ -87,6 +87,7 @@ _SIGNATURES = {
     "fiPairSadU8": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_void_p]),
     # training-step kernels
     "fiBnStats": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fiBnStatsShifted": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "fiBnApplyRelu": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "fiHeadForward": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "fiMseLossGrad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -108,6 +109,9 @@ _SIGNATURES = {
     "fiStemWgrad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "fiBnFinalize": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_float, C.c_void_p, C.c_void_p,
                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fiBnFinalizeShifted": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_float,
+                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_void_p, C.c_void_p]),
     "fiUnpackConvGrad": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "fiAdamStep": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_float, C.c_float, C.c_float,
                              C.c_float, C.c_int, C.c_void_p, C.c_void_p]),

@@ -199,15 +199,16 @@ class TrainStep:
 
     def _bn_forward(self, layer, z, work):
         """Batch statistics -> a = relu(bn(z)); returns (a, work) and updates the running statistics.
-        work: zeroed fp32 [6, C] scratch (sum, sumsq, mean, rstd, scale, shift)."""
+        work: zeroed fp32 [7, C] scratch (sum, sumsq, mean, rstd, scale, shift, pivot). The sums are taken about the
+        pivot (the channel's first pixel) so that flat channels keep their variance in fp32."""
         n, h, w, c = z.shape
         P = n * h * w
         st = E.current_stream()
-        E.check(self.lib.fiBnStats(_ptr(z), P, c, _ptr(work[0]), _ptr(work[1]), st))
+        E.check(self.lib.fiBnStatsShifted(_ptr(z), P, c, _ptr(work[6]), _ptr(work[0]), _ptr(work[1]), st))
         bn = layer.bn
-        E.check(self.lib.fiBnFinalize(_ptr(work[0]), _ptr(work[1]), c, P, bn.eps, BN_MOMENTUM, _ptr(bn.weight),
-                                      _ptr(bn.bias), _ptr(work[2]), _ptr(work[3]), _ptr(work[4]), _ptr(work[5]),
-                                      _ptr(bn.running_mean), _ptr(bn.running_var), st))
+        E.check(self.lib.fiBnFinalizeShifted(_ptr(work[0]), _ptr(work[1]), _ptr(work[6]), c, P, bn.eps, BN_MOMENTUM,
+                                             _ptr(bn.weight), _ptr(bn.bias), _ptr(work[2]), _ptr(work[3]), _ptr(work[4]),
+                                             _ptr(work[5]), _ptr(bn.running_mean), _ptr(bn.running_var), st))
         a = torch.empty_like(z)
         E.check(self.lib.fiBnApplyRelu(_ptr(z), P, c, _ptr(work[4]), _ptr(work[5]), _ptr(a), st))
         return a, work
@@ -303,13 +304,13 @@ class TrainStep:
             self.flat_grad.zero_()
             acts, zs, stats, packs = {}, {}, {}, {}
             # one zeroed scratch for every layer's BatchNorm reductions / affine and weight-gradient accumulators
-            bn_total = sum(6 * l.cout for l in self.layers)
+            bn_total = sum(7 * l.cout for l in self.layers)
             dw_total = sum(9 * l.cout * l.cin for l in self.layers[1:])
             scratch = torch.zeros(bn_total + dw_total, dtype=torch.float32, device=self.device)
             bn_work, dw_work, off = {}, {}, 0
             for l in self.layers:
-                bn_work[l.name] = scratch[off:off + 6 * l.cout].view(6, l.cout)
-                off += 6 * l.cout
+                bn_work[l.name] = scratch[off:off + 7 * l.cout].view(7, l.cout)
+                off += 7 * l.cout
             for l in self.layers[1:]:
                 dw_work[l.name] = scratch[off:off + 9 * l.cout * l.cin]
                 off += 9 * l.cout * l.cin
@@ -398,7 +399,7 @@ class TrainStep:
                 a, z = acts[l.name], zs[l.name]
                 ln, lh, lw, lc = z.shape
                 P = ln * lh * lw
-                wk = stats[l.name]       # rows: sum, sumsq, mean, rstd, scale, shift
+                wk = stats[l.name]       # rows: sum, sumsq, mean, rstd, scale, shift, pivot
                 dA = grads.pop(l.name)
                 dbeta, dgamma = self.grad_view[l.bn.bias], self.grad_view[l.bn.weight]   # zeroed with flat_grad
                 E.check(lib.fiBnReluBackwardReduce(_ptr(dA), _ptr(z), P, lc, _ptr(wk[2]), _ptr(wk[3]), _ptr(wk[4]),
@@ -431,21 +432,9 @@ class TrainStep:
                     below = self.layers[self.layers.index(l) - 1].name   # the tensor that was upsampled
                     bn_, bh, bw_, bc = acts[below].shape
                     if self.convt:
-                        # ConvTranspose2d backward. Per low-resolution pixel the output gradient is a vector over
-                        # (ky, kx, co): d_lo = that vector times W (a per-pixel GEMM, K = 4*Cout), dW = sum over pixels
-                        # of the outer product with the layer input (fiWgradPointwise), dbias = per-channel sum.
                         tmod = self.up_mods[l.name]
-                        cup = d_up.shape[3]
-                        d_s2d = d_up.view(bn_, bh, 2, bw_, 2, cup).permute(0, 1, 3, 2, 4, 5).contiguous().view(
-                            bn_, bh, bw_, 4 * cup)
-                        d_lo = self._conv(d_s2d, packs[l.src1], bc, taps=1)
-                        sumsq = torch.zeros(cup, dtype=torch.float32, device=self.device)
-                        E.check(lib.fiBnStats(_ptr(d_up), bn_ * bh * bw_ * 4, cup, _ptr(self.grad_view[tmod.bias]),
-                                              _ptr(sumsq), st()))
-                        dwt = torch.zeros((4 * cup, bc), dtype=torch.float32, device=self.device)
-                        E.check(lib.fiWgradPointwise(_ptr(d_s2d), _ptr(acts[below]), bc, bn_, bh, bw_, 4 * cup, _ptr(dwt),
-                                                     st()))
-                        self.grad_view[tmod.weight].add_(dwt.view(2, 2, cup, bc).permute(3, 2, 0, 1))
+                        d_lo = self._convt_backward(d_up, acts[below], packs[l.src1], self.grad_view[tmod.weight],
+                                                    self.grad_view[tmod.bias])
                     else:
                         d_lo = torch.empty_like(acts[below])
                         E.check(lib.fiUpsample2xBackward(_ptr(d_up), _ptr(d_lo), bn_, bh, bw_, bc, st()))
@@ -467,6 +456,25 @@ class TrainStep:
         self.last_output = y
         self.last_activations = acts if self.keep_activations else None   # diagnostics only: pins GBs of HBM
         yield loss
+
+    def _convt_backward(self, d_up, x, w_lo, grad_w, grad_b):
+        """ConvTranspose2d(k=2, s=2) backward. Per low-resolution pixel the output gradient is a vector over
+        (ky, kx, co): d_lo = that vector times W (a per-pixel GEMM, K = 4*Cout), dW = sum over pixels of the outer
+        product with the layer input (fiWgradPointwise), dbias = per-channel sum.
+        d_up: bf16 [N,2h,2w,Cout] output gradient; x: bf16 [N,h,w,Cin] layer input; w_lo: bf16 [Cin][(ky,kx,co)] rows
+        of the data-gradient GEMM. dW and dbias are ADDED into grad_w (fp32 [Cin,Cout,2,2]) and grad_b (fp32 [Cout]).
+        Returns d_lo: bf16 [N,h,w,Cin]."""
+        lib, st = self.lib, E.current_stream
+        bn_, bh, bw_, bc = x.shape
+        cup = d_up.shape[3]
+        d_s2d = d_up.view(bn_, bh, 2, bw_, 2, cup).permute(0, 1, 3, 2, 4, 5).contiguous().view(bn_, bh, bw_, 4 * cup)
+        d_lo = self._conv(d_s2d, w_lo, bc, taps=1)
+        sumsq = torch.zeros(cup, dtype=torch.float32, device=self.device)
+        E.check(lib.fiBnStats(_ptr(d_up), bn_ * bh * bw_ * 4, cup, _ptr(grad_b), _ptr(sumsq), st()))
+        dwt = torch.zeros((4 * cup, bc), dtype=torch.float32, device=self.device)
+        E.check(lib.fiWgradPointwise(_ptr(d_s2d), _ptr(x), bc, bn_, bh, bw_, 4 * cup, _ptr(dwt), st()))
+        grad_w.add_(dwt.view(2, 2, cup, bc).permute(3, 2, 0, 1))
+        return d_lo
 
     def _finish(self, early):
         """Rest of the gradient all-reduce across data-parallel replicas (NCCL over NVLink; `early` is the handle of

@@ -217,8 +217,12 @@ int fiPairSadU8(const uint8_t* frames, int64_t frame_stride, int64_t frame_bytes
  * Conv forward and the data gradient reuse fiConvGemm (the latter with the flipped/transposed weights that
  * fiPackConvWeights writes); the host side of one step is model/train.py:TrainStep.
  * ---------------------------------------------------------------------------------------------------------------- */
-/* nn.BatchNorm2d in training mode (model/unet.py:13,16): per-channel sum / sum of squares (accumulated into sum, sumsq). */
+/* nn.BatchNorm2d in training mode (model/unet.py:13,16): per-channel sum / sum of squares (accumulated into sum, sumsq).
+ * fiBnStats: plain sums (also the bias gradient of ConvTranspose2d). fiBnStatsShifted: pivot[c] = z[0][c] is written and
+ * the sums are taken about it, sum += sum (z - pivot), sumsq += sum (z - pivot)^2, for fiBnFinalizeShifted: the variance
+ * then does not cancel on channels whose mean is large against their spread. */
 int fiBnStats(const void* z, int64_t P, int C, float* sum, float* sumsq, void* stream);
+int fiBnStatsShifted(const void* z, int64_t P, int C, float* pivot, float* sum, float* sumsq, void* stream);
 /* a = relu(z*scale[c] + shift[c]) with scale = gamma*rstd, shift = beta - mean*scale. */
 int fiBnApplyRelu(const void* z, int64_t P, int C, const float* scale, const float* shift, void* a, void* stream);
 /* OutConv (model/unet.py:57-63) on bf16 [N*HW][64] -> fp32 NCHW [N,n_classes,H,W]. */
@@ -258,10 +262,15 @@ int fiStemWgrad(const void* dz, const float* x, int N, int H, int W, int cin, fl
  * once its output gradient is viewed per low-resolution pixel as [N,h,w,(ky,kx,co)] (cout = 4*Cout); cin/64 even. */
 int fiWgradPointwise(const void* dz, const void* x, int cin, int N, int H, int W, int cout, float* dW, void* stream);
 /* Batch sums -> mean, rstd = 1/sqrt(var + eps), scale = gamma * rstd, shift = beta - mean * scale (C floats each), and
- * the nn.BatchNorm2d running estimates updated in place (momentum, unbiased variance; either may be NULL). */
+ * the nn.BatchNorm2d running estimates updated in place (momentum, unbiased variance; either may be NULL).
+ * fiBnFinalize: from fiBnStats' plain sums. fiBnFinalizeShifted: from the sums and the pivot fiBnStatsShifted wrote
+ * (what the training step uses). */
 int fiBnFinalize(const float* sum, const float* sumsq, int C, int64_t P, float eps, float momentum, const float* gamma,
                  const float* beta, float* mean, float* rstd, float* scale, float* shift, float* running_mean,
                  float* running_var, void* stream);
+int fiBnFinalizeShifted(const float* sum, const float* sumsq, const float* pivot, int C, int64_t P, float eps,
+                        float momentum, const float* gamma, const float* beta, float* mean, float* rstd, float* scale,
+                        float* shift, float* running_mean, float* running_var, void* stream);
 /* fiWgrad's dW[tap][cout][cin] added into the parameter-gradient layout grad[cout][cin][3][3]. */
 int fiUnpackConvGrad(const float* dW, int cout, int cin, float* grad, void* stream);
 /* torch.optim.Adam (model/train.py:160) on one flat fp32 parameter vector; step counts from 1. hyper_dev (optional,

@@ -212,6 +212,33 @@ def test_bn_finalize_and_running_statistics(cuda_device):
     assert torch.allclose(got, ref.detach(), rtol=1e-3, atol=2e-3)
 
 
+def test_bn_shifted_finalize_and_running_statistics(cuda_device):
+    """The pair TrainStep runs: sums about each channel's first pixel, then the finalize that adds it back."""
+    lib, st = E.lib(), E.current_stream()
+    g = torch.Generator().manual_seed(8)
+    n, c, h, w = 3, 192, 5, 6   # C/8 = 24 does not divide 256: the unpacked reduction walk
+    z = (torch.randn(n, c, h, w, generator=g) * 2 + 0.5).to(torch.bfloat16).float()
+    bn = torch.nn.BatchNorm2d(c)
+    bn.weight.data, bn.bias.data = torch.rand(c, generator=g) + 0.5, torch.randn(c, generator=g)
+    bn.running_mean.data, bn.running_var.data = torch.randn(c, generator=g), torch.rand(c, generator=g) + 0.5
+    rm, rv = bn.running_mean.clone().to(cuda_device), bn.running_var.clone().to(cuda_device)
+    bn.train()
+    ref = bn(z)
+    P = n * h * w
+    zd = nhwc(z, cuda_device)
+    work = torch.zeros(7, c, device=cuda_device)   # sum, sumsq, mean, rstd, scale, shift, pivot
+    gd, bd = bn.weight.detach().to(cuda_device), bn.bias.detach().to(cuda_device)
+    E.check(lib.fiBnStatsShifted(p(zd), P, c, p(work[6]), p(work[0]), p(work[1]), st))
+    E.check(lib.fiBnFinalizeShifted(p(work[0]), p(work[1]), p(work[6]), c, P, bn.eps, 0.1, p(gd), p(bd), p(work[2]),
+                                    p(work[3]), p(work[4]), p(work[5]), p(rm), p(rv), st))
+    torch.cuda.synchronize()
+    assert torch.equal(work[6].cpu(), z[0, :, 0, 0]), "pivot = the first pixel"
+    assert torch.allclose(rm.cpu(), bn.running_mean, rtol=1e-4, atol=1e-5)
+    assert torch.allclose(rv.cpu(), bn.running_var, rtol=1e-3, atol=1e-5)
+    got = nchw(zd.float() * work[4] + work[5])
+    assert torch.allclose(got, ref.detach(), rtol=1e-3, atol=2e-3)
+
+
 def test_unpack_conv_grad(cuda_device):
     lib, st = E.lib(), E.current_stream()
     g = torch.Generator().manual_seed(6)
