@@ -1,6 +1,6 @@
 // CUDA-core kernels of the frame-synthesis path (the stem convolution lives in stem_mma.cu): the bilinear
-// decoder upsample, frame-pair packing, output post-processing, the fused SSIM+PSNR metric kernel and the
-// frame-pair SAD of scene-cut detection.
+// decoder upsample, frame-pair packing, output post-processing, the fused SSIM+PSNR metric kernel, the
+// frame-pair SAD of scene-cut detection and the training-batch gather from the device frame cache.
 #include "aux_kernels.cuh"
 #include "ptx.cuh"
 
@@ -8,16 +8,20 @@ namespace fi {
 
 namespace {
 
-__device__ __forceinline__ float norm_u8(uint32_t u) {
-    // image.astype(float32)/255.0 then 2.0*image-1.0, each rounded to fp32 (reference model/inference.py:32-35).
+__device__ __forceinline__ float div255_u8(uint32_t u) {
+    // image.astype(float32)/255.0 rounded to fp32 (reference model/train.py:138, model/inference.py:32).
     // u/255 is formed as u*(1/255) plus one FMA residual correction, which is the correctly rounded quotient for all
-    // 256 inputs (checked exhaustively by tests/test_gpu_aux_kernels.py::test_pack_pair_bit_exact) at a third of the
-    // instruction count of an IEEE division.
+    // 256 inputs (checked exhaustively by tests/test_gpu_aux_kernels.py::test_pack_pair_bit_exact and
+    // tests/test_gpu_frame_cache.py) at a third of the instruction count of an IEEE division.
     const float x = static_cast<float>(u);
     const float r = 1.0f / 255.0f;
     const float q = __fmul_rn(x, r);
-    const float q2 = __fmaf_rn(__fmaf_rn(-q, 255.0f, x), r, q);
-    return __fmaf_rn(2.0f, q2, -1.0f);  // 2*q2 is exact, so this is fl(2*q2 - 1)
+    return __fmaf_rn(__fmaf_rn(-q, 255.0f, x), r, q);
+}
+
+__device__ __forceinline__ float norm_u8(uint32_t u) {
+    // then 2.0*image-1.0, rounded to fp32 (reference model/inference.py:32-35)
+    return __fmaf_rn(2.0f, div255_u8(u), -1.0f);  // 2*q is exact, so this is fl(2*q - 1)
 }
 
 // ------------------------------------------------------------------------------------------------ bilinear x2
@@ -445,6 +449,53 @@ pair_sad_kernel(const uint8_t* __restrict__ frames, long long frame_stride, long
     }
 }
 
+// ------------------------------------------------------------------------------------------------ triplet gather
+// Training batches from the device-resident u8 frame cache: output row r = 3*b + k is
+// out_k[b] = frames[triplets[samples[b]][k]] / 255 (FrameTripletDataset's img.astype(float32) / 255.0, bit for bit).
+// blockIdx.y walks the rows (grid-stride), blockIdx.x the plane; a row's indices are block-uniform. A sample whose index
+// or any of whose three frame indices is out of range has all three outputs written as NaN and nothing of it is read.
+// Vector path: 16 pixels per thread, one 16-byte load and four 16-byte stores; the byte path covers any H*W.
+constexpr int GT_THREADS = 256;
+
+__global__ void __launch_bounds__(GT_THREADS)
+gather_triplets_u8_kernel(const uint8_t* __restrict__ frames, long long n_frames, const int* __restrict__ triplets,
+                          long long n_triplets, const long long* __restrict__ samples, long long rows, long long plane,
+                          int vec, float* __restrict__ out0, float* __restrict__ out1, float* __restrict__ out2) {
+    const float nan = __int_as_float(0x7fc00000);
+    const long long tid = static_cast<long long>(blockIdx.x) * GT_THREADS + threadIdx.x;
+    const long long nthr = static_cast<long long>(gridDim.x) * GT_THREADS;
+    const long long n16 = vec ? plane / 16 : 0;
+    for (long long row = blockIdx.y; row < rows; row += gridDim.y) {
+        const long long b = row / 3;
+        const int k = static_cast<int>(row - 3 * b);
+        float* out = (k == 0 ? out0 : k == 1 ? out1 : out2) + b * plane;
+        const long long s = __ldg(samples + b);
+        bool ok = s >= 0 && s < n_triplets;
+        long long f = 0;
+        if (ok) {
+            const int t0 = __ldg(triplets + 3 * s), t1 = __ldg(triplets + 3 * s + 1), t2 = __ldg(triplets + 3 * s + 2);
+            ok = t0 >= 0 && t0 < n_frames && t1 >= 0 && t1 < n_frames && t2 >= 0 && t2 < n_frames;
+            f = k == 0 ? t0 : k == 1 ? t1 : t2;
+        }
+        const uint8_t* src = frames + f * plane;
+        for (long long i = tid; i < n16; i += nthr) {
+            float4* o = reinterpret_cast<float4*>(out) + i * 4;
+            if (ok) {
+                const uint4 v = __ldg(reinterpret_cast<const uint4*>(src) + i);
+                const uint32_t wv[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+                for (int q = 0; q < 4; ++q)
+                    o[q] = make_float4(div255_u8(wv[q] & 0xff), div255_u8((wv[q] >> 8) & 0xff),
+                                       div255_u8((wv[q] >> 16) & 0xff), div255_u8(wv[q] >> 24));
+            } else {
+#pragma unroll
+                for (int q = 0; q < 4; ++q) o[q] = make_float4(nan, nan, nan, nan);
+            }
+        }
+        for (long long i = n16 * 16 + tid; i < plane; i += nthr) out[i] = ok ? div255_u8(__ldg(src + i)) : nan;
+    }
+}
+
 int grid_for(size_t work_items, int threads) {
     size_t g = (work_items + threads - 1) / threads;
     const size_t cap = 148 * 16;  // grid-stride loops: a few waves of the 148 SMs is enough
@@ -553,6 +604,27 @@ const char* pair_sad_launch(const uint8_t* frames, int64_t frame_stride, int64_t
     if (e != cudaSuccess) return cudaGetErrorString(e);
     pair_sad_kernel<<<dim3(static_cast<unsigned>(gx), gy), PS_THREADS, 0, stream>>>(
         frames, frame_stride, frame_bytes, n_pairs, vec, reinterpret_cast<unsigned long long*>(sad));
+    return last_launch_error();
+}
+
+const char* gather_triplets_u8_launch(const uint8_t* frames, int64_t n_frames, const int32_t* triplets,
+                                      int64_t n_triplets, const int64_t* samples, int n, int H, int W, float* frame1,
+                                      float* frame2, float* target, cudaStream_t stream) {
+    if (!frames || !triplets || !samples || !frame1 || !frame2 || !target) return "gather: null operand";
+    if (n < 1 || H < 1 || W < 1) return "gather: needs n, H, W >= 1";
+    if (n_frames < 0 || n_triplets < 0) return "gather: negative frame or triplet count";
+    const long long plane = static_cast<long long>(H) * W;
+    const int vec = plane % 16 == 0 && ((reinterpret_cast<uintptr_t>(frames) | reinterpret_cast<uintptr_t>(frame1) |
+                                         reinterpret_cast<uintptr_t>(frame2) | reinterpret_cast<uintptr_t>(target)) %
+                                        16) == 0;
+    const long long units = vec ? plane / 16 : plane;
+    const long long rows = 3LL * n;
+    long long gx = (units + GT_THREADS - 1) / GT_THREADS;
+    if (gx > 148 * 16) gx = 148 * 16;
+    const long long gy = rows < 65535 ? rows : 65535;
+    gather_triplets_u8_kernel<<<dim3(static_cast<unsigned>(gx), static_cast<unsigned>(gy)), GT_THREADS, 0, stream>>>(
+        frames, n_frames, triplets, n_triplets, reinterpret_cast<const long long*>(samples), rows, plane, vec, frame1,
+        frame2, target);
     return last_launch_error();
 }
 

@@ -52,4 +52,10 @@ const char* ssim_psnr_launch(const uint8_t* a, const uint8_t* b, int N, int H, i
 const char* pair_sad_launch(const uint8_t* frames, int64_t frame_stride, int64_t frame_bytes, int n_frames,
                             uint64_t* sad, cudaStream_t stream);
 
+// Training batch from the device frame cache: frame1/frame2/target[b] = frames[triplets[samples[b]][0|1|2]] / 255 as
+// fp32 [n][H*W]; out-of-range samples or frame indices give NaN rows (fiGatherTripletsU8).
+const char* gather_triplets_u8_launch(const uint8_t* frames, int64_t n_frames, const int32_t* triplets,
+                                      int64_t n_triplets, const int64_t* samples, int n, int H, int W, float* frame1,
+                                      float* frame2, float* target, cudaStream_t stream);
+
 }  // namespace fi

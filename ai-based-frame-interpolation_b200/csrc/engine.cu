@@ -1334,6 +1334,18 @@ int fiPairSadU8(const uint8_t* frames, int64_t frame_stride, int64_t frame_bytes
     return FI_OK;
 }
 
+int fiGatherTripletsU8(const uint8_t* frames, int64_t n_frames, const int32_t* triplets, int64_t n_triplets,
+                       const int64_t* samples, int n, int H, int W, float* frame1, float* frame2, float* target,
+                       void* stream) {
+    if (!frames || !triplets || !samples || !frame1 || !frame2 || !target) return fail(FI_ERR_INVALID, "null argument");
+    if (n < 1 || H < 1 || W < 1) return fail(FI_ERR_INVALID, "needs n, H and W >= 1 (got %d, %d, %d)", n, H, W);
+    if (n_frames < 0 || n_triplets < 0) return fail(FI_ERR_INVALID, "negative frame or triplet count");
+    const char* e = fi::gather_triplets_u8_launch(frames, n_frames, triplets, n_triplets, samples, n, H, W, frame1,
+                                                  frame2, target, static_cast<cudaStream_t>(stream));
+    if (e) return fail(FI_ERR_CUDA, "%s", e);
+    return FI_OK;
+}
+
 
 // ---------------------------------------------------------------------------------------------- training-step kernels
 #define TRAIN_CALL(expr)                                        \

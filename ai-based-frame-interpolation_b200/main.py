@@ -20,13 +20,16 @@ def _scene_threshold(text):
 def build_parser():
     p = argparse.ArgumentParser(description="AI-Based Frame Interpolation (B200-native path)")
     sub = p.add_subparsers(dest="command", help="Available commands")
-    # flags, defaults and required-ness as reference main.py:40-72; --gpus and --scene-threshold are the only additions
+    # flags, defaults and required-ness as reference main.py:40-72; --frame-cache, --gpus and --scene-threshold are the
+    # only additions
     t = sub.add_parser("train", help="Train the frame interpolation model")
     t.add_argument("--data-dir", required=True, help="Directory containing training data")
     t.add_argument("--epochs", type=int, default=100, help="Number of training epochs")
     t.add_argument("--batch-size", type=int, default=8, help="Training batch size")
     t.add_argument("--lr", type=float, default=0.001, help="Learning rate")
     t.add_argument("--device", default="auto", help="Device to use (cuda/auto)")
+    t.add_argument("--frame-cache", action="store_true",
+                   help="Decode every frame once into GPU memory and build the batches there (default: off)")
     i = sub.add_parser("infer", help="Run inference on two frames")
     i.add_argument("--frame1", required=True, help="Path to first frame")
     i.add_argument("--frame2", required=True, help="Path to second frame")
@@ -72,6 +75,8 @@ def main(argv=None):
                 fwd += ["--lr", str(args.lr)]
             if "--batch-size" in typed:
                 fwd += ["--batch-size", str(args.batch_size)]
+            if args.frame_cache:
+                fwd.append("--frame-cache")
             train_main(fwd)
             return 0
         if args.command == "infer":

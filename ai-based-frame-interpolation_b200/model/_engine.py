@@ -85,6 +85,8 @@ _SIGNATURES = {
     "fiSsimPsnrU8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                C.c_void_p]),
     "fiPairSadU8": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_void_p]),
+    "fiGatherTripletsU8": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int, C.c_int,
+                                     C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     # training-step kernels
     "fiBnStats": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "fiBnStatsShifted": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -339,6 +341,30 @@ def pair_sad_u8(frames: torch.Tensor) -> torch.Tensor:
         check(lib().fiPairSadU8(frames.data_ptr(), frames.stride(0), frames[0].numel(), frames.shape[0], out.data_ptr(),
                                 current_stream()))
     return out
+
+
+def gather_triplets_u8(frames: torch.Tensor, triplets: torch.Tensor, samples: torch.Tensor):
+    """frames: uint8 CUDA [F,H,W]; triplets: int32 CUDA [T,3] frame indices of (t0, t1, ground truth); samples: int64
+    CUDA [n] triplet indices. Returns three fresh fp32 tensors [n,1,H,W] (frame1, frame2, target) = the frames / 255,
+    written by one fiGatherTripletsU8 launch on the current stream (no host synchronisation). A sample that is out of
+    range, or names a frame that is, comes back as NaN."""
+    require_cuda(frames.device)
+    if frames.dtype != torch.uint8 or frames.dim() != 3 or not frames.is_contiguous():
+        raise FiError("frames must be a contiguous uint8 tensor [F,H,W]")
+    if triplets.dtype != torch.int32 or triplets.dim() != 2 or triplets.shape[1] != 3 or not triplets.is_contiguous():
+        raise FiError("triplets must be a contiguous int32 tensor [T,3]")
+    if samples.dtype != torch.int64 or samples.dim() != 1 or not samples.is_contiguous() or samples.numel() < 1:
+        raise FiError("samples must be a non-empty contiguous int64 tensor [n]")
+    if not (triplets.device == samples.device == frames.device):
+        raise FiError("frames, triplets and samples must be on the same device")
+    f, h, w = frames.shape
+    n = samples.numel()
+    out = torch.empty((3, n, 1, h, w), dtype=torch.float32, device=frames.device)
+    with torch.cuda.device(frames.device):
+        check(lib().fiGatherTripletsU8(frames.data_ptr(), f, triplets.data_ptr(), triplets.shape[0], samples.data_ptr(),
+                                       n, h, w, out[0].data_ptr(), out[1].data_ptr(), out[2].data_ptr(),
+                                       current_stream()))
+    return out[0], out[1], out[2]
 
 
 def pack_pair_u8(f1: torch.Tensor, f2: torch.Tensor) -> torch.Tensor:

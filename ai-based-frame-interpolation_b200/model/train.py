@@ -667,6 +667,9 @@ def main(argv=None):
     ap.add_argument("--val-split", type=float, default=0.2)
     ap.add_argument("--lr", type=float, default=1e-4)
     ap.add_argument("--no-cuda-graph", action="store_true", help="run the step eagerly instead of replaying CUDA graphs")
+    ap.add_argument("--frame-cache", action="store_true",
+                    help="decode every frame once into GPU memory (64 KB a frame) and build batches there instead of "
+                         "decoding three files per sample in DataLoader workers")
     args = ap.parse_args(argv)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if world > 1:
@@ -684,11 +687,22 @@ def main(argv=None):
     train_set, val_set = torch.utils.data.random_split(data, [len(data) - n_val, n_val], generator=split_gen)
     if rank0:
         print(f"Dataset split: {len(train_set)} train, {len(val_set)} validation")
+    cache = None
+    if args.frame_cache:
+        try:
+            from .framecache import CachedTripletLoader, FrameCache, build_info
+        except ImportError:
+            from framecache import CachedTripletLoader, FrameCache, build_info
+        cache = FrameCache.build(data, device)        # one cache: train and validation triplets share its frames
+        if rank0:
+            print(build_info(cache))
 
     def mk(d, shuffle):
         sampler = None
         if world > 1:
             sampler = torch.utils.data.distributed.DistributedSampler(d, shuffle=shuffle, drop_last=shuffle)
+        if cache is not None:
+            return CachedTripletLoader(d, cache, args.batch_size, sampler=sampler, shuffle=shuffle and sampler is None)
         return torch.utils.data.DataLoader(d, batch_size=args.batch_size, shuffle=shuffle and sampler is None,
                                            sampler=sampler, num_workers=4, pin_memory=True)
 

@@ -210,6 +210,15 @@ int fiSsimPsnrU8(const uint8_t* pred, const uint8_t* target, int N, int H, int W
  * frame_stride < frame_bytes. */
 int fiPairSadU8(const uint8_t* frames, int64_t frame_stride, int64_t frame_bytes, int n_frames, uint64_t* sad,
                 void* stream);
+/* FrameTripletDataset.__getitem__ + the DataLoader collate (model/train.py:89-151) for frames already on the device:
+ * frames u8 [n_frames][H][W], triplets int32 [n_triplets][3] = frame indices of (t0, t1, ground truth), samples int64
+ * [n] = triplet indices, all device pointers. frame1[b] = frames[triplets[samples[b]][0]] / 255, frame2 from column 1,
+ * target from column 2, each fp32 [n][1][H][W] and bit-identical to img.astype(float32) / 255.0. A sample index outside
+ * [0, n_triplets) or a triplet entry outside [0, n_frames) is never dereferenced: that sample's three outputs are NaN.
+ * FI_ERR_INVALID on NULL pointers, n < 1, H < 1, W < 1 or negative counts. */
+int fiGatherTripletsU8(const uint8_t* frames, int64_t n_frames, const int32_t* triplets, int64_t n_triplets,
+                       const int64_t* samples, int n, int H, int W, float* frame1, float* frame2, float* target,
+                       void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------
  * Training step (model/train.py:153-249; SURVEY.md §8f row 2): the kernels around the tensor-core convolutions.
