@@ -1197,6 +1197,34 @@ int fiNetReadActivation(fiNet* net, const char* name, float* out_host, int64_t c
     return FI_OK;
 }
 
+int fiNetCopyActivation(fiNet* net, const char* name, void* dst, void* dst_lo, int64_t capacity_elems, int* C, int* H,
+                        int* W, void* stream) {
+    if (!net || !name) return fail(FI_ERR_INVALID, "null argument");
+    if (!net->has_plan()) return fail(FI_ERR_INVALID, "no activation named '%s': no forward has run yet", name);
+    Plan& pl = net->plan();
+    auto it = pl.acts.find(name);
+    if (!pl.arena.p || it == pl.acts.end()) return fail(FI_ERR_INVALID, "no activation named '%s' in the current plan", name);
+    if (pl.reuse)
+        return fail(FI_ERR_STATE, "activation taps are unavailable: this plan's arena re-uses the memory of dead tensors "
+                                  "(FI_ARENA_REUSE=0 keeps every tensor)");
+    const Act& a = it->second;
+    if (C) *C = a.C;
+    if (H) *H = a.H;
+    if (W) *W = a.W;
+    if (!dst) return FI_OK;  // shape query
+    if (net->precise && !dst_lo) return fail(FI_ERR_INVALID, "fp32-grade mode: dst_lo is required for the lo half");
+    const int64_t n = static_cast<int64_t>(pl.last_n) * a.C * a.H * a.W;
+    if (capacity_elems < n) return fail(FI_ERR_INVALID, "buffer too small: need %lld elements", static_cast<long long>(n));
+    ON_DEVICE(net->device);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    CUDA_TRY(cudaMemcpyAsync(dst, static_cast<char*>(pl.arena.p) + a.off, static_cast<size_t>(n) * 2,
+                             cudaMemcpyDeviceToDevice, st));
+    if (net->precise)
+        CUDA_TRY(cudaMemcpyAsync(dst_lo, static_cast<char*>(pl.arena.p) + a.off_lo, static_cast<size_t>(n) * 2,
+                                 cudaMemcpyDeviceToDevice, st));
+    return FI_OK;
+}
+
 int fiConvGemm(const fiConvDesc* desc, void* stream) {
     if (!desc) return fail(FI_ERR_INVALID, "desc is null");
     int dev = 0;

@@ -70,6 +70,8 @@ _SIGNATURES = {
     "fiNetPlanStats": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_longlong), C.POINTER(C.c_size_t)]),
     "fiNetReadActivation": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int),
                                       C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "fiNetCopyActivation": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int),
+                                      C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_void_p]),
     "fiConvGemm": (C.c_int, [C.POINTER(ConvDesc), C.c_void_p]),
     "fiStemPackedK": (C.c_int, [C.c_int]),
     "fiStemPackWeights": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
@@ -309,6 +311,22 @@ class Net:
         check(lib().fiNetReadActivation(self._h, name.encode(), buf.data_ptr(), max_elems, C.byref(c), C.byref(h),
                                         C.byref(w)))
         return buf[: n * c.value * h.value * w.value].view(n, c.value, h.value, w.value).clone()
+
+    def activation(self, name, n):
+        """Activation `name` of the last forward (of n images, as read_activation) as a CUDA bf16 tensor [n, H, W, C]
+        in the library's own NHWC layout, copied on the device (fiNetCopyActivation) in stream order. In the fp32-grade
+        mode a pair (hi, lo) with value hi + lo. Refused under arena reuse, like read_activation."""
+        c, h, w = C.c_int(), C.c_int(), C.c_int()
+        with torch.cuda.device(self.device):
+            check(lib().fiNetCopyActivation(self._h, name.encode(), None, None, 0, C.byref(c), C.byref(h), C.byref(w),
+                                            current_stream()))
+            shape = (n, h.value, w.value, c.value)
+            hi = torch.empty(shape, dtype=torch.bfloat16, device=self.device)
+            lo = torch.empty(shape, dtype=torch.bfloat16, device=self.device) if self.precision == "fp32" else None
+            check(lib().fiNetCopyActivation(self._h, name.encode(), hi.data_ptr(),
+                                            lo.data_ptr() if lo is not None else None, hi.numel(), None, None, None,
+                                            current_stream()))
+        return (hi, lo) if lo is not None else hi
 
 
 # --------------------------------------------------------------------------------------------- single kernels

@@ -133,6 +133,14 @@ int fiNetPlanStats(fiNet* net, int* cached, long long* builds, size_t* arena_byt
 /* Debug tap: copy an intermediate activation (bf16 NHWC) of the last forward to the host as fp32 NCHW.
  * name in {inc, down1..down4, up1..up4 (block outputs), up1.up..up4.up (upsampled tensors)}. */
 int fiNetReadActivation(fiNet* net, const char* name, float* out_host, int64_t capacity, int* C, int* H, int* W);
+/* Device tap: the same activation as fiNetReadActivation (any tensor of the current plan: also pool1..pool4, the
+ * .mid tensors, and inc.mid where the stem is its own launch), copied device to device in its own layout, bf16 NHWC [n_last_forward, H, W, C], with cudaMemcpyAsync on
+ * `stream` (ordered after the forward enqueued on it). In the fp32-grade mode the lo half goes to dst_lo (required
+ * there, ignored otherwise); value = hi + lo. capacity_elems: bf16 elements each of dst and dst_lo can hold. dst NULL:
+ * only C, H, W are reported. Refuses a plan with arena reuse (the tensor may be overwritten) and a too-small buffer,
+ * like the host tap. */
+int fiNetCopyActivation(fiNet* net, const char* name, void* dst, void* dst_lo, int64_t capacity_elems, int* C, int* H,
+                        int* W, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------
  * Single layers (the same kernels the handle launches), for layer-level parity tests and reuse.
