@@ -158,10 +158,14 @@ struct fiNet {
         cudaEvent_t in_ready = nullptr, done = nullptr, out_ready = nullptr;
         uint64_t* pin_sad = nullptr;  // per-pair SAD of the batch (fiNetInterpolateClipHostU8Sad only)
         uint64_t* dev_sad = nullptr;
+        DevBuf pool;                  // fiNetInterpolateDyadicHostU8: every node of the group's bisection tree
+        void* pin_nodes = nullptr;    // ... and the requested nodes on their way to the host
+        size_t pin_nodes_bytes = 0;
     } clip[2];
     size_t clip_in_bytes = 0, clip_out_bytes = 0;
     int clip_sad_pairs = 0;  // capacity of pin_sad / dev_sad
     cudaStream_t clip_h2d = nullptr, clip_d2h = nullptr;
+    DevBuf dyadic_gather;    // in0 | in1 of one bisection forward: the parents of up to pairs_per_batch nodes
     // pinned staging for the host-buffer convenience call
     void* pin_in = nullptr;
     void* pin_out = nullptr;
@@ -690,6 +694,71 @@ struct DeviceGuard {
     DeviceGuard _device_guard(device); \
     if (_device_guard.rc) return _device_guard.rc
 
+// Copy streams, events and the double-buffered staging of the pipelined host-clip calls: per slot at least in_bytes of
+// pinned and device input, out_bytes of pinned and device output (0: none needed), and with `sad` B per-pair SAD values.
+// Buffers only grow: a reallocation keeps the larger of the held and the asked sizes.
+int clip_staging(fiNet* net, int B, size_t in_bytes, size_t out_bytes, bool sad) {
+    if (!net->clip_h2d) {
+        CUDA_TRY(cudaStreamCreateWithFlags(&net->clip_h2d, cudaStreamNonBlocking));
+        CUDA_TRY(cudaStreamCreateWithFlags(&net->clip_d2h, cudaStreamNonBlocking));
+        for (auto& c : net->clip) {
+            CUDA_TRY(cudaEventCreateWithFlags(&c.in_ready, cudaEventDisableTiming));
+            CUDA_TRY(cudaEventCreateWithFlags(&c.done, cudaEventDisableTiming));
+            CUDA_TRY(cudaEventCreateWithFlags(&c.out_ready, cudaEventDisableTiming));
+        }
+    }
+    if (net->clip_in_bytes < in_bytes || net->clip_out_bytes < out_bytes) {
+        in_bytes = std::max(in_bytes, net->clip_in_bytes);
+        out_bytes = std::max(out_bytes, net->clip_out_bytes);
+        CUDA_TRY(cudaDeviceSynchronize());
+        for (auto& c : net->clip) {
+            if (c.pin_in) cudaFreeHost(c.pin_in);
+            if (c.pin_out) cudaFreeHost(c.pin_out);
+            if (c.dev_in) cudaFree(c.dev_in);
+            if (c.dev_out) cudaFree(c.dev_out);
+            c.pin_in = c.pin_out = c.dev_in = c.dev_out = nullptr;
+        }
+        net->clip_in_bytes = net->clip_out_bytes = 0;
+        for (auto& c : net->clip) {
+            CUDA_TRY(cudaMallocHost(&c.pin_in, in_bytes));
+            CUDA_TRY(cudaMalloc(&c.dev_in, in_bytes));
+            if (out_bytes) {
+                CUDA_TRY(cudaMallocHost(&c.pin_out, out_bytes));
+                CUDA_TRY(cudaMalloc(&c.dev_out, out_bytes));
+            }
+        }
+        net->clip_in_bytes = in_bytes;
+        net->clip_out_bytes = out_bytes;
+    }
+    if (sad && net->clip_sad_pairs < B) {
+        CUDA_TRY(cudaDeviceSynchronize());
+        for (auto& c : net->clip) {
+            if (c.pin_sad) cudaFreeHost(c.pin_sad);
+            if (c.dev_sad) cudaFree(c.dev_sad);
+            c.pin_sad = c.dev_sad = nullptr;
+        }
+        net->clip_sad_pairs = 0;
+        for (auto& c : net->clip) {
+            CUDA_TRY(cudaMallocHost(reinterpret_cast<void**>(&c.pin_sad), B * sizeof(uint64_t)));
+            CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&c.dev_sad), B * sizeof(uint64_t)));
+        }
+        net->clip_sad_pairs = B;
+    }
+    return FI_OK;
+}
+
+// Planes of `n` planar u8 images of `channels` x H x W, `stride` bytes apart, starting at ptr.
+fiPlanes u8_planes(const void* ptr, int channels, int H, int W, int64_t stride) {
+    fiPlanes p;
+    p.ptr = ptr;
+    p.channels = channels;
+    p.px_stride = 1;
+    p.row_stride = W;
+    p.chan_stride = static_cast<int64_t>(H) * W;
+    p.batch_stride = stride;
+    return p;
+}
+
 }  // namespace
 
 extern "C" {
@@ -751,6 +820,7 @@ int fiNetDestroy(fiNet* net) {
         if (c.dev_out) cudaFree(c.dev_out);
         if (c.pin_sad) cudaFreeHost(c.pin_sad);
         if (c.dev_sad) cudaFree(c.dev_sad);
+        if (c.pin_nodes) cudaFreeHost(c.pin_nodes);
         if (c.in_ready) cudaEventDestroy(c.in_ready);
         if (c.done) cudaEventDestroy(c.done);
         if (c.out_ready) cudaEventDestroy(c.out_ready);
@@ -1031,48 +1101,7 @@ int fiNetInterpolateClipHostU8Sad(fiNet* net, const uint8_t* frames_host, int64_
     const size_t in_bytes = (B + 1) * frame_bytes, out_bytes = B * outf_bytes;
     if (frame_stride < static_cast<int64_t>(frame_bytes) || out_stride < static_cast<int64_t>(outf_bytes))
         return fail(FI_ERR_INVALID, "frame strides are smaller than a frame");
-    if (!net->clip_h2d) {
-        CUDA_TRY(cudaStreamCreateWithFlags(&net->clip_h2d, cudaStreamNonBlocking));
-        CUDA_TRY(cudaStreamCreateWithFlags(&net->clip_d2h, cudaStreamNonBlocking));
-        for (auto& c : net->clip) {
-            CUDA_TRY(cudaEventCreateWithFlags(&c.in_ready, cudaEventDisableTiming));
-            CUDA_TRY(cudaEventCreateWithFlags(&c.done, cudaEventDisableTiming));
-            CUDA_TRY(cudaEventCreateWithFlags(&c.out_ready, cudaEventDisableTiming));
-        }
-    }
-    if (net->clip_in_bytes < in_bytes || net->clip_out_bytes < out_bytes) {
-        CUDA_TRY(cudaDeviceSynchronize());
-        for (auto& c : net->clip) {
-            if (c.pin_in) cudaFreeHost(c.pin_in);
-            if (c.pin_out) cudaFreeHost(c.pin_out);
-            if (c.dev_in) cudaFree(c.dev_in);
-            if (c.dev_out) cudaFree(c.dev_out);
-            c.pin_in = c.pin_out = c.dev_in = c.dev_out = nullptr;
-        }
-        net->clip_in_bytes = net->clip_out_bytes = 0;
-        for (auto& c : net->clip) {
-            CUDA_TRY(cudaMallocHost(&c.pin_in, in_bytes));
-            CUDA_TRY(cudaMallocHost(&c.pin_out, out_bytes));
-            CUDA_TRY(cudaMalloc(&c.dev_in, in_bytes));
-            CUDA_TRY(cudaMalloc(&c.dev_out, out_bytes));
-        }
-        net->clip_in_bytes = in_bytes;
-        net->clip_out_bytes = out_bytes;
-    }
-    if (pair_sad_host && net->clip_sad_pairs < B) {
-        CUDA_TRY(cudaDeviceSynchronize());
-        for (auto& c : net->clip) {
-            if (c.pin_sad) cudaFreeHost(c.pin_sad);
-            if (c.dev_sad) cudaFree(c.dev_sad);
-            c.pin_sad = c.dev_sad = nullptr;
-        }
-        net->clip_sad_pairs = 0;
-        for (auto& c : net->clip) {
-            CUDA_TRY(cudaMallocHost(reinterpret_cast<void**>(&c.pin_sad), B * sizeof(uint64_t)));
-            CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&c.dev_sad), B * sizeof(uint64_t)));
-        }
-        net->clip_sad_pairs = B;
-    }
+    if ((rc = clip_staging(net, B, in_bytes, out_bytes, pair_sad_host != nullptr))) return rc;
     const int n_pairs = n_frames - 1;
     const int n_batches = (n_pairs + B - 1) / B;
     auto collect = [&](int b) -> int {  // wait for batch b's D2H and hand its frames to the caller
@@ -1108,15 +1137,9 @@ int fiNetInterpolateClipHostU8Sad(fiNet* net, const uint8_t* frames_host, int64_
         if (pair_sad_host)  // the batch's cnt+1 frames were just uploaded: the SAD reads them from L2, not the host
             KERNEL_TRY(fi::pair_sad_launch(static_cast<const uint8_t*>(c.dev_in), static_cast<int64_t>(frame_bytes),
                                            static_cast<int64_t>(frame_bytes), cnt + 1, c.dev_sad, st));
-        fiPlanes p0, p1;
-        p0.ptr = c.dev_in;
-        p0.channels = channels_per_frame;
-        p0.px_stride = 1;
-        p0.row_stride = W;
-        p0.chan_stride = static_cast<int64_t>(H) * W;
-        p0.batch_stride = p0.chan_stride * channels_per_frame;
-        p1 = p0;
-        p1.ptr = static_cast<const uint8_t*>(c.dev_in) + frame_bytes;
+        const fiPlanes p0 = u8_planes(c.dev_in, channels_per_frame, H, W, frame_bytes);
+        const fiPlanes p1 = u8_planes(static_cast<const uint8_t*>(c.dev_in) + frame_bytes, channels_per_frame, H, W,
+                                      frame_bytes);
         rc = fiNetForward(net, &p0, &p1, FI_IN_U8, nullptr, static_cast<uint8_t*>(c.dev_out), cnt, H, W, stream);
         if (rc) return rc;
         CUDA_TRY(cudaEventRecord(c.done, st));
@@ -1128,6 +1151,193 @@ int fiNetInterpolateClipHostU8Sad(fiNet* net, const uint8_t* frames_host, int64_
         if (b > 0 && (rc = collect(b - 1))) return rc;
     }
     return collect(n_batches - 1);
+}
+
+int fiNetInterpolateDyadicHostU8(fiNet* net, const uint8_t* frames_host, int64_t frame_stride, int n_frames,
+                                 int channels_per_frame, int H, int W, int depth, const int32_t* req_pair_host,
+                                 const int32_t* req_num_host, int n_req, uint8_t* out_host, int64_t out_stride,
+                                 int pairs_per_batch, void* stream, uint64_t* pair_sad_host, int64_t* n_forwards_host) {
+    if (!net) return fail(FI_ERR_INVALID, "net is null");
+    if (!frames_host) return fail(FI_ERR_INVALID, "frames_host is null");
+    if (n_req < 0) return fail(FI_ERR_INVALID, "n_req %d is negative", n_req);
+    if (n_req > 0 && (!req_pair_host || !req_num_host || !out_host))
+        return fail(FI_ERR_INVALID, "req_pair_host, req_num_host and out_host are required when n_req > 0");
+    if (2 * channels_per_frame != net->n_channels)
+        return fail(FI_ERR_INVALID, "2 x %d channels per frame != n_channels %d", channels_per_frame, net->n_channels);
+    if (net->n_classes != channels_per_frame)
+        return fail(FI_ERR_INVALID, "n_classes %d != channels_per_frame %d: bisection feeds each node back into the network",
+                    net->n_classes, channels_per_frame);
+    if (depth < 1 || depth > 6) return fail(FI_ERR_INVALID, "depth %d is outside 1..6", depth);
+    if (n_frames < 2) return fail(FI_ERR_INVALID, "n_frames %d: a clip needs at least two frames", n_frames);
+    if (H < 16 || W < 16) return fail(FI_ERR_INVALID, "input %dx%d is smaller than 16x16 (4 poolings)", H, W);
+    if (pairs_per_batch < 1) return fail(FI_ERR_INVALID, "pairs_per_batch %d < 1", pairs_per_batch);
+    const size_t fb = static_cast<size_t>(channels_per_frame) * H * W;  // a frame and a node have the same size
+    if (frame_stride < static_cast<int64_t>(fb)) return fail(FI_ERR_INVALID, "frame_stride is smaller than a frame");
+    if (n_req > 0 && out_stride < static_cast<int64_t>(fb)) return fail(FI_ERR_INVALID, "out_stride is smaller than a frame");
+    const int n_pairs = n_frames - 1, full = 1 << depth;
+    for (int j = 0; j < n_req; ++j) {
+        const int p = req_pair_host[j], v = req_num_host[j];
+        if (p < 0 || p >= n_pairs) return fail(FI_ERR_INVALID, "req_pair[%d] = %d is outside [0, %d)", j, p, n_pairs);
+        if (j > 0 && p < req_pair_host[j - 1])
+            return fail(FI_ERR_INVALID, "req_pair is not sorted: req_pair[%d] = %d < req_pair[%d] = %d", j, p, j - 1,
+                        req_pair_host[j - 1]);
+        if (v <= 0 || v >= full)
+            return fail(FI_ERR_INVALID, "req_num[%d] = %d is outside (0, 2^depth = %d)", j, v, full);
+    }
+    if (!net->loaded) return fail(FI_ERR_STATE, "fiNetLoadWeights has not been called");
+    ON_DEVICE(net->device);
+    int rc = FI_OK;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int B = pairs_per_batch;
+
+    // A node of local pair q is keyed (q << depth) | v with v in (0, 2^depth) its position in units of 2^-depth; v = 0
+    // and v = 2^depth are the uploaded frames q and q+1. Marks the closure of requests [r0, r1) of the group starting at
+    // pair `first`: a node at level l (v an odd multiple of 2^(depth-l)) needs its parents v -/+ 2^(depth-l).
+    std::vector<uint8_t> need;
+    std::vector<int> stack;
+    auto closure = [&](int first, int cnt, int r0, int r1) {
+        need.assign(static_cast<size_t>(cnt) << depth, 0);
+        int nodes = 0;
+        for (int r = r0; r < r1; ++r) stack.push_back(((req_pair_host[r] - first) << depth) | req_num_host[r]);
+        while (!stack.empty()) {
+            const int key = stack.back(), v = key & (full - 1), low = v & -v;
+            stack.pop_back();
+            if (need[key]) continue;
+            need[key] = 1;
+            ++nodes;
+            if (v - low > 0) stack.push_back(key - low);
+            if (v + low < full) stack.push_back(key + low);
+        }
+        return nodes;
+    };
+    struct Group {
+        int first, cnt, r0, r1;
+    };
+    std::vector<Group> groups;  // groups of B pairs that have requests (all of them when the SAD is asked for)
+    size_t max_nodes = 0, max_req = 0;
+    for (int first = 0, r = 0; first < n_pairs; first += B) {
+        Group g{first, std::min(B, n_pairs - first), r, r};
+        while (r < n_req && req_pair_host[r] < first + g.cnt) ++r;
+        g.r1 = r;
+        if (g.r0 == g.r1 && !pair_sad_host) continue;
+        groups.push_back(g);
+        max_nodes = std::max(max_nodes, static_cast<size_t>(closure(g.first, g.cnt, g.r0, g.r1)));
+        max_req = std::max(max_req, static_cast<size_t>(g.r1 - g.r0));
+    }
+    if (groups.empty()) {
+        if (n_forwards_host) *n_forwards_host = 0;
+        return FI_OK;
+    }
+    // the clip call's input staging and SAD buffers; its output staging is not used (nodes go through pin_nodes)
+    if ((rc = clip_staging(net, B, (B + 1) * fb, 0, pair_sad_host != nullptr))) return rc;
+    const size_t gather_bytes = max_nodes > 0 ? 2 * B * fb : 0, pool_bytes = max_nodes * fb, nodes_bytes = max_req * fb;
+    bool grow = net->dyadic_gather.bytes < gather_bytes;
+    for (auto& c : net->clip) grow = grow || c.pool.bytes < pool_bytes || c.pin_nodes_bytes < nodes_bytes;
+    if (grow) {
+        CUDA_TRY(cudaDeviceSynchronize());
+        auto grow_dev = [](DevBuf& d, size_t bytes) {
+            if (d.bytes >= bytes) return cudaSuccess;
+            d.release();
+            const cudaError_t e = cudaMalloc(&d.p, bytes);
+            if (e == cudaSuccess) d.bytes = bytes;
+            return e;
+        };
+        CUDA_TRY(grow_dev(net->dyadic_gather, gather_bytes));
+        for (auto& c : net->clip) {
+            CUDA_TRY(grow_dev(c.pool, pool_bytes));
+            if (c.pin_nodes_bytes < nodes_bytes) {
+                if (c.pin_nodes) cudaFreeHost(c.pin_nodes);
+                c.pin_nodes = nullptr;
+                c.pin_nodes_bytes = 0;
+                CUDA_TRY(cudaMallocHost(&c.pin_nodes, nodes_bytes));
+                c.pin_nodes_bytes = nodes_bytes;
+            }
+        }
+    }
+    // one plan of the clip call's capacity serves every level's batches (<= B images each)
+    if (max_nodes > 0 && (rc = build_plan(net, B, H, W))) return rc;
+
+    auto collect = [&](size_t b) -> int {  // wait for group b's D2H and hand its requested nodes to the caller
+        const Group& g = groups[b];
+        fiNet::ClipSlot& c = net->clip[b & 1];
+        CUDA_TRY(cudaEventSynchronize(c.out_ready));
+        for (int r = g.r0; r < g.r1; ++r)
+            memcpy(out_host + static_cast<int64_t>(r) * out_stride, static_cast<const char*>(c.pin_nodes) + (r - g.r0) * fb,
+                   fb);
+        if (pair_sad_host) memcpy(pair_sad_host + g.first, c.pin_sad, g.cnt * sizeof(uint64_t));
+        return FI_OK;
+    };
+    uint8_t* const in0 = static_cast<uint8_t*>(net->dyadic_gather.p);
+    uint8_t* const in1 = in0 + B * fb;
+    const fiPlanes p0 = u8_planes(in0, channels_per_frame, H, W, fb);
+    const fiPlanes p1 = u8_planes(in1, channels_per_frame, H, W, fb);
+    std::vector<int> slot, todo;  // pool index of each needed node; the nodes of one level
+    int64_t forwards = 0;
+    for (size_t b = 0; b < groups.size(); ++b) {
+        const Group& g = groups[b];
+        fiNet::ClipSlot& c = net->clip[b & 1];
+        // slot reuse is safe: group b-2 was collected (host-synchronised) in iteration b-1
+        if (frame_stride == static_cast<int64_t>(fb)) {
+            memcpy(c.pin_in, frames_host + static_cast<size_t>(g.first) * fb, (g.cnt + 1) * fb);
+        } else {
+            for (int i = 0; i <= g.cnt; ++i)
+                memcpy(static_cast<char*>(c.pin_in) + i * fb, frames_host + static_cast<int64_t>(g.first + i) * frame_stride,
+                       fb);
+        }
+        CUDA_TRY(cudaMemcpyAsync(c.dev_in, c.pin_in, (g.cnt + 1) * fb, cudaMemcpyHostToDevice, net->clip_h2d));
+        CUDA_TRY(cudaEventRecord(c.in_ready, net->clip_h2d));
+        CUDA_TRY(cudaStreamWaitEvent(st, c.in_ready, 0));
+        if (pair_sad_host)
+            KERNEL_TRY(fi::pair_sad_launch(static_cast<const uint8_t*>(c.dev_in), static_cast<int64_t>(fb),
+                                           static_cast<int64_t>(fb), g.cnt + 1, c.dev_sad, st));
+        closure(g.first, g.cnt, g.r0, g.r1);
+        slot.assign(need.size(), -1);
+        const uint8_t* frames_dev = static_cast<const uint8_t*>(c.dev_in);
+        uint8_t* pool = static_cast<uint8_t*>(c.pool.p);
+        auto node = [&](int q, int v) -> const uint8_t* {
+            if (v == 0) return frames_dev + q * fb;
+            if (v == full) return frames_dev + (q + 1) * fb;
+            return pool + slot[(q << depth) | v] * fb;
+        };
+        int next = 0;  // pool slots in evaluation order, so that each forward's outputs are contiguous
+        for (int level = 1; level <= depth; ++level) {
+            const int half = 1 << (depth - level);  // a level-l node sits half-way between its parents
+            todo.clear();
+            for (int q = 0; q < g.cnt; ++q)
+                for (int v = half; v < full; v += 2 * half)
+                    if (need[(q << depth) | v]) todo.push_back((q << depth) | v);
+            for (size_t k0 = 0; k0 < todo.size(); k0 += B) {
+                const int nb = static_cast<int>(std::min(todo.size() - k0, static_cast<size_t>(B)));
+                for (int k = 0; k < nb; ++k) {
+                    const int key = todo[k0 + k], q = key >> depth, v = key & (full - 1);
+                    CUDA_TRY(cudaMemcpyAsync(in0 + k * fb, node(q, v - half), fb, cudaMemcpyDeviceToDevice, st));
+                    CUDA_TRY(cudaMemcpyAsync(in1 + k * fb, node(q, v + half), fb, cudaMemcpyDeviceToDevice, st));
+                    slot[key] = next + k;
+                }
+                rc = fiNetForward(net, &p0, &p1, FI_IN_U8, nullptr, pool + next * fb, nb, H, W, stream);
+                if (rc) return rc;
+                next += nb;
+            }
+        }
+        forwards += next;
+        CUDA_TRY(cudaEventRecord(c.done, st));
+        CUDA_TRY(cudaStreamWaitEvent(net->clip_d2h, c.done, 0));
+        for (int r = g.r0; r < g.r1;) {  // requested nodes, runs of consecutive pool slots in one copy
+            const int s = slot[((req_pair_host[r] - g.first) << depth) | req_num_host[r]];
+            int e = r + 1;
+            while (e < g.r1 && slot[((req_pair_host[e] - g.first) << depth) | req_num_host[e]] == s + (e - r)) ++e;
+            CUDA_TRY(cudaMemcpyAsync(static_cast<char*>(c.pin_nodes) + (r - g.r0) * fb, pool + s * fb, (e - r) * fb,
+                                     cudaMemcpyDeviceToHost, net->clip_d2h));
+            r = e;
+        }
+        if (pair_sad_host)
+            CUDA_TRY(cudaMemcpyAsync(c.pin_sad, c.dev_sad, g.cnt * sizeof(uint64_t), cudaMemcpyDeviceToHost, net->clip_d2h));
+        CUDA_TRY(cudaEventRecord(c.out_ready, net->clip_d2h));
+        if (b > 0 && (rc = collect(b - 1))) return rc;
+    }
+    if ((rc = collect(groups.size() - 1))) return rc;
+    if (n_forwards_host) *n_forwards_host = forwards;
+    return FI_OK;
 }
 
 int fiNetForwardCost(fiNet* net, int N, int H, int W, double* flops, int* launches) {

@@ -17,11 +17,27 @@ def _scene_threshold(text):
         raise argparse.ArgumentTypeError(str(e)) from None
 
 
+def _frame_rate(text):
+    from model.timing import parse_rate
+    try:
+        return parse_rate(text)
+    except ValueError as e:
+        raise argparse.ArgumentTypeError(str(e)) from None
+
+
+class _TypedFactor(argparse.Action):
+    """Stores --factor and notes that it was given; argparse calls it for abbreviations (--fac 3) as well."""
+
+    def __call__(self, parser, namespace, values, option_string=None):
+        setattr(namespace, self.dest, values)
+        namespace.factor_typed = True
+
+
 def build_parser():
     p = argparse.ArgumentParser(description="AI-Based Frame Interpolation (B200-native path)")
     sub = p.add_subparsers(dest="command", help="Available commands")
-    # flags, defaults and required-ness as reference main.py:40-72; --frame-cache, --gpus and --scene-threshold are the
-    # only additions
+    # flags, defaults and required-ness as reference main.py:40-72; --frame-cache, --gpus, --scene-threshold and --fps
+    # are the only additions
     t = sub.add_parser("train", help="Train the frame interpolation model")
     t.add_argument("--data-dir", required=True, help="Directory containing training data")
     t.add_argument("--epochs", type=int, default=100, help="Number of training epochs")
@@ -39,7 +55,7 @@ def build_parser():
     v = sub.add_parser("video", help="Interpolate frames in a video")
     v.add_argument("--input", required=True, help="Input video path")
     v.add_argument("--output", required=True, help="Output video path")
-    v.add_argument("--factor", type=int, default=2, help="Interpolation factor")
+    v.add_argument("--factor", type=int, default=2, action=_TypedFactor, help="Interpolation factor")
     v.add_argument("--model", default="best_model.pth", help="Path to trained model")
     v.add_argument("--device", default="auto", help="Device to use (cuda/auto)")
     v.add_argument("--gpus", type=int, default=None,
@@ -47,6 +63,8 @@ def build_parser():
     v.add_argument("--scene-threshold", type=_scene_threshold, default=None, metavar="T",
                    help="Detect scene cuts (score in (0, 100], try 10) and repeat the frame before a cut instead of "
                         "blending two shots (default: off)")
+    v.add_argument("--fps", type=_frame_rate, default=None, metavar="RATE",
+                   help="Convert to this output frame rate, e.g. 60, 59.94 or 60000/1001 (instead of --factor)")
     s = sub.add_parser("serve", help="Start the web API server")
     s.add_argument("--host", default="0.0.0.0", help="Host to bind to")
     s.add_argument("--port", type=int, default=8000, help="Port to bind to")
@@ -57,7 +75,10 @@ def build_parser():
 
 
 def main(argv=None):
-    args = build_parser().parse_args(argv)
+    parser = build_parser()
+    args = parser.parse_args(argv)
+    if args.command == "video" and args.fps is not None and getattr(args, "factor_typed", False):
+        parser.error("video: --fps and --factor exclude each other (--fps sets the output rate)")
     if not args.command:
         build_parser().print_help()
         return 0
@@ -93,8 +114,12 @@ def main(argv=None):
         elif args.command == "video":
             from model.inference import FrameInterpolator
             interpolator = FrameInterpolator(args.model, device, gpus=args.gpus, scene_threshold=args.scene_threshold)
-            print(f"Interpolating video: {args.input}\nOutput: {args.output}\nFactor: {args.factor}x")
-            n = interpolator.interpolate_video(args.input, args.output, args.factor)
+            if args.fps is None:
+                print(f"Interpolating video: {args.input}\nOutput: {args.output}\nFactor: {args.factor}x")
+                n = interpolator.interpolate_video(args.input, args.output, args.factor)
+            else:
+                print(f"Interpolating video: {args.input}\nOutput: {args.output}\nFrame rate: {args.fps} fps")
+                n = interpolator.interpolate_video(args.input, args.output, fps=args.fps)
             print(f"Video interpolation completed! ({n} frames written)")
             if args.scene_threshold is not None:
                 print(f"Scene cuts found: {len(interpolator.last_scene_cuts)} (threshold {args.scene_threshold:g})")

@@ -66,6 +66,9 @@ _SIGNATURES = {
                                                     C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "fiNetInterpolateClipHostU8Sad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p,
                                                 C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "fiNetInterpolateDyadicHostU8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int,
+                                               C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_int,
+                                               C.c_void_p, C.c_void_p, C.POINTER(C.c_int64)]),
     "fiNetForwardCost": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_int)]),
     "fiNetPlanStats": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_longlong), C.POINTER(C.c_size_t)]),
     "fiNetReadActivation": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int),
@@ -168,6 +171,40 @@ def require_cuda(device) -> torch.device:
     return device
 
 
+def _frame_contiguous(a):
+    """Every frame a[i] of a [F,C,H,W] array is C-contiguous (strides of length-1 axes do not matter)."""
+    want = (a.shape[2] * a.shape[3], a.shape[3], 1)
+    inner = all(a.shape[k + 1] == 1 or a.strides[k + 1] == want[k] for k in range(3))
+    return inner and (a.shape[0] == 1 or a.strides[0] >= a.shape[1] * a.shape[2] * a.shape[3])
+
+
+def _host_clip(frames):
+    """A uint8 [F,C,H,W] host clip whose frames are each contiguous (copied only when they are not)."""
+    import numpy as np
+    frames = np.asarray(frames)
+    if frames.dtype != np.uint8 or frames.ndim != 4:
+        raise FiError("frames must be a uint8 array [F,C,H,W]")
+    return frames if _frame_contiguous(frames) else np.ascontiguousarray(frames)
+
+
+def _host_out(out, n, c, h, w):
+    """`out`, checked to be a writable uint8 [n,c,h,w] host array with contiguous frames, or a new one."""
+    import numpy as np
+    if out is None:
+        return np.empty((n, c, h, w), dtype=np.uint8)
+    if (out.dtype != np.uint8 or out.shape != (n, c, h, w) or not out.flags.writeable
+            or (n > 0 and not _frame_contiguous(out))):
+        raise FiError(f"out must be a writable uint8 array of shape {(n, c, h, w)} whose frames are contiguous")
+    return out
+
+
+def _check_sad_out(sad_out, f):
+    import numpy as np
+    if sad_out is not None and (sad_out.dtype != np.uint64 or sad_out.shape != (f - 1,) or not sad_out.flags.writeable
+                                or not sad_out.flags.c_contiguous):
+        raise FiError(f"sad_out must be a writable contiguous uint64 array of shape {(f - 1,)}")
+
+
 class Net:
     """Owner of one fiNet handle (weights + activation arena on one GPU)."""
 
@@ -251,34 +288,45 @@ class Net:
         itself contiguous), e.g. `seq[0::2]` in and `seq[1::2]` out of one interleaved sequence. `sad_out`: optional
         contiguous uint64 [F-1] array that receives the scene-cut statistic of every pair, sum |f[i+1] - f[i]| over
         all C*H*W bytes, computed on the GPU from the uploaded frames (fiNetInterpolateClipHostU8Sad)."""
-        import numpy as np
-        frames = np.asarray(frames)
-        if frames.dtype != np.uint8 or frames.ndim != 4:
-            raise FiError("frames must be a uint8 array [F,C,H,W]")
+        frames = _host_clip(frames)
         f, c, h, w = frames.shape
-
-        def frame_contiguous(a):   # every frame a[i] is C-contiguous (strides of length-1 axes do not matter)
-            want = (a.shape[2] * a.shape[3], a.shape[3], 1)
-            inner = all(a.shape[k + 1] == 1 or a.strides[k + 1] == want[k] for k in range(3))
-            return inner and (a.shape[0] == 1 or a.strides[0] >= a.shape[1] * a.shape[2] * a.shape[3])
-
-        if not frame_contiguous(frames):
-            frames = np.ascontiguousarray(frames)
-        if out is None:
-            out = np.empty((f - 1, self.n_classes, h, w), dtype=np.uint8)
-        elif (out.dtype != np.uint8 or out.shape != (f - 1, self.n_classes, h, w) or not out.flags.writeable
-              or (f > 1 and not frame_contiguous(out))):
-            raise FiError(f"out must be a writable uint8 array of shape {(f - 1, self.n_classes, h, w)} whose frames "
-                          "are contiguous")
-        if sad_out is not None and (sad_out.dtype != np.uint64 or sad_out.shape != (f - 1,) or not sad_out.flags.writeable
-                                    or not sad_out.flags.c_contiguous):
-            raise FiError(f"sad_out must be a writable contiguous uint64 array of shape {(f - 1,)}")
+        out = _host_out(out, f - 1, self.n_classes, h, w)
+        _check_sad_out(sad_out, f)
         with torch.cuda.device(self.device):
             check(lib().fiNetInterpolateClipHostU8Sad(self._h, frames.ctypes.data, frames.strides[0], f, c,
                                                       out.ctypes.data, out.strides[0] if f > 1 else 0, h, w,
                                                       pairs_per_batch, current_stream(),
                                                       sad_out.ctypes.data if sad_out is not None else None))
         return out
+
+    def interpolate_dyadic_host_u8(self, frames, pairs, nums, depth, pairs_per_batch=4, out=None, sad_out=None):
+        """Frames at dyadic times between the frames of a clip, by recursive bisection on the device
+        (fiNetInterpolateDyadicHostU8). frames: numpy uint8 [F,C,H,W] host clip (strided along the frame axis like
+        interpolate_clip_host_u8) with C == n_classes. Request j is node (pairs[j], nums[j] / 2**depth): pairs sorted,
+        0 < nums[j] < 2**depth. Returns (out, n_forwards): out uint8 [len(pairs),C,H,W] (optional preallocated, frames
+        contiguous) and the number of images the network forwarded. sad_out: optional uint64 [F-1] that receives every
+        pair's SAD, as in interpolate_clip_host_u8."""
+        import numpy as np
+        frames = _host_clip(frames)
+        f, c, h, w = frames.shape
+        pairs = np.asarray(pairs)
+        nums = np.asarray(nums)
+        if pairs.ndim != 1 or nums.shape != pairs.shape or not (np.issubdtype(pairs.dtype, np.integer)
+                                                               and np.issubdtype(nums.dtype, np.integer)):
+            raise FiError("pairs and nums must be integer arrays of the same length")
+        pairs = np.ascontiguousarray(pairs, dtype=np.int32)
+        nums = np.ascontiguousarray(nums, dtype=np.int32)
+        out = _host_out(out, len(pairs), self.n_classes, h, w)
+        _check_sad_out(sad_out, f)
+        forwards = C.c_int64(0)
+        with torch.cuda.device(self.device):
+            check(lib().fiNetInterpolateDyadicHostU8(self._h, frames.ctypes.data, frames.strides[0], f, c, h, w,
+                                                     int(depth), pairs.ctypes.data, nums.ctypes.data, len(pairs),
+                                                     out.ctypes.data, out.strides[0] if len(pairs) else 0,
+                                                     int(pairs_per_batch), current_stream(),
+                                                     sad_out.ctypes.data if sad_out is not None else None,
+                                                     C.byref(forwards)))
+        return out, forwards.value
 
     def set_profiling(self, on):
         check(lib().fiNetSetProfiling(self._h, int(bool(on))))

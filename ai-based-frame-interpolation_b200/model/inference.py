@@ -9,6 +9,7 @@ from __future__ import annotations
 import argparse
 import os
 import sys
+from fractions import Fraction
 
 import cv2
 import numpy as np
@@ -18,11 +19,13 @@ try:
     from . import _engine as _E
     from .multigpu import GpuPool
     from .scene import check_threshold, scene_cuts, scene_scores
+    from .timing import MAX_DEPTH, depth_for, output_window, parse_rate, position, snap, video_rate
     from .unet import FrameInterpolationUNet, UNet
 except ImportError:  # `python model/inference.py` / model/ on sys.path, like the reference's scripts
     import _engine as _E
     from multigpu import GpuPool
     from scene import check_threshold, scene_cuts, scene_scores
+    from timing import MAX_DEPTH, depth_for, output_window, parse_rate, position, snap, video_rate
     from unet import FrameInterpolationUNet, UNet
 
 
@@ -270,24 +273,7 @@ class FrameInterpolator:
         elif out.shape != (arr.shape[0] - 1,) + arr.shape[1:] or out.dtype != np.uint8:
             raise ValueError("out must be a uint8 array with one frame less than the clip")
         sad = np.zeros(arr.shape[0] - 1, dtype=np.uint64) if detect else None
-        if arr.ndim == 3:                                   # grey frames: may be strided along the frame axis
-            if self.n_channels != 2:
-                raise _E.FiError(f"model expects {self.n_channels} input channels, frames are grey")
-            self._clip_call(arr[:, None], out[:, None], sad)
-        elif self.n_channels == 2:                          # grey model: every colour plane is its own clip
-            plane = np.empty(out.shape[:3], dtype=np.uint8)
-            plane_sad = np.empty_like(sad) if detect else None
-            for k in range(arr.shape[3]):
-                self._clip_call(np.ascontiguousarray(arr[..., k])[:, None], plane[:, None], plane_sad)
-                out[..., k] = plane
-                if detect:
-                    sad += plane_sad                        # the SAD of a BGR pair is that of its three planes
-        elif self.n_channels == 2 * arr.shape[3]:           # colour model: planar frames
-            mids = np.empty((out.shape[0], arr.shape[3]) + out.shape[1:3], dtype=np.uint8)
-            self._clip_call(np.ascontiguousarray(arr.transpose(0, 3, 1, 2)), mids, sad)
-            out[...] = mids.transpose(0, 2, 3, 1)
-        else:
-            raise _E.FiError(f"model expects {self.n_channels} input channels, frames have {arr.shape[3]} per frame")
+        self._planar(self._clip_call, arr, out, sad)
         if not detect:
             return out, None, prev_mafd
         scores, last_mafd = scene_scores(sad, arr[0].size, prev_mafd)
@@ -295,6 +281,91 @@ class FrameInterpolator:
         for i in cuts:
             out[i] = arr[i]
         return out, cuts, last_mafd
+
+    def _planar(self, call, arr, out, sad):
+        """Runs call(frames [F,C,H,W], out [N,n_classes,H,W], sad) on the clip arr ([F,H,W] grey or [F,H,W,C]) in the
+        layout the model takes, with out [N, ...frame shape]: grey frames as they are (may be strided along the frame
+        axis), a grey model on colour frames once per plane, a colour model on planar frames. sad: None or uint64 [F-1]
+        zeros that receive each pair's SAD (summed over the planes)."""
+        if arr.ndim == 3:
+            if self.n_channels != 2:
+                raise _E.FiError(f"model expects {self.n_channels} input channels, frames are grey")
+            call(arr[:, None], out[:, None], sad)
+        elif self.n_channels == 2:                          # grey model: every colour plane is its own clip
+            plane = np.empty(out.shape[:3], dtype=np.uint8)
+            plane_sad = np.empty_like(sad) if sad is not None else None
+            for k in range(arr.shape[3]):
+                call(np.ascontiguousarray(arr[..., k])[:, None], plane[:, None], plane_sad)
+                out[..., k] = plane
+                if sad is not None:
+                    sad += plane_sad                        # the SAD of a BGR pair is that of its three planes
+        elif self.n_channels == 2 * arr.shape[3]:           # colour model: planar frames
+            mids = np.empty((out.shape[0], arr.shape[3]) + out.shape[1:3], dtype=np.uint8)
+            call(np.ascontiguousarray(arr.transpose(0, 3, 1, 2)), mids, sad)
+            out[...] = mids.transpose(0, 2, 3, 1)
+        else:
+            raise _E.FiError(f"model expects {self.n_channels} input channels, frames have {arr.shape[3]} per frame")
+
+    def interpolate_at(self, frames, positions, depth=3):
+        """Frames at arbitrary times of a clip: frames [F,H,W] grey or [F,H,W,3] BGR uint8, positions in source-frame
+        units in [0, F-1], any order (floats or Fractions) -> [len(positions), ...frame shape]. Each position is
+        snapped to the nearest node of a depth-`depth` bisection tree (model/timing.py; at most 2^-(depth+1) of a frame
+        interval away): a source frame is copied, any other node is computed on the GPU by recursive bisection
+        (fiNetInterpolateDyadicHostU8), each needed node once. With `scene_threshold` set, every output inside a cut
+        pair i is a copy of frames[i] and `last_scene_cuts` lists the cut pairs."""
+        out, cuts, _ = self._at(frames, positions, depth, 0.0)
+        if cuts is not None:
+            self.last_scene_cuts = cuts
+        return out
+
+    def _at(self, frames, positions, depth, prev_mafd):
+        """interpolate_at with the scene state of `_clip`: returns (frames, cuts or None, last mafd)."""
+        arr = np.asarray(frames)
+        if arr.dtype != np.uint8 or arr.ndim not in (3, 4) or arr.shape[0] < 1:
+            raise ValueError("expected a uint8 clip [F,H,W] or [F,H,W,C] with at least one frame")
+        if not 1 <= depth <= MAX_DEPTH:
+            raise ValueError(f"depth must be in 1..{MAX_DEPTH}, got {depth!r}")
+        n_src = arr.shape[0]
+        snapped = []
+        for p in positions:
+            p = Fraction(p)
+            if not 0 <= p <= n_src - 1:
+                raise ValueError(f"position {p} is outside [0, {n_src - 1}]")
+            snapped.append((p,) + snap(p, depth))
+        full = 1 << depth
+        nodes = sorted({(i, num) for _, i, num in snapped if 0 < num < full})
+        result = np.empty((len(snapped),) + arr.shape[1:], dtype=np.uint8)
+        detect = self.scene_threshold is not None and n_src >= 2
+        sad = np.zeros(n_src - 1, dtype=np.uint64) if detect else None
+        computed = np.empty((len(nodes),) + arr.shape[1:], dtype=np.uint8)
+        if nodes or detect:
+            pairs = np.array([i for i, _ in nodes], dtype=np.int32)
+            nums = np.array([num for _, num in nodes], dtype=np.int32)
+            self._planar(lambda fr, out, s: self._dyadic_call(fr, pairs, nums, depth, out, s), arr, computed, sad)
+        cuts, last_mafd = None, prev_mafd
+        if detect:
+            scores, last_mafd = scene_scores(sad, arr[0].size, prev_mafd)
+            cuts = scene_cuts(scores, self.scene_threshold)
+        elif self.scene_threshold is not None:
+            cuts = []
+        cut = set(cuts or ())
+        row = {node: j for j, node in enumerate(nodes)}
+        for k, (p, i, num) in enumerate(snapped):
+            if i in cut and p > i:                          # inside a cut pair: repeat the frame before the cut
+                result[k] = arr[i]
+            elif num == 0 or num == full:
+                result[k] = arr[i if num == 0 else i + 1]
+            else:
+                result[k] = computed[row[(i, num)]]
+        return result, cuts, last_mafd
+
+    def _dyadic_call(self, frames, pairs, nums, depth, out, sad):
+        """[F,C,H,W] u8 host clip -> the bisection nodes (pairs[j], nums[j] / 2^depth) in out[j]: one GPU = the library
+        call, several GPUs = contiguous pair ranges, one per GPU (as `_clip_call`)."""
+        if self._single_device:
+            return self.model._engine(self.device).interpolate_dyadic_host_u8(frames, pairs, nums, depth,
+                                                                              self.pairs_per_batch, out=out, sad_out=sad)
+        return self._gpu_pool().clip_dyadic(frames, pairs, nums, depth, self.pairs_per_batch, out, sad_out=sad)
 
     def interpolate_sequence(self, frames, factor=2, out=None):
         """factor-1 new frames between every consecutive pair. factor = 2^k: recursive bisection (every new frame is
@@ -354,19 +425,33 @@ class FrameInterpolator:
             out += [f] + [m] * (factor - 1)
         return out + [frames[-1]], cuts, last_mafd
 
-    def interpolate_video(self, input_path, output_path, factor=2, chunk=64):
+    def interpolate_video(self, input_path, output_path, factor=2, chunk=64, fps=None):
         """Read `input_path` with cv2, write `output_path` (mp4v) at factor x the frame rate. Three stages run
         concurrently — a decoder thread, the GPU stage (this thread) and an encoder thread — joined by bounded queues,
         so decode / encode (cv2 releases the GIL) overlap the forwards of the neighbouring chunks. With
         `scene_threshold` set, the scene state crosses chunk edges and `last_scene_cuts` numbers the cut pairs of the
-        input video (pair i = frames i, i+1), so the cuts found do not depend on `chunk` or on the number of GPUs."""
+        input video (pair i = frames i, i+1), so the cuts found do not depend on `chunk` or on the number of GPUs.
+
+        fps: convert to this output rate instead (a number, or text like "59.94" or "60000/1001"; `factor` is then
+        unused). Output k shows source position k * src / fps, snapped to the nearest bisection node as model/timing.py
+        states, so the result depends neither on `chunk` nor on the number of GPUs."""
         import queue
         import threading
+        rate = None if fps is None else parse_rate(fps)
         cap = cv2.VideoCapture(input_path)
         if not cap.isOpened():
             raise FileNotFoundError(f"could not open video {input_path}")
         chunk = chunk * len(self.devices)                   # every GPU gets `chunk` pairs of each decoded chunk
-        fps = cap.get(cv2.CAP_PROP_FPS) or 30.0
+        src_fps = cap.get(cv2.CAP_PROP_FPS)
+        fps = src_fps or 30.0
+        if rate is not None:
+            src_rate = video_rate(src_fps)
+            try:
+                depth = depth_for(src_rate, rate)
+            except ValueError:
+                cap.release()
+                raise
+        out_fps = fps * factor if rate is None else float(rate)
         decoded, encoded = queue.Queue(maxsize=2), queue.Queue(maxsize=2)
         failure, written = [], [0]
 
@@ -397,7 +482,7 @@ class FrameInterpolator:
                         continue        # keep draining so the producer never blocks
                     if writer is None:
                         h, w = seq[0].shape[:2]
-                        writer = cv2.VideoWriter(output_path, cv2.VideoWriter_fourcc(*"mp4v"), fps * factor, (w, h), True)
+                        writer = cv2.VideoWriter(output_path, cv2.VideoWriter_fourcc(*"mp4v"), out_fps, (w, h), True)
                         if not writer.isOpened():
                             raise RuntimeError(f"could not open video writer for {output_path}")
                     for f in seq:
@@ -435,7 +520,16 @@ class FrameInterpolator:
             while not failure:
                 new = decoded.get()
                 frames = new if prev is None else [prev] + new
-                if len(frames) >= 2:
+                if rate is not None:
+                    if frames:          # the outputs inside this chunk's pairs (and at the last frame of the video)
+                        ks = output_window(src_rate, rate, first_pair, len(frames) - 1, end=len(new) < chunk)
+                        seq, chunk_cuts, prev_mafd = self._at(
+                            np.stack(frames), [position(k, src_rate, rate) - first_pair for k in ks], depth, prev_mafd)
+                        cuts += [first_pair + i for i in chunk_cuts or ()]
+                        first_pair += len(frames) - 1
+                        if len(seq):
+                            encoded.put(seq)
+                elif len(frames) >= 2:
                     seq, chunk_cuts, prev_mafd = self._sequence(frames, factor, result_buffer(len(frames), frames[0].shape),
                                                                 prev_mafd)
                     cuts += [first_pair + i for i in chunk_cuts or ()]

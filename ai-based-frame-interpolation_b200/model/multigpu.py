@@ -17,6 +17,8 @@ from __future__ import annotations
 
 import threading
 
+import numpy as np
+
 try:
     from .sharding import shard_pairs
 except ImportError:  # model/ on sys.path, like the reference's scripts
@@ -25,7 +27,8 @@ except ImportError:  # model/ on sys.path, like the reference's scripts
 
 class GpuPool:
     """`runners`: one object per GPU with `.interpolate_clip_host_u8(frames, pairs_per_batch, out=..., sad_out=...)`
-    (an `_engine.Net`, or a stand-in in the CPU tests of the scheduling logic)."""
+    and, for clip_dyadic, `.interpolate_dyadic_host_u8(frames, pairs, nums, depth, pairs_per_batch, out=...,
+    sad_out=...)` (an `_engine.Net`, or a stand-in in the CPU tests of the scheduling logic)."""
 
     def __init__(self, runners):
         if not runners:
@@ -81,7 +84,48 @@ class GpuPool:
         n_frames = frames.shape[0]
         if n_frames < 2:
             return out
-        pending = [(0, n_frames - 1)]       # ranges of pairs still to compute: (first pair, count)
+
+        def job(runner, first, n):
+            extra = {} if sad_out is None else {"sad_out": sad_out[first:first + n]}
+            runner.interpolate_clip_host_u8(frames[first:first + n + 1], pairs_per_batch, out=out[first:first + n],
+                                            **extra)
+
+        self._run_ranges(n_frames - 1, job)
+        return out
+
+    def clip_dyadic(self, frames, pairs, nums, depth, pairs_per_batch, out, sad_out=None):
+        """Bisection nodes (`_engine.Net.interpolate_dyadic_host_u8`) of a clip sharded like clip_midpoints: each worker
+        takes a contiguous range of pairs with the requests inside it. frames: uint8 [F,C,H,W] host array; pairs / nums:
+        the requests, sorted by pair; out: uint8 [len(pairs),C,H,W]. Request j lands in out[j] whichever GPU computed
+        it, and sad_out[i] (optional uint64 [F-1]) receives pair i's SAD. Returns (out, images forwarded by the ranges
+        that completed)."""
+        pairs = np.ascontiguousarray(pairs, dtype=np.int32)
+        nums = np.ascontiguousarray(nums, dtype=np.int32)
+        n_frames = frames.shape[0]
+        if len(pairs) and (np.any(np.diff(pairs) < 0) or pairs[0] < 0 or pairs[-1] >= n_frames - 1):
+            raise ValueError(f"pairs must be sorted and inside [0, {n_frames - 1})")
+        if n_frames < 2:
+            return out, 0
+        forwards, lock = [0], threading.Lock()
+
+        def job(runner, first, n):
+            lo, hi = np.searchsorted(pairs, [first, first + n])
+            if lo == hi and sad_out is None:
+                return
+            _, f = runner.interpolate_dyadic_host_u8(frames[first:first + n + 1], pairs[lo:hi] - first, nums[lo:hi],
+                                                     depth, pairs_per_batch, out=out[lo:hi],
+                                                     sad_out=None if sad_out is None else sad_out[first:first + n])
+            with lock:
+                forwards[0] += f
+
+        self._run_ranges(n_frames - 1, job)
+        return out, forwards[0]
+
+    def _run_ranges(self, n_pairs, job):
+        """Calls job(runner, first_pair, n_pairs) for contiguous, equally sized ranges of [0, n_pairs), one per live
+        worker, concurrently. A worker whose job raises is retired and what it had left is re-queued for the others; an
+        invalid request (FI_ERR_INVALID) is raised as is and retires nobody."""
+        pending = [(0, n_pairs)]            # ranges of pairs still to compute: (first pair, count)
         lock = threading.Lock()
         rejected = []                       # invalid-argument errors: raised to the caller, no worker is retired
         while pending:
@@ -104,9 +148,7 @@ class GpuPool:
                     try:
                         if self.fault_hook is not None:
                             self.fault_hook(widx, first, n)
-                        extra = {} if sad_out is None else {"sad_out": sad_out[first:first + n]}
-                        self.runners[widx].interpolate_clip_host_u8(frames[first:first + n + 1], pairs_per_batch,
-                                                                     out=out[first:first + n], **extra)
+                        job(self.runners[widx], first, n)
                     except Exception as e:  # noqa: BLE001 - retire this worker, re-queue what it had left
                         if getattr(e, "code", None) == -1:   # FI_ERR_INVALID: the request is bad, not the GPU
                             with lock:
@@ -129,4 +171,3 @@ class GpuPool:
                     t.join()
             if rejected:
                 raise rejected[0]
-        return out

@@ -109,6 +109,27 @@ int fiNetInterpolateClipHostU8Sad(fiNet* net, const uint8_t* frames_host, int64_
                                   int channels_per_frame, uint8_t* out_host, int64_t out_stride, int H, int W,
                                   int pairs_per_batch, void* stream, uint64_t* pair_sad_host);
 
+/* Frame-rate conversion (main.py video --fps; the reference has none): frames at dyadic times between the frames of a
+ * clip, by recursive bisection on the device. The network has no time input, so node (i, a/2^d) with a odd is the
+ * network midpoint of (i, (a-1)/2^d) and (i, (a+1)/2^d), each in lowest terms; (i, 0) is frame i and (i, 1) frame i+1.
+ * That is exactly the frame host-side recursive bisection produces (the forward gives the same bits at any batch size).
+ *   frames_host: n_frames planar u8 frames [C, H, W], frame_stride bytes apart; n_classes must equal C
+ *                (channels_per_frame), because every node is fed back into the network;
+ *   request j:   node (req_pair_host[j], req_num_host[j] / 2^depth), depth in 1..6, 0 <= pair < n_frames-1,
+ *                0 < num < 2^depth, requests sorted by pair (any order of num, repeats allowed); it is written to
+ *                out_host + j*out_stride as u8 [C, H, W].
+ * Pairs go in groups of pairs_per_batch; each group's frames are uploaded once, the closure of its requests is evaluated
+ * level by level in batches of <= pairs_per_batch images with every node kept in a device pool (parents gathered with
+ * device-to-device copies), and only the requested nodes are copied back. Upload of group g+1, the levels of group g and
+ * the download of group g-1 overlap, as in the clip call. pair_sad_host (optional) receives every pair's SAD as in
+ * fiNetInterpolateClipHostU8Sad; with NULL, groups without requests are never uploaded. n_forwards_host (optional)
+ * receives the number of images forwarded. Any invalid argument returns FI_ERR_INVALID, naming it, before anything is
+ * launched or written. Synchronous: returns when out_host is complete. */
+int fiNetInterpolateDyadicHostU8(fiNet* net, const uint8_t* frames_host, int64_t frame_stride, int n_frames,
+                                 int channels_per_frame, int H, int W, int depth, const int32_t* req_pair_host,
+                                 const int32_t* req_num_host, int n_req, uint8_t* out_host, int64_t out_stride,
+                                 int pairs_per_batch, void* stream, uint64_t* pair_sad_host, int64_t* n_forwards_host);
+
 /* Algorithmic FLOPs (2*MACs, no padding) of one forward at this shape, and the number of kernel launches it makes. */
 int fiNetForwardCost(fiNet* net, int N, int H, int W, double* flops, int* launches);
 /* Measurement hook for bench.py: when enabled, every launch of the following forwards is bracketed by a CUDA event
