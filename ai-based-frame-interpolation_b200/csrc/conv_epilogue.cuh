@@ -12,39 +12,14 @@ struct EpiTile {
 };
 
 // DOUBLE_BUF as in epilogue_chunk_halo below: two alternating staging tiles per warp, or a single one.
-// split_src != nullptr (split-K, last arriver): the chunk's accumulators are the sum of `split_n` fp32 partial rows,
-// `split_stride` floats apart, that the CTAs sharing this tile left in global memory (summed in split order, so the
-// result does not depend on which CTA arrives last).
 template <int BLOCK_N, int MODE, bool SPLIT, bool DOUBLE_BUF = true>
 __device__ __forceinline__ void epilogue_chunk_8x16(const ConvMaps& maps, const ConvKernelParams& p, const EpiTile& tc,
                                                     uint32_t taddr, int c, int q, int lane, uint32_t my_stage,
-                                                    uint32_t my_pool, int& buf, bool store_enabled,
-                                                    const float* split_src = nullptr, int split_n = 0,
-                                                    size_t split_stride = 0) {
+                                                    uint32_t my_pool, int& buf, bool store_enabled) {
     uint32_t v0[32], v1[32];
-    if (split_src == nullptr) {
-        tmem_ld_32x32b_x32(taddr + c * 64, v0);
-        tmem_ld_32x32b_x32(taddr + c * 64 + 32, v1);
-        tmem_ld_wait();
-    } else {
-#pragma unroll
-        for (int j = 0; j < 32; ++j) v0[j] = v1[j] = 0u;  // +0.0f
-        for (int s = 0; s < split_n; ++s) {
-            const float4* src4 = reinterpret_cast<const float4*>(split_src + s * split_stride);
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-                const float4 a = __ldcg(src4 + j), b = __ldcg(src4 + 8 + j);
-                v0[4 * j + 0] = __float_as_uint(__uint_as_float(v0[4 * j + 0]) + a.x);
-                v0[4 * j + 1] = __float_as_uint(__uint_as_float(v0[4 * j + 1]) + a.y);
-                v0[4 * j + 2] = __float_as_uint(__uint_as_float(v0[4 * j + 2]) + a.z);
-                v0[4 * j + 3] = __float_as_uint(__uint_as_float(v0[4 * j + 3]) + a.w);
-                v1[4 * j + 0] = __float_as_uint(__uint_as_float(v1[4 * j + 0]) + b.x);
-                v1[4 * j + 1] = __float_as_uint(__uint_as_float(v1[4 * j + 1]) + b.y);
-                v1[4 * j + 2] = __float_as_uint(__uint_as_float(v1[4 * j + 2]) + b.z);
-                v1[4 * j + 3] = __float_as_uint(__uint_as_float(v1[4 * j + 3]) + b.w);
-            }
-        }
-    }
+    tmem_ld_32x32b_x32(taddr + c * 64, v0);
+    tmem_ld_32x32b_x32(taddr + c * 64 + 32, v1);
+    tmem_ld_wait();
     const int n_glob = tc.nb * BLOCK_N + c * 64;
     const float4* bias4 = reinterpret_cast<const float4*>(p.bias + n_glob);
     float f[64];

@@ -120,10 +120,9 @@ conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
     pdl_launch_dependents();  // the next layer may run its prologue on SMs this grid vacates
     pdl_wait();               // the previous layer's output is complete and visible from here on
 
-    // work item = (output tile, K split): ksplit CTAs share a tile, each reducing a contiguous range of the taps
-    const int ksplit = p.ksplit;
-    const int total_tiles = p.n_blocks * p.n_img * p.tiles_y * p.tiles_x * ksplit;
+    const int total_tiles = p.n_blocks * p.n_img * p.tiles_y * p.tiles_x;
     const int slabs = p.slabs;
+    const int k_iters = p.taps * slabs;
 
     if (warp == 0) {
         // ------------------------------------------------------------ TMA producer (warp converged, one lane issues)
@@ -131,9 +130,8 @@ conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
             int stage = 0;
             uint32_t phase = 0;
             for (int t = blockIdx.x; t < total_tiles; t += gridDim.x) {
-                const int tile = t / ksplit, ks = t - tile * ksplit;
-                const TileCoord tc = decode_tile(tile, p);
-                for (int tap = ks * p.taps / ksplit; tap < (ks + 1) * p.taps / ksplit; ++tap) {
+                const TileCoord tc = decode_tile(t, p);
+                for (int tap = 0; tap < p.taps; ++tap) {
                     const int dy = (p.taps == 9) ? tap / 3 - 1 : 0;
                     const int dx = (p.taps == 9) ? tap % 3 - 1 : 0;
                     int seg = 0, left = p.seg_slabs[0];
@@ -168,8 +166,6 @@ conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
             uint32_t phase = 0;
             int it = 0;
             for (int t = blockIdx.x; t < total_tiles; t += gridDim.x, ++it) {
-                const int ks = t % ksplit;
-                const int k_iters = ((ks + 1) * p.taps / ksplit - ks * p.taps / ksplit) * slabs;
                 const int acc = it & 1;
                 const uint32_t acc_phase = (it >> 1) & 1;
                 mbar_wait(bar_tempty + 8 * acc, acc_phase ^ 1);
@@ -207,60 +203,16 @@ conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
         int buf = 0;
         int it = 0;
         for (int t = blockIdx.x; t < total_tiles; t += gridDim.x, ++it) {
-            const int tile = t / ksplit, ks = t - tile * ksplit;
-            const TileCoord tc = decode_tile(tile, p);
+            const TileCoord tc = decode_tile(t, p);
             const int acc = it & 1;
             const uint32_t acc_phase = (it >> 1) & 1;
             mbar_wait(bar_tfull + 8 * acc, acc_phase);
             tc_fence_after();
             const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * BLOCK_N;
-            if (ksplit == 1) {
 #pragma unroll 1
-                for (int c = set; c < BLOCK_N / 64; c += EPI_SETS) {
-                    epilogue_chunk_8x16<BLOCK_N, MODE, SPLIT, !EIGHT>(maps, p, EpiTile{tc.nb, tc.img, tc.y0, tc.x0}, taddr,
-                                                                       c, q, lane, my_stage, my_pool, buf, true);
-                }
-            }
-            if constexpr (!SPLIT && (MODE == EPI_STORE || MODE == EPI_STORE_POOL)) {
-                if (ksplit > 1) {
-                    // Split K: park this CTA's partial rows (warp q owns accumulator rows 32q..32q+31) in global
-                    // memory; the last of the ksplit warps to arrive sums all partials and runs the real epilogue.
-                    const size_t part = static_cast<size_t>(BLOCK_M) * BLOCK_N;    // floats per (tile, split)
-                    float* mine = p.split_ws + (static_cast<size_t>(tile) * ksplit + ks) * part +
-                                  static_cast<size_t>(q * 32 + lane) * BLOCK_N;
-#pragma unroll 1
-                    for (int c = set; c < BLOCK_N / 64; c += EPI_SETS) {
-                        uint32_t v[32];
-#pragma unroll
-                        for (int h = 0; h < 2; ++h) {
-                            tmem_ld_32x32b_x32(taddr + c * 64 + 32 * h, v);
-                            tmem_ld_wait();
-                            float4* dst4 = reinterpret_cast<float4*>(mine + c * 64 + 32 * h);
-#pragma unroll
-                            for (int j = 0; j < 8; ++j)
-                                __stcg(dst4 + j, make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]),
-                                                             __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3])));
-                        }
-                    }
-                    __threadfence();
-                    __syncwarp();
-                    unsigned int arrived = 0;
-                    unsigned int* cnt = p.split_cnt + (static_cast<size_t>(tile) * 4 + q) * EPI_SETS + set;
-                    if (lane == 0) arrived = atomicAdd(cnt, 1u);
-                    arrived = __shfl_sync(0xffffffffu, arrived, 0);
-                    if (arrived == static_cast<unsigned int>(ksplit - 1)) {
-                        if (lane == 0) *cnt = 0u;   // left zero for the next launch that uses the scratch
-                        __threadfence();
-                        const float* first = p.split_ws + static_cast<size_t>(tile) * ksplit * part +
-                                             static_cast<size_t>(q * 32 + lane) * BLOCK_N;
-#pragma unroll 1
-                        for (int c = set; c < BLOCK_N / 64; c += EPI_SETS) {
-                            epilogue_chunk_8x16<BLOCK_N, MODE, SPLIT, !EIGHT>(maps, p, EpiTile{tc.nb, tc.img, tc.y0, tc.x0},
-                                                                               taddr, c, q, lane, my_stage, my_pool, buf,
-                                                                               true, first + c * 64, ksplit, part);
-                        }
-                    }
-                }
+            for (int c = set; c < BLOCK_N / 64; c += EPI_SETS) {
+                epilogue_chunk_8x16<BLOCK_N, MODE, SPLIT, !EIGHT>(maps, p, EpiTile{tc.nb, tc.img, tc.y0, tc.x0}, taddr, c,
+                                                                   q, lane, my_stage, my_pool, buf, true);
             }
             // All TMEM reads of this accumulator are complete (tmem_ld_wait above): hand it back to the MMA warp.
             tc_fence_before();
@@ -391,19 +343,13 @@ const char* conv_prepare(const ConvDesc& d, int num_sms, ConvLaunch* out) {
         pool_w = TILE_W / 2, pool_h = 1;
     const char* no_halo = getenv("FI_NO_HALO");
     l.halo = conv_halo_eligible(d) && !(no_halo && no_halo[0] == '1');
-    l.rows = l.halo && conv_rows_eligible(d);
-    if (l.rows) {
-        l.halo = 0;   // 64-channel layers without a pooled output: filter rows stacked along N (conv_rows.cu)
-        conv_rows_geometry(&tile_w, &tile_h, &box_w, &box_h);
-        block_n = d.n_total;
-    }
     if (l.halo) {
         int t;
         conv_halo_geometry(&t, &box_w, &box_h, &out_w, &out_h, &pool_w, &pool_h);
         tile_w = tile_h = t;
         block_n = d.n_total;
     }
-    if (!l.halo && !l.rows && (d.mode == EPI_STORE || d.mode == EPI_STORE_POOL)) {
+    if (!l.halo && (d.mode == EPI_STORE || d.mode == EPI_STORE_POOL)) {
         // Column-block width of the per-tap kernel. N = 256 is the efficient shape (tensor-bound M128/M256 x N256 MMAs,
         // CTA pairs halve the weight traffic: 1500-1600 TFLOP/s), narrower blocks are bound by the A-operand reads
         // (~56 % tensor-pipe activity at N = 128 under ncu). But a small frame gives a wide layer very few tiles:
@@ -450,8 +396,8 @@ const char* conv_prepare(const ConvDesc& d, int num_sms, ConvLaunch* out) {
         const char* cta2 = getenv("FI_CTA2");
         const bool want = cta2 ? cta2[0] != '0' : true;
         const bool narrow_resident = l.halo && d.n_total == 64 && kmul * (d.c0 + d.c1) == BLOCK_K;
-        l.pair = want && !l.rows && ((l.halo && !narrow_resident) || (!l.halo && block_n == 256 && d.mode != EPI_HEAD &&
-                                                            (d.mode != EPI_CONVT || d.c0 >= 1024)));
+        l.pair = want && ((l.halo && !narrow_resident) ||
+                          (!l.halo && block_n == 256 && d.mode != EPI_HEAD && (d.mode != EPI_CONVT || d.c0 >= 1024)));
     }
     {
         const uint64_t k_total = static_cast<uint64_t>(d.taps) * kmul * (d.c0 + d.c1);
@@ -486,10 +432,6 @@ const char* conv_prepare(const ConvDesc& d, int num_sms, ConvLaunch* out) {
     ConvKernelParams& p = l.p;
     p.tiles_x = (d.W + tile_w - 1) / tile_w;
     p.tiles_y = (d.H + tile_h - 1) / tile_h;
-    {
-        const char* pf = getenv("FI_HALO_PREFETCH");
-        p.prefetch_dist = pf ? atoi(pf) : 2;
-    }
     p.n_img = d.N;
     p.n_blocks = d.n_total / block_n;
     p.taps = d.taps;
@@ -517,54 +459,30 @@ const char* conv_prepare(const ConvDesc& d, int num_sms, ConvLaunch* out) {
     p.head_b = d.head_b;
     p.out_f32 = d.out_f32;
     p.out_u8 = d.out_u8;
-    p.dst = d.dst;
     l.block_n = block_n;
     l.mode = d.mode;
     l.split = precise ? 1 : 0;
-    long long total = static_cast<long long>(p.n_blocks) * p.n_img * p.tiles_y * p.tiles_x;
+    const long long total = static_cast<long long>(p.n_blocks) * p.n_img * p.tiles_y * p.tiles_x;
     if (total > 0x7fffffffLL) return "conv: too many tiles";
-    // Split K (the nine taps) over several CTAs of a layer that has too few tiles to occupy the GPU and a long K loop:
-    // the deepest layers of one small frame (down4.conv.3 of a 256x256 pair: 32 tiles, 144 K steps each). OPT-IN
-    // (FI_KSPLIT=n forces n-way where eligible, FI_KSPLIT=auto picks num_sms / tiles for layers with >= 144 K steps):
-    // measured on B200 (profiles/r02_small_profile*.json) the split costs ~8 us per layer (partial tiles through L2,
-    // fence, arrival counter, the last warp's sum), so it pays at 144 K steps (down4.conv.3 40 -> 31 us, up1.conv.0
-    // 41 -> 35 us, forward 0.329 -> 0.314 ms) and loses at 72 (25 -> 33 us) — and, unlike every other kernel choice, it
-    // changes the summation order, so results would depend on the plan's batch capacity in the last bf16 bit. A 5 %
-    // gain on one-pair latency does not buy that: the default keeps K in one CTA. Needs the caller's scratch.
-    p.ksplit = 1;
-    p.split_ws = d.split_ws;
-    p.split_cnt = d.split_cnt;
-    {
-        const char* ks = getenv("FI_KSPLIT");
-        const bool automatic = ks && ks[0] == 'a';
-        const int forced = (ks && !automatic) ? atoi(ks) : 0;
-        const bool eligible = !l.halo && !l.rows && !l.pair && !precise && d.taps == 9 && d.split_ws && d.split_cnt &&
-                              (d.mode == EPI_STORE || d.mode == EPI_STORE_POOL) && (automatic || forced > 1);
-        if (eligible && total > 0) {
-            int want = forced > 1 ? forced : static_cast<int>(num_sms / total);
-            if (automatic && (2 * total > num_sms || d.taps * p.slabs < 144)) want = 1;
-            if (want > d.taps) want = d.taps;
-            const size_t per_split = static_cast<size_t>(total) * BLOCK_M * block_n * sizeof(float);
-            while (want > 1 && (per_split * want > d.split_ws_bytes || total * 8 > d.split_cnt_count)) --want;
-            if (want > 1) p.ksplit = want;
-        }
-    }
-    total *= p.ksplit;
-    l.grid = static_cast<int>(total < num_sms ? total : num_sms);
-    if (l.pair) {
-        const long long m_tiles = static_cast<long long>(p.n_img) * p.tiles_y * p.tiles_x;
-        const long long pairs = p.n_blocks * ((m_tiles + 1) / 2);
-        const long long clusters = pairs < num_sms / 2 ? pairs : num_sms / 2;
-        l.grid = static_cast<int>(2 * clusters);
-    }
+    l.grid = conv_grid(l, num_sms);
     l.flops = 2.0 * d.N * d.H * d.W * static_cast<double>(d.n_total) * d.taps * (d.c0 + d.c1);
     if (d.mode == EPI_HEAD) l.flops += 2.0 * d.N * d.H * d.W * 64.0 * d.n_classes;
     *out = l;
     return nullptr;
 }
 
+int conv_grid(const ConvLaunch& l, int num_sms) {
+    const ConvKernelParams& p = l.p;
+    const long long m_tiles = static_cast<long long>(p.n_img) * p.tiles_y * p.tiles_x;
+    if (l.pair) {
+        const long long pairs = p.n_blocks * ((m_tiles + 1) / 2);
+        return static_cast<int>(2 * (pairs < num_sms / 2 ? pairs : num_sms / 2));
+    }
+    const long long tiles = p.n_blocks * m_tiles;
+    return static_cast<int>(tiles < num_sms ? tiles : num_sms);
+}
+
 const char* conv_launch(const ConvLaunch& l, cudaStream_t stream) {
-    if (l.rows) return conv_rows_launch(l, stream);
     if (l.halo) return l.pair ? conv_halo_pair_launch(l, stream) : conv_halo_launch(l, stream);
     if (l.pair) return conv_pair_launch(l, stream);
     switch (l.block_n * 4 + l.mode) {

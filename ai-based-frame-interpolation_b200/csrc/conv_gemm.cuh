@@ -48,12 +48,6 @@ struct ConvDesc {
     const void* src1_lo;
     void* dst_lo;       // lo halves of dst / dst_pool (EPI_STORE*, EPI_CONVT)
     void* dst_pool_lo;
-    // optional scratch for splitting K (the taps) of a layer with very few tiles over several CTAs (small frames):
-    // fp32 partial tiles + one arrival counter per (tile, epilogue warp); counters must be zero and are left zero
-    float* split_ws;
-    size_t split_ws_bytes;
-    unsigned int* split_cnt;
-    int split_cnt_count;
 };
 
 constexpr int MAX_SEGS = 6;
@@ -70,16 +64,11 @@ struct ConvKernelParams {
     int cout2;  // EPI_CONVT: 2*Cout (columns per output-row parity a)
     int H, W;
     int n_classes;
-    int prefetch_dist;  // halo kernel: L2-prefetch the halo boxes of the tile this many grid strides ahead (0 = off)
-    int ksplit;         // per-tap kernel: CTAs sharing one output tile, each reducing a range of taps (1 = off)
-    float* split_ws;    // [tile][split][128 rows][BLOCK_N] fp32 partial accumulators
-    unsigned int* split_cnt;  // [tile][4 epilogue warps] arrivals
     const float* bias;
     const float* head_w;
     const float* head_b;
     float* out_f32;
     uint8_t* out_u8;
-    void* dst;          // row-stacked kernel (conv_rows.cu): bf16 NHWC destination written with plain global stores
 };
 
 // A fully prepared launch: tensor maps are encoded once per (layer, shape) and reused every forward.
@@ -97,7 +86,6 @@ struct ConvLaunch {
     int mode;
     int split;  // 1: precise mode, epilogue writes hi + lo tensors
     int halo;  // 1: conv_halo.cu (halo-reuse kernel for Cout 64/128), 0: conv_gemm.cu
-    int rows;  // 1: conv_rows.cu (filter rows stacked along N for Cout = 64 without a pooled output)
     int pair;  // 1: conv_gemm2.cu (CTA-pair kernel, cta_group::2) for Cout multiples of 256
     int grid;
     double flops;  // algorithmic FLOPs of this launch (2*MACs, no padding counted)
@@ -106,6 +94,9 @@ struct ConvLaunch {
 // Returns nullptr on success, else a static error string.
 const char* conv_prepare(const ConvDesc& d, int num_sms, ConvLaunch* out);
 const char* conv_launch(const ConvLaunch& l, cudaStream_t stream);
+// Persistent grid of a prepared launch for its current l.p.n_img: one CTA (or CTA pair) per work item, at most one
+// per SM (pair). conv_prepare sets l.grid with it; a forward on fewer images than the plan holds calls it again.
+int conv_grid(const ConvLaunch& l, int num_sms);
 
 // bf16 tensor map (128B swizzle, zero OOB fill); dims/box innermost first, strides in elements for dims 1..rank-1.
 const char* encode_bf16_map_public(CUtensorMap* map, const void* base, int rank, const uint64_t* dims,
@@ -120,11 +111,6 @@ struct StemDesc;
 bool inc_fused_eligible(int cin, const ConvLaunch& conv);
 const char* inc_fused_launch(const StemDesc& d, const ConvLaunch& conv, const float* host_bias, int n_img, int num_sms,
                              cudaStream_t stream);
-
-// conv_rows.cu
-bool conv_rows_eligible(const ConvDesc& d);
-void conv_rows_geometry(int* tile_w, int* tile_h, int* box_w, int* box_h);
-const char* conv_rows_launch(const ConvLaunch& l, cudaStream_t stream);
 
 // conv_halo.cu
 bool conv_halo_eligible(const ConvDesc& d);

@@ -28,6 +28,7 @@ constexpr int HALO_BYTES = HALO_W * HALO_H * 128;      // 55296
 constexpr int HALO_THREADS = 224;        // 3 role warps + 4 epilogue warps (precise mode)
 constexpr int HALO_THREADS_8 = 352;      // 3 role warps + 8 epilogue warps (one set per column half)
 constexpr int A_STAGES = 2;
+constexpr int PREFETCH_DIST = 2;         // L2-prefetch the halo boxes this many grid strides ahead (DESIGN §3 item 3)
 constexpr int B_RING_BYTES = 65536;
 constexpr int H_STAGING_PER_WARP = 2 * 4096;
 constexpr int H_POOL_PER_WARP = 2 * 1024;
@@ -143,8 +144,8 @@ conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
                 const HTile tc = decode_htile(t, p);
                 // Only A_STAGES-1 halo boxes can be in flight towards smem, which does not cover HBM latency:
                 // pull the boxes of this CTA's tile after next into L2 now (no smem needed for that).
-                const int tp = t + p.prefetch_dist * static_cast<int>(gridDim.x);
-                if (p.prefetch_dist > 0 && tp < total_tiles && lane == 0) {
+                const int tp = t + PREFETCH_DIST * static_cast<int>(gridDim.x);
+                if (tp < total_tiles && lane == 0) {
                     const HTile pc = decode_htile(tp, p);
                     for (int g = 0; g < p.nseg; ++g) {
                         const int mid = p.seg_map[g];

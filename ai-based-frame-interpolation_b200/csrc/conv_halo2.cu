@@ -26,6 +26,7 @@ constexpr int H2_HALO_BYTES = H2_W * H2_H * 128;  // 55296
 constexpr int H2_THREADS = 224;
 constexpr int H2_THREADS_8 = 352;
 constexpr int H2_A_STAGES = 2;
+constexpr int H2_PREFETCH_DIST = 2;               // as conv_halo.cu: L2 prefetch this many cluster strides ahead
 constexpr int H2_B_BYTES = 73728;                 // weight region: a ring, or up to 72 KB of resident half slabs
 constexpr int H2_STAGING = 4 * (2 * 4096 + 2 * 1024);
 constexpr int H2_SMEM = 1024 + H2_A_STAGES * H2_HALO_BYTES + H2_B_BYTES + H2_STAGING + 512;
@@ -139,8 +140,8 @@ conv_halo2_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams 
         uint32_t phase = 0;
         for (int qi = cluster_id; qi < total; qi += n_clusters) {
             const PairHTile pt = decode_pair_htile(qi, rank, p);
-            const int qp = qi + p.prefetch_dist * n_clusters;
-            if (p.prefetch_dist > 0 && qp < total && lane == 0) {
+            const int qp = qi + H2_PREFETCH_DIST * n_clusters;
+            if (qp < total && lane == 0) {
                 const PairHTile pc = decode_pair_htile(qp, rank, p);
                 for (int g = 0; g < p.nseg; ++g) {
                     const int mid = p.seg_map[g];

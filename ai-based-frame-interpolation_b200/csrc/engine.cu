@@ -102,7 +102,6 @@ struct Step {
 struct Plan {
     int N = 0, H = 0, W = 0;  // N = batch CAPACITY of the arena / tensor maps; any batch <= N runs without re-planning
     DevBuf arena;
-    DevBuf split_ws, split_cnt;  // split-K scratch shared by the layers of this plan (they run one after the other)
     std::map<std::string, Act> acts;
     std::vector<Step> steps;
     int head_step = -1;
@@ -113,8 +112,6 @@ struct Plan {
         steps.clear();
         acts.clear();
         arena.release();
-        split_ws.release();
-        split_cnt.release();
         N = H = W = 0;
         head_step = -1;
         last_n = 0;
@@ -468,14 +465,6 @@ int fill_plan(fiNet* net, Plan& pl, int N, int H, int W) {
         pl.arena.p = p;
         pl.arena.bytes = cursor;
     }
-    // split-K scratch (conv_prepare uses it only for layers with too few tiles to fill the GPU: small frames)
-    constexpr size_t SPLIT_WS_BYTES = size_t(8) << 20;
-    constexpr int SPLIT_COUNTERS = 8192;
-    if (cudaMalloc(&pl.split_ws.p, SPLIT_WS_BYTES) == cudaSuccess) pl.split_ws.bytes = SPLIT_WS_BYTES;
-    if (cudaMalloc(&pl.split_cnt.p, SPLIT_COUNTERS * sizeof(unsigned int)) == cudaSuccess) {
-        pl.split_cnt.bytes = SPLIT_COUNTERS * sizeof(unsigned int);
-        CUDA_TRY(cudaMemset(pl.split_cnt.p, 0, pl.split_cnt.bytes));
-    }
     auto ptr = [&](const std::string& name) -> void* {
         return static_cast<char*>(pl.arena.p) + pl.acts.at(name).off;
     };
@@ -512,12 +501,6 @@ int fill_plan(fiNet* net, Plan& pl, int N, int H, int W) {
         d.c0 = a.C;
         d.H = a.H;
         d.W = a.W;
-        if (pl.split_ws.p && pl.split_cnt.p) {
-            d.split_ws = static_cast<float*>(pl.split_ws.p);
-            d.split_ws_bytes = pl.split_ws.bytes;
-            d.split_cnt = static_cast<unsigned int*>(pl.split_cnt.p);
-            d.split_cnt_count = SPLIT_COUNTERS;
-        }
         if (!src1.empty()) {
             const Act& b = pl.acts.at(src1);
             d.src1 = ptr(src1);
@@ -962,14 +945,7 @@ int fiNetForward(fiNet* net, const fiPlanes* in0, const fiPlanes* in1, int in_dt
             }
             // the plan's arena and tensor maps are sized for pl.N images; this call uses the first N of them
             s.conv.p.n_img = N;
-            const long long m_tiles = static_cast<long long>(N) * s.conv.p.tiles_y * s.conv.p.tiles_x;
-            if (s.conv.pair) {
-                const long long pairs = s.conv.p.n_blocks * ((m_tiles + 1) / 2);
-                s.conv.grid = static_cast<int>(2 * (pairs < net->num_sms / 2 ? pairs : net->num_sms / 2));
-            } else {
-                const long long tiles = s.conv.p.n_blocks * m_tiles * s.conv.p.ksplit;
-                s.conv.grid = static_cast<int>(tiles < net->num_sms ? tiles : net->num_sms);
-            }
+            s.conv.grid = fi::conv_grid(s.conv, net->num_sms);
             KERNEL_TRY(fi::conv_launch(s.conv, st));
         }
         if (evs) CUDA_TRY(cudaEventRecord(evs[2 * i + 1], st));

@@ -197,17 +197,6 @@ __device__ __forceinline__ void tmem_ld_32x32b_x32(uint32_t taddr, uint32_t (&r)
         : "memory");
 }
 
-// 32 lanes x 16 consecutive fp32 columns.
-__device__ __forceinline__ void tmem_ld_32x32b_x16(uint32_t taddr, uint32_t (&r)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr)
-        : "memory");
-}
-
 // ------------------------------------------------------------------ tcgen05.mma (single CTA, bf16/f16 -> fp32)
 // D[tmem] (+)= A[smem desc] * B[smem desc]; issued by ONE thread.
 __device__ __forceinline__ void umma_bf16_ss(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,

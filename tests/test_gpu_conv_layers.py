@@ -11,12 +11,10 @@ from layer_utils import bf16_round, ref_conv3x3, run_conv, run_conv_precise
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(params=["rows", "halo", "per-tap", "pair"], autouse=True)
+@pytest.fixture(params=["halo", "per-tap", "pair"], autouse=True)
 def kernel_variant(request, monkeypatch):
-    """Cout 64/128 layers have two kernels (conv_halo.cu / conv_gemm.cu), Cout 64 with a plain store a third
-    (conv_rows.cu, opt-in: slower than the halo kernels, kept with its measurements), and Cout multiples of 256 have the single-CTA and the CTA-pair kernel
-    (conv_gemm.cu / conv_gemm2.cu); run every case through all selections."""
-    monkeypatch.setenv("FI_ROWS", "2" if request.param == "rows" else "0")   # 2: one-slab layers as well
+    """Cout 64/128 layers have two kernels (conv_halo.cu / conv_gemm.cu) and Cout multiples of 256 have the single-CTA
+    and the CTA-pair kernel (conv_gemm.cu / conv_gemm2.cu); run every case through all selections."""
     monkeypatch.setenv("FI_NO_HALO", "1" if request.param == "per-tap" else "0")
     monkeypatch.setenv("FI_CTA2", "1" if request.param == "pair" else "0")
     return request.param
@@ -44,7 +42,7 @@ def rnd(g, *shape, scale=1.0):
     (1, 64, 64, 200, 208),     # 325 tiles on <=148 CTAs: TMEM double buffering and barrier phases
     (1, 128, 64, 5, 7),        # image smaller than one tile
     (3, 192, 320, 9, 17),      # odd everything; cout 320 -> BLOCK_N 64 x 5 blocks
-    (2, 64, 64, 13, 95),       # row-stacked kernel: 4-row x 30-column tiles, ragged in both dims
+    (2, 64, 64, 13, 95),       # ragged halo tiles in both dims, two images
     (1, 128, 64, 9, 61),       # ... with two K slabs from one source
 ])
 def test_conv3x3_store(cuda_device, n, cin, cout, h, w):
@@ -79,7 +77,7 @@ def test_conv3x3_pool(cuda_device, n, c, cout, h, w):
 
 @pytest.mark.parametrize("c0,c1,cout,h,w,h1,w1", [
     (64, 64, 64, 16, 32, 16, 32),        # plain concat
-    (64, 64, 64, 17, 33, 16, 32),        # Cout 64 (row-stacked kernel) with F.pad
+    (64, 64, 64, 17, 33, 16, 32),        # Cout 64 with F.pad
     (64, 64, 64, 70, 118, 70, 118),      # ... several tiles per CTA row
     (128, 128, 128, 17, 33, 16, 32),     # F.pad: one zero row at the bottom / column on the right
     (256, 256, 256, 19, 20, 16, 16),     # pad on both sides (diff 3 -> 1 before, 2 after; diff 4 -> 2, 2)

@@ -44,8 +44,7 @@ ULP = 2.0 ** -7
 K_BF16, K_STEM, K_FP32 = 1e-5, 2.0 ** -14, 2.0 ** -14      # coefficients of A
 R_FP32 = 2.0 ** -15
 BAND_ELEMS = 1 << 27                 # fp64 elements per band operand (1 GiB)
-SELECTION_ENV = ("FI_CTA2", "FI_NO_HALO", "FI_ROWS", "FI_BLOCK_N", "FI_KSPLIT", "FI_FUSE_INC", "FI_ARENA_REUSE",
-                 "FI_HALO_PREFETCH")
+SELECTION_ENV = ("FI_CTA2", "FI_NO_HALO", "FI_BLOCK_N", "FI_FUSE_INC", "FI_ARENA_REUSE")
 
 
 @pytest.fixture(autouse=True)

@@ -200,7 +200,7 @@ def main():
     if all(d for _, d in pp):
         w("Pairs per forward (`bench.py --pairs K`): " + ", ".join(f"K={k}: {d['value']:.1f} frames/s" for k, d in pp) + ".\n")
     notes = [(f"{R}_fused_inc.md", "fused `inc` kernel: ncu source-page reading (per-role wait shares, shared-memory port)"),
-             (f"{R}_rows.md", "row-stacked conv kernel (`FI_ROWS`): parity-green, measured slower than the halo kernels, why"),
+             (f"{R}_rows.md", "row-stacked conv kernel (removed kernel, commit c63f920): parity-green, measured slower than the halo kernels, why"),
              ("sass_summary.txt", "opcode counts per kernel from `cuobjdump -sass` (tcgen05 MMA, TMA, TMEM, PDL; no legacy HMMA)"),
              ("ncu_traffic.json", "DRAM bytes per conv launch from the `--set full` capture (the `roofline.traffic` source of bench.py)")]
     notes = [(f, t) for f, t in notes if (P / f).exists()]
