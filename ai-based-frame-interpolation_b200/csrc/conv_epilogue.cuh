@@ -1,4 +1,4 @@
-// Epilogue of one 64-column chunk of an 8x16-pixel accumulator tile (shared by conv_gemm.cu and conv_gemm2.cu):
+// Epilogue of one 64-column chunk of an 8x16-pixel accumulator tile (the per-tap kernels of conv_gemm.cu):
 // TMEM -> registers, bias (+ReLU), then by mode: bf16 (or hi/lo) tile -> swizzled staging -> TMA store (+ 2x2 max-pooled
 // tile), the transposed-conv pixel scatter, or the fused 1x1 head + postprocess.
 #pragma once

@@ -13,7 +13,22 @@
 // B operand: BN-folded weights, bf16 [N][K] K-major, one TMA box {64, BLOCK_N} per K slab.
 // Both land in 128B-swizzled K-major smem tiles that tcgen05.mma reads through shared-memory descriptors.
 // Accumulators: fp32 in TMEM, double buffered (2 x BLOCK_N columns) so the epilogue of tile i overlaps tile i+1.
-// Warp roles (192 threads): warp 0 = TMA producer, warp 1 = TMEM owner + MMA issuer, warps 2..5 = epilogue.
+// Warp roles (192 threads): warp 0 = TMA producer, warp 1 = TMEM owner + MMA issuer, warps 2..5 = epilogue
+// (320 threads and warps 2..9 where two epilogue sets split the 64-column chunks of a tile).
+//
+// CTA pairs (conv_gemm2_kernel, cta_group::2) for the wide layers (Cout multiple of 256). Measured with
+// tools/probe/mma_probe.cu, a tcgen05.mma costs max(N/2, operand bytes per SM / ~120) cycles, and the TMA fills compete
+// for the same ~128 B/cycle of shared-memory bandwidth. A single CTA doing M128 x N256 reads 12 KB of operands and
+// receives 12 KB of new tiles per MMA-time: 192 B/cycle of demand. In a CTA pair each SM keeps its own 128 pixel rows
+// of A but only HALF of the weight slab (128 of the 256 rows); the pair's MMA is M256 x N256, the hardware reads both
+// halves, and each SM's traffic drops to 8 KB + 8 KB per 128 cycles = 128 B/cycle.
+// Protocol (cluster of 2, same code in both CTAs, rank 0 = leader, adjacent pixel tiles):
+//   producers (warp 0 of both)   wait on their LOCAL empty barrier, load their own A tile and their half of B with
+//                                cp.async.bulk.tensor...cta_group::2, completion bytes go to the LEADER's full barrier
+//   MMA issuer (warp 1, leader)  waits on its full barrier (2 x 32 KB), issues tcgen05.mma.cta_group::2, and commits
+//                                with a multicast to the empty / accumulator-full barriers of BOTH CTAs
+//   epilogue (warps 2..5, both)  read their own TMEM lanes; release the accumulator by arriving (locally or through
+//                                mapa) on the leader's accumulator-empty barrier (8 arrivals per phase)
 #include "conv_epilogue.cuh"
 #include "conv_gemm.cuh"
 #include "ptx.cuh"
@@ -26,7 +41,7 @@ namespace fi {
 
 namespace {
 
-constexpr int NUM_THREADS = 192;    // 2 role warps + 4 epilogue warps (precise mode, head)
+constexpr int NUM_THREADS = 192;    // 2 role warps + 4 epilogue warps (precise mode, head, CTA pairs)
 constexpr int NUM_THREADS_8 = 320;  // 2 role warps + 8 epilogue warps: two sets split the 64-column chunks of a tile
 constexpr int A_STAGE_BYTES = BLOCK_M * 128;             // 16 KB
 constexpr int STAGING_BYTES_PER_WARP = 2 * 4096;         // 2 x (32 rows x 128 B)
@@ -35,6 +50,7 @@ constexpr int EPI_BYTES = 4 * (STAGING_BYTES_PER_WARP + POOL_BYTES_PER_WARP);
 constexpr int BAR_BYTES = 256;
 constexpr int SMEM_LIMIT = 232448;                       // 227 KB usable per CTA on sm_100
 
+// Ring depth and shared memory follow from the B slab one CTA holds: BLOCK_N rows, or half of them in a CTA pair.
 __host__ __device__ constexpr int b_stage_bytes(int block_n) { return block_n * 128; }
 __host__ __device__ constexpr int num_stages(int block_n) {
     int s = (SMEM_LIMIT - 1024 - BAR_BYTES - EPI_BYTES) / (A_STAGE_BYTES + b_stage_bytes(block_n));
@@ -45,38 +61,48 @@ __host__ __device__ constexpr int smem_bytes(int block_n) {
 }
 __host__ __device__ constexpr int tmem_cols(int block_n) { return 2 * block_n < 32 ? 32 : 2 * block_n; }
 
-struct TileCoord {
-    int nb, img, y0, x0;
+struct Unit {
+    EpiTile t;
+    bool valid;  // false: odd tile count, the last pair's second CTA recomputes the last tile with its stores off
 };
-__device__ __forceinline__ TileCoord decode_tile(int t, const ConvKernelParams& p) {
-    // Tiles that share a weight block are adjacent in time across the grid so the B slabs stay hot in L2.
+// Work unit u -> this CTA's tile. Units that share a weight block are adjacent in time across the grid so the B slabs
+// stay hot in L2; the two CTAs of a pair take adjacent pixel tiles of the same weight block.
+template <int CTAS>
+__device__ __forceinline__ Unit decode_unit(int u, uint32_t rank, const ConvKernelParams& p) {
     const int per_img = p.tiles_y * p.tiles_x;
     const int m_tiles = p.n_img * per_img;
-    TileCoord c;
-    c.nb = t / m_tiles;
-    int m = t - c.nb * m_tiles;
-    c.img = m / per_img;
-    m -= c.img * per_img;
+    const int per_nb = (m_tiles + CTAS - 1) / CTAS;
+    Unit r;
+    r.t.nb = u / per_nb;
+    int m = CTAS * (u - r.t.nb * per_nb) + static_cast<int>(rank);
+    r.valid = CTAS == 1 || m < m_tiles;
+    if (!r.valid) m = m_tiles - 1;
+    r.t.img = m / per_img;
+    m -= r.t.img * per_img;
     const int ty = m / p.tiles_x;
-    c.y0 = ty * TILE_H;
-    c.x0 = (m - ty * p.tiles_x) * TILE_W;
-    return c;
+    r.t.y0 = ty * TILE_H;
+    r.t.x0 = (m - ty * p.tiles_x) * TILE_W;
+    return r;
 }
 
-__host__ __device__ constexpr bool eight_epilogue_warps(int block_n, int mode, bool split) {
-    return !split && mode != EPI_HEAD && block_n >= 128;  // needs >= 2 chunks per tile and single staging tiles
+__host__ __device__ constexpr bool eight_epilogue_warps(int ctas, int block_n, int mode, bool split) {
+    // needs >= 2 chunks per tile and single staging tiles; a pair's leader counts the arrivals of 4 warps per CTA
+    return ctas == 1 && !split && mode != EPI_HEAD && block_n >= 128;
+}
+__host__ __device__ constexpr int num_threads(int ctas, int block_n, int mode, bool split) {
+    return eight_epilogue_warps(ctas, block_n, mode, split) ? NUM_THREADS_8 : NUM_THREADS;
 }
 
-template <int BLOCK_N, int MODE, bool SPLIT>
-__global__ void __launch_bounds__(eight_epilogue_warps(BLOCK_N, MODE, SPLIT) ? NUM_THREADS_8 : NUM_THREADS, 1)
-conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p) {
-    constexpr int STAGES = num_stages(BLOCK_N);
-    constexpr int B_STAGE_BYTES = b_stage_bytes(BLOCK_N);
+// CTAS = 1: one CTA per tile. CTAS = 2: a CTA pair (cluster of 2) computes two adjacent tiles as one M256 GEMM.
+template <int CTAS, int BLOCK_N, int MODE, bool SPLIT>
+__device__ __forceinline__ void conv_gemm_body(const ConvMaps& maps, const ConvKernelParams& p) {
+    constexpr int STAGES = num_stages(BLOCK_N / CTAS);
+    constexpr int B_STAGE_BYTES = b_stage_bytes(BLOCK_N / CTAS);  // this CTA's rows of the weight slab
     constexpr uint32_t STAGE_TX = A_STAGE_BYTES + B_STAGE_BYTES;
     constexpr int TMEM_COLS = tmem_cols(BLOCK_N);
-    constexpr uint32_t IDESC = umma_idesc_bf16(BLOCK_M, BLOCK_N);
+    constexpr uint32_t IDESC = umma_idesc_bf16(BLOCK_M * CTAS, BLOCK_N);
     static_assert(MODE != EPI_HEAD || BLOCK_N == 64, "head epilogue consumes exactly 64 channels");
-    constexpr bool EIGHT = eight_epilogue_warps(BLOCK_N, MODE, SPLIT);
+    constexpr bool EIGHT = eight_epilogue_warps(CTAS, BLOCK_N, MODE, SPLIT);
     constexpr int EPI_SETS = EIGHT ? 2 : 1;
 
     extern __shared__ uint8_t smem_raw[];
@@ -95,6 +121,8 @@ conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
+    const uint32_t rank = CTAS == 1 ? 0 : cluster_ctarank();
+    const bool leader = CTAS == 1 || rank == 0;
 
     if (warp == 0 && lane == 0) {
         tma_prefetch_desc(&maps.a[0]);
@@ -103,24 +131,27 @@ conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
         if (MODE != EPI_HEAD) tma_prefetch_desc(&maps.out[0]);
         if (MODE == EPI_STORE_POOL) tma_prefetch_desc(&maps.pool[0]);
         for (int s = 0; s < STAGES; ++s) {
-            mbar_init(bar_full + 8 * s, 1);
-            mbar_init(bar_empty + 8 * s, 1);
+            mbar_init(bar_full + 8 * s, 1);   // pair: the leader's own arrive.expect_tx; bytes arrive from both CTAs
+            mbar_init(bar_empty + 8 * s, 1);  // one (multicast) commit per use
         }
         for (int a = 0; a < 2; ++a) {
             mbar_init(bar_tfull + 8 * a, 1);
-            mbar_init(bar_tempty + 8 * a, 4 * EPI_SETS);  // one arrive per epilogue warp
+            mbar_init(bar_tempty + 8 * a, 4 * EPI_SETS * CTAS);  // one arrive per epilogue warp (of both CTAs)
         }
         fence_mbar_init();
     }
-    if (warp == 1) tmem_alloc(tmem_slot, TMEM_COLS);
+    if (warp == 1) tmem_alloc<CTAS>(tmem_slot, TMEM_COLS);
     tc_fence_before();
     __syncthreads();
+    if constexpr (CTAS == 2) cluster_sync_all();  // both CTAs' barriers exist before any remote signal can arrive
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot_ptr;
     pdl_launch_dependents();  // the next layer may run its prologue on SMs this grid vacates
     pdl_wait();               // the previous layer's output is complete and visible from here on
 
-    const int total_tiles = p.n_blocks * p.n_img * p.tiles_y * p.tiles_x;
+    const int units = p.n_blocks * ((p.n_img * p.tiles_y * p.tiles_x + CTAS - 1) / CTAS);
+    const int unit0 = static_cast<int>(blockIdx.x / CTAS);
+    const int unit_step = static_cast<int>(gridDim.x / CTAS);
     const int slabs = p.slabs;
     const int k_iters = p.taps * slabs;
 
@@ -129,8 +160,8 @@ conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
         {
             int stage = 0;
             uint32_t phase = 0;
-            for (int t = blockIdx.x; t < total_tiles; t += gridDim.x) {
-                const TileCoord tc = decode_tile(t, p);
+            for (int u = unit0; u < units; u += unit_step) {
+                const EpiTile tc = decode_unit<CTAS>(u, rank, p).t;
                 for (int tap = 0; tap < p.taps; ++tap) {
                     const int dy = (p.taps == 9) ? tap / 3 - 1 : 0;
                     const int dx = (p.taps == 9) ? tap % 3 - 1 : 0;
@@ -143,12 +174,13 @@ conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
                         mbar_wait(bar_empty + 8 * stage, phase ^ 1);
                         const uint32_t full = bar_full + 8 * stage;
                         if (elect_one()) {
-                            mbar_expect_tx(full, STAGE_TX);
+                            if (leader) mbar_expect_tx(full, CTAS * STAGE_TX);
                             const int ox = mid >= 2 ? p.off_x : 0, oy = mid >= 2 ? p.off_y : 0;  // F.pad of src1
-                            tma_load_4d(smem_a + stage * A_STAGE_BYTES, &maps.a[mid], full, local * BLOCK_K,
-                                        tc.x0 + dx - ox, tc.y0 + dy - oy, tc.img);
-                            tma_load_2d(smem_b + stage * B_STAGE_BYTES, &maps.b, full, (tap * slabs + s) * BLOCK_K,
-                                        tc.nb * BLOCK_N);
+                            tma_load_4d<CTAS>(smem_a + stage * A_STAGE_BYTES, &maps.a[mid], full, local * BLOCK_K,
+                                              tc.x0 + dx - ox, tc.y0 + dy - oy, tc.img);
+                            tma_load_2d<CTAS>(smem_b + stage * B_STAGE_BYTES, &maps.b, full,
+                                              (tap * slabs + s) * BLOCK_K,
+                                              tc.nb * BLOCK_N + static_cast<int>(rank) * (BLOCK_N / CTAS));
                         }
                         __syncwarp();
                         if (++stage == STAGES) {
@@ -160,12 +192,13 @@ conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
             }
         }
     } else if (warp == 1) {
-        // ------------------------------------------------------------ MMA issuer (warp converged, one lane issues)
-        {
+        // ------------------------------------------------------------ MMA issuer (warp converged, one lane issues;
+        // a pair's MMAs are all issued by the leader CTA)
+        if (leader) {
             int stage = 0;
             uint32_t phase = 0;
             int it = 0;
-            for (int t = blockIdx.x; t < total_tiles; t += gridDim.x, ++it) {
+            for (int u = unit0; u < units; u += unit_step, ++it) {
                 const int acc = it & 1;
                 const uint32_t acc_phase = (it >> 1) & 1;
                 mbar_wait(bar_tempty + 8 * acc, acc_phase ^ 1);
@@ -180,10 +213,10 @@ conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
 #pragma unroll
                         for (int k = 0; k < BLOCK_K / 16; ++k) {
                             // +32 bytes along K inside the 128B swizzle row = +2 in the (addr >> 4) field
-                            umma_bf16_ss(d_tmem, da + 2 * k, db + 2 * k, IDESC, (kb | k) != 0);
+                            umma_bf16_ss<CTAS>(d_tmem, da + 2 * k, db + 2 * k, IDESC, (kb | k) != 0);
                         }
-                        umma_commit(bar_empty + 8 * stage);  // frees the smem slot once these MMAs retire
-                        if (kb == k_iters - 1) umma_commit(bar_tfull + 8 * acc);  // accumulator complete -> epilogue
+                        umma_commit<CTAS>(bar_empty + 8 * stage);  // frees the smem slot once these MMAs retire
+                        if (kb == k_iters - 1) umma_commit<CTAS>(bar_tfull + 8 * acc);  // accumulator complete
                     }
                     __syncwarp();
                     if (++stage == STAGES) {
@@ -197,13 +230,13 @@ conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
         // ------------------------------------------------------------ epilogue warps 2..5
         const int q = warp & 3;  // TMEM lanes [32q, 32q+32) <-> tile rows 2q, 2q+1
         const int ew = warp - 2;   // 0..3, or 0..7 with two epilogue sets
-        const int set = ew >> 2;
+        const int set = EIGHT ? ew >> 2 : 0;
         const uint32_t my_stage = smem_stage + ew * (EIGHT ? 4096 : STAGING_BYTES_PER_WARP);
         const uint32_t my_pool = smem_pool + ew * (EIGHT ? 1024 : POOL_BYTES_PER_WARP);
         int buf = 0;
         int it = 0;
-        for (int t = blockIdx.x; t < total_tiles; t += gridDim.x, ++it) {
-            const TileCoord tc = decode_tile(t, p);
+        for (int u = unit0; u < units; u += unit_step, ++it) {
+            const Unit w = decode_unit<CTAS>(u, rank, p);
             const int acc = it & 1;
             const uint32_t acc_phase = (it >> 1) & 1;
             mbar_wait(bar_tfull + 8 * acc, acc_phase);
@@ -211,13 +244,16 @@ conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
             const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * BLOCK_N;
 #pragma unroll 1
             for (int c = set; c < BLOCK_N / 64; c += EPI_SETS) {
-                epilogue_chunk_8x16<BLOCK_N, MODE, SPLIT, !EIGHT>(maps, p, EpiTile{tc.nb, tc.img, tc.y0, tc.x0}, taddr, c,
-                                                                   q, lane, my_stage, my_pool, buf, true);
+                epilogue_chunk_8x16<BLOCK_N, MODE, SPLIT, !EIGHT>(maps, p, w.t, taddr, c, q, lane, my_stage, my_pool,
+                                                                   buf, w.valid);
             }
             // All TMEM reads of this accumulator are complete (tmem_ld_wait above): hand it back to the MMA warp.
             tc_fence_before();
             __syncwarp();
-            if (elect_one()) mbar_arrive(bar_tempty + 8 * acc);
+            if (elect_one()) {
+                if (leader) mbar_arrive(bar_tempty + 8 * acc);
+                else mbar_arrive_cluster(bar_tempty + 8 * acc, 0);
+            }
         }
         __syncwarp();
         if (MODE != EPI_HEAD && elect_one()) tma_store_wait_all();
@@ -225,10 +261,23 @@ conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
 
     tc_fence_before();
     __syncthreads();
+    if constexpr (CTAS == 2) cluster_sync_all();  // the peer may still be reading TMEM / receiving commits
     if (warp == 1) {
         tc_fence_after();
-        tmem_dealloc(tmem_base, TMEM_COLS);
+        tmem_dealloc<CTAS>(tmem_base, TMEM_COLS);
     }
+}
+
+template <int BLOCK_N, int MODE, bool SPLIT>
+__global__ void __launch_bounds__(num_threads(1, BLOCK_N, MODE, SPLIT), 1)
+conv_gemm_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p) {
+    conv_gemm_body<1, BLOCK_N, MODE, SPLIT>(maps, p);
+}
+
+template <int MODE, bool SPLIT>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(num_threads(2, 256, MODE, SPLIT), 1)
+conv_gemm2_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p) {
+    conv_gemm_body<2, 256, MODE, SPLIT>(maps, p);
 }
 
 // ------------------------------------------------------------------------------------------------ host side
@@ -285,18 +334,40 @@ const char* encode_nhwc(CUtensorMap* map, const void* base, int n, int h, int w,
     return encode_bf16_map(map, base, 4, dims, strides, box);
 }
 
-template <int BLOCK_N, int MODE, bool SPLIT = false>
+template <int CTAS, int BLOCK_N, int MODE, bool SPLIT = false>
 const char* launch_inst(const ConvLaunch& l, cudaStream_t stream) {
     if constexpr (!SPLIT && MODE != EPI_HEAD) {
-        if (l.split) return launch_inst<BLOCK_N, MODE, true>(l, stream);
+        if (l.split) return launch_inst<CTAS, BLOCK_N, MODE, true>(l, stream);
     }
-    auto kfn = conv_gemm_kernel<BLOCK_N, MODE, SPLIT>;
+    static_assert(CTAS == 1 || BLOCK_N == 256, "CTA pairs run 256-column blocks");
+    void (*kfn)(ConvMaps, ConvKernelParams);
+    if constexpr (CTAS == 1) kfn = conv_gemm_kernel<BLOCK_N, MODE, SPLIT>;
+    else kfn = conv_gemm2_kernel<MODE, SPLIT>;
     static std::atomic<uint64_t> configured{0};  // per instantiation: devices with the shared-memory opt-in
-    constexpr int smem = smem_bytes(BLOCK_N);
+    constexpr int smem = smem_bytes(BLOCK_N / CTAS);
     if (!smem_opt_in(kfn, smem, configured)) return "cudaFuncSetAttribute(MaxDynamicSharedMemorySize) failed";
-    const cudaError_t e = launch_kernel(kfn, dim3(l.grid), dim3(eight_epilogue_warps(BLOCK_N, MODE, SPLIT) ? NUM_THREADS_8 : NUM_THREADS),
-                                        smem, stream, l.maps, l.p);
+    const cudaError_t e =
+        launch_kernel(kfn, dim3(l.grid), dim3(num_threads(CTAS, BLOCK_N, MODE, SPLIT)), smem, stream, l.maps, l.p);
     return e == cudaSuccess ? nullptr : cudaGetErrorString(e);
+}
+
+template <int CTAS>
+const char* launch_per_tap(const ConvLaunch& l, cudaStream_t stream) {
+    switch (l.block_n * 4 + l.mode) {
+        case 256 * 4 + EPI_STORE: return launch_inst<CTAS, 256, EPI_STORE>(l, stream);
+        case 256 * 4 + EPI_STORE_POOL: return launch_inst<CTAS, 256, EPI_STORE_POOL>(l, stream);
+        case 256 * 4 + EPI_CONVT: return launch_inst<CTAS, 256, EPI_CONVT>(l, stream);
+    }
+    if constexpr (CTAS == 1) {
+        switch (l.block_n * 4 + l.mode) {
+            case 64 * 4 + EPI_STORE: return launch_inst<1, 64, EPI_STORE>(l, stream);
+            case 64 * 4 + EPI_STORE_POOL: return launch_inst<1, 64, EPI_STORE_POOL>(l, stream);
+            case 64 * 4 + EPI_HEAD: return launch_inst<1, 64, EPI_HEAD>(l, stream);
+            case 128 * 4 + EPI_STORE: return launch_inst<1, 128, EPI_STORE>(l, stream);
+            case 128 * 4 + EPI_STORE_POOL: return launch_inst<1, 128, EPI_STORE_POOL>(l, stream);
+        }
+    }
+    return "conv: no kernel instantiation for this (block_n, mode)";
 }
 
 }  // namespace
@@ -473,29 +544,15 @@ const char* conv_prepare(const ConvDesc& d, int num_sms, ConvLaunch* out) {
 
 int conv_grid(const ConvLaunch& l, int num_sms) {
     const ConvKernelParams& p = l.p;
+    const int ctas = l.pair ? 2 : 1;
     const long long m_tiles = static_cast<long long>(p.n_img) * p.tiles_y * p.tiles_x;
-    if (l.pair) {
-        const long long pairs = p.n_blocks * ((m_tiles + 1) / 2);
-        return static_cast<int>(2 * (pairs < num_sms / 2 ? pairs : num_sms / 2));
-    }
-    const long long tiles = p.n_blocks * m_tiles;
-    return static_cast<int>(tiles < num_sms ? tiles : num_sms);
+    const long long units = p.n_blocks * ((m_tiles + ctas - 1) / ctas);
+    return static_cast<int>(ctas * (units < num_sms / ctas ? units : num_sms / ctas));
 }
 
 const char* conv_launch(const ConvLaunch& l, cudaStream_t stream) {
-    if (l.halo) return l.pair ? conv_halo_pair_launch(l, stream) : conv_halo_launch(l, stream);
-    if (l.pair) return conv_pair_launch(l, stream);
-    switch (l.block_n * 4 + l.mode) {
-        case 64 * 4 + EPI_STORE: return launch_inst<64, EPI_STORE>(l, stream);
-        case 64 * 4 + EPI_STORE_POOL: return launch_inst<64, EPI_STORE_POOL>(l, stream);
-        case 64 * 4 + EPI_HEAD: return launch_inst<64, EPI_HEAD>(l, stream);
-        case 128 * 4 + EPI_STORE: return launch_inst<128, EPI_STORE>(l, stream);
-        case 128 * 4 + EPI_STORE_POOL: return launch_inst<128, EPI_STORE_POOL>(l, stream);
-        case 256 * 4 + EPI_STORE: return launch_inst<256, EPI_STORE>(l, stream);
-        case 256 * 4 + EPI_STORE_POOL: return launch_inst<256, EPI_STORE_POOL>(l, stream);
-        case 256 * 4 + EPI_CONVT: return launch_inst<256, EPI_CONVT>(l, stream);
-        default: return "conv: no kernel instantiation for this (block_n, mode)";
-    }
+    if (l.halo) return conv_halo_launch(l, stream);
+    return l.pair ? launch_per_tap<2>(l, stream) : launch_per_tap<1>(l, stream);
 }
 
 }  // namespace fi

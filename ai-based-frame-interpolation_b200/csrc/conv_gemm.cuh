@@ -85,8 +85,8 @@ struct ConvLaunch {
     int block_n;
     int mode;
     int split;  // 1: precise mode, epilogue writes hi + lo tensors
-    int halo;  // 1: conv_halo.cu (halo-reuse kernel for Cout 64/128), 0: conv_gemm.cu
-    int pair;  // 1: conv_gemm2.cu (CTA-pair kernel, cta_group::2) for Cout multiples of 256
+    int halo;  // 1: conv_halo.cu (halo-reuse kernel for Cout 64/128), 0: conv_gemm.cu (per-tap kernel)
+    int pair;  // 1: the family's CTA-pair kernel (cta_group::2, cluster of 2)
     int grid;
     double flops;  // algorithmic FLOPs of this launch (2*MACs, no padding counted)
 };
@@ -101,10 +101,6 @@ int conv_grid(const ConvLaunch& l, int num_sms);
 // bf16 tensor map (128B swizzle, zero OOB fill); dims/box innermost first, strides in elements for dims 1..rank-1.
 const char* encode_bf16_map_public(CUtensorMap* map, const void* base, int rank, const uint64_t* dims,
                                    const uint64_t* strides_elems, const uint32_t* box);
-
-// conv_gemm2.cu / conv_halo2.cu: CTA-pair (cta_group::2) variants
-const char* conv_pair_launch(const ConvLaunch& l, cudaStream_t stream);
-const char* conv_halo_pair_launch(const ConvLaunch& l, cudaStream_t stream);
 
 // conv_inc_fused.cu: inc.double_conv.0 (stem) computed inside inc.double_conv.3's kernel (grey network, bf16 mode)
 struct StemDesc;

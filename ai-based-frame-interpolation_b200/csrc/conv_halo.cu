@@ -9,8 +9,20 @@
 // The start address is no longer 1024 B aligned when dx != 0; the 128B-swizzle XOR is a function of the absolute smem
 // address bits [7,10), which is also what TMA used when it wrote the box, so the shifted view reads the right chunks
 // (validated on B200 against the oracle; putting the row phase into the descriptor's base-offset field instead is wrong).
-// Weights stream per (tap, slab) through their own ring. Warp roles (224 threads): 0 = A producer, 1 = TMEM owner +
-// MMA issuer, 2 = B producer, 3..6 = epilogue. TMEM: 2 accumulator sets x 2 halves x Cout columns.
+// Weights stream per (tap, slab) through their own ring. Warp roles (224 threads, 352 with two epilogue sets): 0 = A
+// producer, 1 = TMEM owner + MMA issuer, 2 = B producer, 3.. = epilogue. TMEM: 2 accumulator sets x 2 halves x Cout
+// columns.
+//
+// CTA pairs (conv_halo2_kernel, cta_group::2). The narrow layers are bound by shared-memory bandwidth: a single-CTA
+// tcgen05.mma of N = 64 reads 4 KB of A and 2 KB of B per 32 tensor-pipe cycles (measured 50.8 cycles per instruction,
+// tools/probe/mma_probe.cu), N = 128 reads 8 KB per 64 cycles while TMA fills compete for the same port. In a CTA pair
+// each SM keeps its own super tile's halo (A) but only HALF of every weight slab (Cout/2 rows); the M256 x Cout
+// instruction reads both halves. That halves the weight traffic per SM (fills and operand reads), and it lets the
+// weights of two more layers stay resident (up4.conv.0: 144 KB -> 72 KB per SM; down1.conv.0: 144 KB -> 72 KB).
+// Protocol: as the per-tap pair in conv_gemm.cu. Both CTAs run the same code on adjacent super tiles (rank picks the
+// tile); producers wait on local "empty" barriers and send completion bytes to the leader's "full" barriers; the leader
+// issues every MMA and commits with a multicast to both CTAs; epilogue warps of both CTAs release the accumulator on
+// the leader.
 #include "conv_epilogue.cuh"
 #include "conv_gemm.cuh"
 #include "ptx.cuh"
@@ -29,20 +41,20 @@ constexpr int HALO_THREADS = 224;        // 3 role warps + 4 epilogue warps (pre
 constexpr int HALO_THREADS_8 = 352;      // 3 role warps + 8 epilogue warps (one set per column half)
 constexpr int A_STAGES = 2;
 constexpr int PREFETCH_DIST = 2;         // L2-prefetch the halo boxes this many grid strides ahead (DESIGN §3 item 3)
-constexpr int B_RING_BYTES = 65536;
+constexpr int B_RING_BYTES = 65536;      // streamed weights: a ring of weight slices
+constexpr int B_REGION_BYTES = 73728;    // weight region: the ring, or up to 72 KB of resident weight slices
 constexpr int H_STAGING_PER_WARP = 2 * 4096;
 constexpr int H_POOL_PER_WARP = 2 * 1024;
 constexpr int H_BAR_BYTES = 512;
+constexpr int HALO_SMEM =
+    1024 + A_STAGES * HALO_BYTES + B_REGION_BYTES + 4 * (H_STAGING_PER_WARP + H_POOL_PER_WARP) + H_BAR_BYTES;
+static_assert(HALO_SMEM <= 232448, "halo kernel exceeds the 227 KB shared memory limit");
 
-__host__ __device__ constexpr int halo_b_stage_bytes(int cout) { return cout * 128; }
-__host__ __device__ constexpr int halo_b_stages(int cout) { return B_RING_BYTES / halo_b_stage_bytes(cout); }
-// RESIDENT: a single-slab layer (Cin = 64) keeps all nine [Cout x 64] weight slabs in smem for the CTA's lifetime.
-__host__ __device__ constexpr int halo_b_bytes(int cout, bool resident) {
-    return resident ? 9 * halo_b_stage_bytes(cout) : B_RING_BYTES;
-}
-__host__ __device__ constexpr int halo_smem_bytes(int cout, bool resident) {
-    return 1024 + A_STAGES * HALO_BYTES + halo_b_bytes(cout, resident) +
-           4 * (H_STAGING_PER_WARP + H_POOL_PER_WARP) + H_BAR_BYTES;
+// One weight slice: this CTA's rows (all Cout, or half of them in a CTA pair) of one [Cout x 64] (tap, slab) slab.
+__host__ __device__ constexpr int halo_b_stage_bytes(int ctas, int cout) { return cout / ctas * 128; }
+// RESIDENT: all 9 x slabs weight slices this CTA holds fit in the weight region and stay for the CTA's lifetime.
+__host__ __device__ constexpr bool halo_resident_fits(int ctas, int cout, int slabs) {
+    return 9 * slabs * halo_b_stage_bytes(ctas, cout) <= B_REGION_BYTES;
 }
 
 __device__ __forceinline__ uint64_t halo_desc(uint32_t smem_addr) {
@@ -55,28 +67,34 @@ __device__ __forceinline__ uint64_t halo_desc(uint32_t smem_addr) {
     return d;
 }
 
-struct HTile {
-    int img, y0, x0;
+struct Unit {
+    HaloTile t;
+    bool valid;  // false: odd tile count, the last pair's second CTA recomputes the last tile with its stores off
 };
-__device__ __forceinline__ HTile decode_htile(int t, const ConvKernelParams& p) {
+template <int CTAS>
+__device__ __forceinline__ Unit decode_unit(int u, uint32_t rank, const ConvKernelParams& p) {
     const int per_img = p.tiles_y * p.tiles_x;
-    HTile c;
-    c.img = t / per_img;
-    int m = t - c.img * per_img;
+    const int tiles = p.n_img * per_img;
+    int m = CTAS * u + static_cast<int>(rank);
+    Unit r;
+    r.valid = CTAS == 1 || m < tiles;
+    if (!r.valid) m = tiles - 1;
+    r.t.img = m / per_img;
+    m -= r.t.img * per_img;
     const int ty = m / p.tiles_x;
-    c.y0 = ty * HT;
-    c.x0 = (m - ty * p.tiles_x) * HT;
-    return c;
+    r.t.y0 = ty * HT;
+    r.t.x0 = (m - ty * p.tiles_x) * HT;
+    return r;
 }
 
-template <int COUT, int MODE, bool RESIDENT, bool SPLIT>
-__global__ void __launch_bounds__(SPLIT ? HALO_THREADS : HALO_THREADS_8, 1)
-conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p) {
-    constexpr int B_STAGES = halo_b_stages(COUT);
-    constexpr int B_STAGE_BYTES = halo_b_stage_bytes(COUT);
+// CTAS = 1: one CTA per super tile. CTAS = 2: a CTA pair (cluster of 2) computes two adjacent super tiles.
+template <int CTAS, int COUT, int MODE, bool RESIDENT, bool SPLIT>
+__device__ __forceinline__ void conv_halo_body(const ConvMaps& maps, const ConvKernelParams& p) {
+    constexpr int B_STAGE_BYTES = halo_b_stage_bytes(CTAS, COUT);
+    constexpr int B_STAGES = B_RING_BYTES / B_STAGE_BYTES;  // ring depth when streaming
     constexpr int ACC_COLS = 2 * COUT;          // two column halves
     constexpr int TMEM_COLS = 2 * ACC_COLS;     // double buffered: 256 (Cout 64) or 512 (Cout 128)
-    constexpr uint32_t IDESC = umma_idesc_bf16(128, COUT);
+    constexpr uint32_t IDESC = umma_idesc_bf16(128 * CTAS, COUT);
     static_assert(MODE != EPI_HEAD || COUT == 64, "head epilogue consumes exactly 64 channels");
     // bf16 mode: 8 epilogue warps, one set of 4 per column half, single staging tile each; precise mode: 4 warps
     constexpr int EPI_SETS = SPLIT ? 1 : 2;
@@ -87,7 +105,7 @@ conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     const uint32_t smem_a = smem_base;
     const uint32_t smem_b = smem_a + A_STAGES * HALO_BYTES;
-    const uint32_t smem_stage = smem_b + halo_b_bytes(COUT, RESIDENT);
+    const uint32_t smem_stage = smem_b + B_REGION_BYTES;
     const uint32_t smem_pool = smem_stage + 4 * H_STAGING_PER_WARP;
     const uint32_t smem_bar = smem_pool + 4 * H_POOL_PER_WARP;
     const uint32_t bar_afull = smem_bar;                       // A_STAGES
@@ -102,6 +120,8 @@ conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
+    const uint32_t rank = CTAS == 1 ? 0 : cluster_ctarank();
+    const bool leader = CTAS == 1 || rank == 0;
 
     if (warp == 0 && lane == 0) {
         tma_prefetch_desc(&maps.a[0]);
@@ -119,34 +139,38 @@ conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
         }
         for (int a = 0; a < 2; ++a) {
             mbar_init(bar_tfull + 8 * a, 1);
-            mbar_init(bar_tempty + 8 * a, 4 * EPI_SETS);
+            mbar_init(bar_tempty + 8 * a, 4 * EPI_SETS * CTAS);  // one arrive per epilogue warp (of both CTAs)
         }
         mbar_init(bar_bres, 1);
         fence_mbar_init();
     }
-    if (warp == 1) tmem_alloc(tmem_slot, TMEM_COLS);
+    if (warp == 1) tmem_alloc<CTAS>(tmem_slot, TMEM_COLS);
     tc_fence_before();
     __syncthreads();
+    if constexpr (CTAS == 2) cluster_sync_all();  // both CTAs' barriers exist before any remote signal can arrive
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot_ptr;
     pdl_launch_dependents();
     pdl_wait();
 
-    const int total_tiles = p.n_img * p.tiles_y * p.tiles_x;
+    const int units = (p.n_img * p.tiles_y * p.tiles_x + CTAS - 1) / CTAS;
+    const int unit0 = static_cast<int>(blockIdx.x / CTAS);
+    const int unit_step = static_cast<int>(gridDim.x / CTAS);
     const int slabs = p.slabs;
+    const int b_row0 = static_cast<int>(rank) * (COUT / CTAS);  // this CTA's rows of every weight slab
 
     if (warp == 0) {
         // ------------------------------------------------------------ A producer: one halo box per (tile, slab)
         {
             int stage = 0;
             uint32_t phase = 0;
-            for (int t = blockIdx.x; t < total_tiles; t += gridDim.x) {
-                const HTile tc = decode_htile(t, p);
+            for (int u = unit0; u < units; u += unit_step) {
+                const HaloTile tc = decode_unit<CTAS>(u, rank, p).t;
                 // Only A_STAGES-1 halo boxes can be in flight towards smem, which does not cover HBM latency:
                 // pull the boxes of this CTA's tile after next into L2 now (no smem needed for that).
-                const int tp = t + PREFETCH_DIST * static_cast<int>(gridDim.x);
-                if (tp < total_tiles && lane == 0) {
-                    const HTile pc = decode_htile(tp, p);
+                const int up = u + PREFETCH_DIST * unit_step;
+                if (up < units && lane == 0) {
+                    const HaloTile pc = decode_unit<CTAS>(up, rank, p).t;
                     for (int g = 0; g < p.nseg; ++g) {
                         const int mid = p.seg_map[g];
                         if (g > 0 && p.seg_map[g - 1] == mid) continue;  // same tensor as the previous segment
@@ -164,10 +188,10 @@ conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
                     mbar_wait(bar_aempty + 8 * stage, phase ^ 1);
                     const uint32_t full = bar_afull + 8 * stage;
                     if (elect_one()) {
-                        mbar_expect_tx(full, HALO_BYTES);
+                        if (leader) mbar_expect_tx(full, CTAS * HALO_BYTES);
                         const int ox = mid >= 2 ? p.off_x : 0, oy = mid >= 2 ? p.off_y : 0;  // F.pad of src1
-                        tma_load_4d(smem_a + stage * HALO_BYTES, &maps.a[mid], full, local * BLOCK_K, tc.x0 - 1 - ox,
-                                    tc.y0 - 1 - oy, tc.img);
+                        tma_load_4d<CTAS>(smem_a + stage * HALO_BYTES, &maps.a[mid], full, local * BLOCK_K,
+                                          tc.x0 - 1 - ox, tc.y0 - 1 - oy, tc.img);
                     }
                     __syncwarp();
                     if (++stage == A_STAGES) {
@@ -178,24 +202,28 @@ conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
             }
         }
     } else if (warp == 2) {
-        // ------------------------------------------------------------ B producer: one [Cout x 64] weight slab per tap
+        // ------------------------------------------------------------ B producer: one weight slice per (slab, tap)
         if (RESIDENT) {
             if (lane == 0) {
-                mbar_expect_tx(bar_bres, 9 * B_STAGE_BYTES);
-                for (int tap = 0; tap < 9; ++tap)
-                    tma_load_2d(smem_b + tap * B_STAGE_BYTES, &maps.b, bar_bres, tap * BLOCK_K, 0);
+                const int res_slabs = CTAS == 1 ? 1 : slabs;  // a single CTA holds Cout 64 x Cin 64 only (72 KB)
+                if (leader) mbar_expect_tx(bar_bres, CTAS * 9 * res_slabs * B_STAGE_BYTES);
+                for (int s = 0; s < res_slabs; ++s)
+                    for (int tap = 0; tap < 9; ++tap)
+                        tma_load_2d<CTAS>(smem_b + (s * 9 + tap) * B_STAGE_BYTES, &maps.b, bar_bres,
+                                          (tap * slabs + s) * BLOCK_K, b_row0);
             }
         } else {
             int stage = 0;
             uint32_t phase = 0;
-            for (int t = blockIdx.x; t < total_tiles; t += gridDim.x) {
+            for (int u = unit0; u < units; u += unit_step) {
                 for (int s = 0; s < slabs; ++s) {
                     for (int tap = 0; tap < 9; ++tap) {
                         mbar_wait(bar_bempty + 8 * stage, phase ^ 1);
                         const uint32_t full = bar_bfull + 8 * stage;
                         if (elect_one()) {
-                            mbar_expect_tx(full, B_STAGE_BYTES);
-                            tma_load_2d(smem_b + stage * B_STAGE_BYTES, &maps.b, full, (tap * slabs + s) * BLOCK_K, 0);
+                            if (leader) mbar_expect_tx(full, CTAS * B_STAGE_BYTES);
+                            tma_load_2d<CTAS>(smem_b + stage * B_STAGE_BYTES, &maps.b, full,
+                                              (tap * slabs + s) * BLOCK_K, b_row0);
                         }
                         __syncwarp();
                         if (++stage == B_STAGES) {
@@ -207,13 +235,14 @@ conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
             }
         }
     } else if (warp == 1) {
-        // ------------------------------------------------------------ MMA issuer (warp converged, one elected lane issues)
-        {
+        // ------------------------------------------------------------ MMA issuer (warp converged, one elected lane
+        // issues; a pair's MMAs are all issued by the leader CTA)
+        if (leader) {
             int a_stage = 0, b_stage = 0;
             uint32_t a_phase = 0, b_phase = 0;
             int it = 0;
             if (RESIDENT) mbar_wait(bar_bres, 0);
-            for (int t = blockIdx.x; t < total_tiles; t += gridDim.x, ++it) {
+            for (int u = unit0; u < units; u += unit_step, ++it) {
                 const int acc = it & 1;
                 const uint32_t acc_phase = (it >> 1) & 1;
                 mbar_wait(bar_tempty + 8 * acc, acc_phase ^ 1);
@@ -227,7 +256,7 @@ conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
                         tc_fence_after();
                         const int dy = tap / 3, dx = tap - 3 * dy;
                         const uint64_t db =
-                            umma_desc_sw128(smem_b + (RESIDENT ? tap : b_stage) * B_STAGE_BYTES);
+                            umma_desc_sw128(smem_b + (RESIDENT ? s * 9 + tap : b_stage) * B_STAGE_BYTES);
                         const uint64_t da0 = halo_desc(a_base + (dy * HALO_W + dx) * 128);
                         if (elect_one()) {
                             // The two column halves are independent accumulators: alternating them keeps back-to-back
@@ -237,14 +266,14 @@ conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
 #pragma unroll
                                 for (int half = 0; half < 2; ++half) {
                                     // +8 pixels (1024 B) per column half, +32 B per K step, in 16-byte units
-                                    umma_bf16_ss(d_tmem + half * COUT, da0 + 64 * half + 2 * k, db + 2 * k, IDESC,
-                                                 (s | tap | k) != 0);
+                                    umma_bf16_ss<CTAS>(d_tmem + half * COUT, da0 + 64 * half + 2 * k, db + 2 * k,
+                                                       IDESC, (s | tap | k) != 0);
                                 }
                             }
-                            if (!RESIDENT) umma_commit(bar_bempty + 8 * b_stage);
+                            if (!RESIDENT) umma_commit<CTAS>(bar_bempty + 8 * b_stage);
                             if (tap == 8) {
-                                umma_commit(bar_aempty + 8 * a_stage);
-                                if (s == slabs - 1) umma_commit(bar_tfull + 8 * acc);
+                                umma_commit<CTAS>(bar_aempty + 8 * a_stage);
+                                if (s == slabs - 1) umma_commit<CTAS>(bar_tfull + 8 * acc);
                             }
                         }
                         __syncwarp();
@@ -263,7 +292,7 @@ conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
             }
         }
     } else {
-        // ------------------------------------------------------------ epilogue warps 3..6
+        // ------------------------------------------------------------ epilogue warps 3..6 (3..10 with two sets)
         const int q = warp & 3;  // TMEM lanes [32q, 32q+32) <-> tile rows 4q..4q+3, 8 columns of one half
         const int ew = warp - 3;          // 0..7 (0..3 in precise mode)
         const int set = ew >> 2;          // which column half this warp drains (bf16 mode)
@@ -271,8 +300,8 @@ conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
         const uint32_t my_pool = smem_pool + ew * POOL_PER_WARP;
         int buf = 0;
         int it = 0;
-        for (int t = blockIdx.x; t < total_tiles; t += gridDim.x, ++it) {
-            const HTile tc = decode_htile(t, p);
+        for (int u = unit0; u < units; u += unit_step, ++it) {
+            const Unit w = decode_unit<CTAS>(u, rank, p);
             const int acc = it & 1;
             const uint32_t acc_phase = (it >> 1) & 1;
             mbar_wait(bar_tfull + 8 * acc, acc_phase);
@@ -280,12 +309,15 @@ conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
             const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * ACC_COLS;
 #pragma unroll 1
             for (int c = set * (ACC_COLS / 64 / EPI_SETS); c < (set + 1) * (ACC_COLS / 64 / EPI_SETS); ++c) {
-                epilogue_chunk_halo<COUT, MODE, SPLIT, SPLIT>(maps, p, HaloTile{tc.img, tc.y0, tc.x0}, taddr, c, q, lane, my_stage,
-                                                       my_pool, buf, true);
+                epilogue_chunk_halo<COUT, MODE, SPLIT, SPLIT>(maps, p, w.t, taddr, c, q, lane, my_stage, my_pool, buf,
+                                                              w.valid);
             }
             tc_fence_before();
             __syncwarp();
-            if (elect_one()) mbar_arrive(bar_tempty + 8 * acc);
+            if (elect_one()) {
+                if (leader) mbar_arrive(bar_tempty + 8 * acc);
+                else mbar_arrive_cluster(bar_tempty + 8 * acc, 0);
+            }
         }
         __syncwarp();
         if (MODE != EPI_HEAD && elect_one()) tma_store_wait_all();
@@ -293,28 +325,54 @@ conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p
 
     tc_fence_before();
     __syncthreads();
+    if constexpr (CTAS == 2) cluster_sync_all();  // the peer may still be reading TMEM / receiving commits
     if (warp == 1) {
         tc_fence_after();
-        tmem_dealloc(tmem_base, TMEM_COLS);
+        tmem_dealloc<CTAS>(tmem_base, TMEM_COLS);
     }
 }
 
-template <int COUT, int MODE, bool RESIDENT = false, bool SPLIT = false>
-const char* launch_halo_inst(const ConvLaunch& l, cudaStream_t stream) {
-    if constexpr (COUT == 64 && !RESIDENT && !SPLIT) {
-        if (l.p.slabs == 1 && !l.split) return launch_halo_inst<COUT, MODE, true, false>(l, stream);
-    }
+template <int COUT, int MODE, bool RESIDENT, bool SPLIT>
+__global__ void __launch_bounds__(SPLIT ? HALO_THREADS : HALO_THREADS_8, 1)
+conv_halo_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p) {
+    conv_halo_body<1, COUT, MODE, RESIDENT, SPLIT>(maps, p);
+}
+
+template <int COUT, int MODE, bool RESIDENT, bool SPLIT>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(SPLIT ? HALO_THREADS : HALO_THREADS_8, 1)
+conv_halo2_kernel(const __grid_constant__ ConvMaps maps, const ConvKernelParams p) {
+    conv_halo_body<2, COUT, MODE, RESIDENT, SPLIT>(maps, p);
+}
+
+template <int CTAS, int COUT, int MODE, bool RESIDENT = false, bool SPLIT = false>
+const char* launch_inst(const ConvLaunch& l, cudaStream_t stream) {
     if constexpr (!SPLIT && !RESIDENT && MODE != EPI_HEAD) {
-        if (l.split) return launch_halo_inst<COUT, MODE, false, true>(l, stream);
+        if (l.split) return launch_inst<CTAS, COUT, MODE, false, true>(l, stream);
     }
-    auto kfn = conv_halo_kernel<COUT, MODE, RESIDENT, SPLIT>;
+    // Only where some layer can satisfy the rule: a precise-mode layer has at least 3 slabs.
+    if constexpr (!RESIDENT && halo_resident_fits(CTAS, COUT, SPLIT ? 3 : 1)) {
+        if (halo_resident_fits(CTAS, COUT, l.p.slabs)) return launch_inst<CTAS, COUT, MODE, true, SPLIT>(l, stream);
+    }
+    void (*kfn)(ConvMaps, ConvKernelParams);
+    if constexpr (CTAS == 1) kfn = conv_halo_kernel<COUT, MODE, RESIDENT, SPLIT>;
+    else kfn = conv_halo2_kernel<COUT, MODE, RESIDENT, SPLIT>;
     static std::atomic<uint64_t> configured{0};  // per instantiation: devices with the shared-memory opt-in
-    constexpr int smem = halo_smem_bytes(COUT, RESIDENT);
-    static_assert(smem <= 232448, "halo kernel exceeds the 227 KB shared memory limit");
-    if (!smem_opt_in(kfn, smem, configured)) return "cudaFuncSetAttribute(MaxDynamicSharedMemorySize) failed";
-    const cudaError_t e = launch_kernel(kfn, dim3(l.grid), dim3(SPLIT ? HALO_THREADS : HALO_THREADS_8), smem, stream,
-                                        l.maps, l.p);
+    if (!smem_opt_in(kfn, HALO_SMEM, configured)) return "cudaFuncSetAttribute(MaxDynamicSharedMemorySize) failed";
+    const cudaError_t e = launch_kernel(kfn, dim3(l.grid), dim3(SPLIT ? HALO_THREADS : HALO_THREADS_8), HALO_SMEM,
+                                        stream, l.maps, l.p);
     return e == cudaSuccess ? nullptr : cudaGetErrorString(e);
+}
+
+template <int CTAS>
+const char* launch_halo(const ConvLaunch& l, cudaStream_t stream) {
+    switch (l.block_n * 4 + l.mode) {
+        case 64 * 4 + EPI_STORE: return launch_inst<CTAS, 64, EPI_STORE>(l, stream);
+        case 64 * 4 + EPI_STORE_POOL: return launch_inst<CTAS, 64, EPI_STORE_POOL>(l, stream);
+        case 64 * 4 + EPI_HEAD: return launch_inst<CTAS, 64, EPI_HEAD>(l, stream);
+        case 128 * 4 + EPI_STORE: return launch_inst<CTAS, 128, EPI_STORE>(l, stream);
+        case 128 * 4 + EPI_STORE_POOL: return launch_inst<CTAS, 128, EPI_STORE_POOL>(l, stream);
+        default: return "conv(halo): no kernel instantiation for this (cout, mode)";
+    }
 }
 
 }  // namespace
@@ -337,14 +395,7 @@ void conv_halo_geometry(int* tile, int* box_w, int* box_h, int* out_w, int* out_
 }
 
 const char* conv_halo_launch(const ConvLaunch& l, cudaStream_t stream) {
-    switch (l.block_n * 4 + l.mode) {
-        case 64 * 4 + EPI_STORE: return launch_halo_inst<64, EPI_STORE>(l, stream);
-        case 64 * 4 + EPI_STORE_POOL: return launch_halo_inst<64, EPI_STORE_POOL>(l, stream);
-        case 64 * 4 + EPI_HEAD: return launch_halo_inst<64, EPI_HEAD>(l, stream);
-        case 128 * 4 + EPI_STORE: return launch_halo_inst<128, EPI_STORE>(l, stream);
-        case 128 * 4 + EPI_STORE_POOL: return launch_halo_inst<128, EPI_STORE_POOL>(l, stream);
-        default: return "conv(halo): no kernel instantiation for this (cout, mode)";
-    }
+    return l.pair ? launch_halo<2>(l, stream) : launch_halo<1>(l, stream);
 }
 
 }  // namespace fi

@@ -126,23 +126,66 @@ __device__ __forceinline__ void tc_fence_after() {
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 }
 
+// ------------------------------------------------------------------ CTA pairs (cta_group::2, cluster of 2)
+// A shared::cta address carries the CTA's rank within the pair in bit 24 when used as a shared::cluster address;
+// clearing it addresses the same offset in CTA 0 (the MMA leader).
+constexpr uint32_t PEER_BIT_MASK = 0xFEFFFFFFu;
+
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+    uint32_t r;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+    return r;
+}
+__device__ __forceinline__ void cluster_sync_all() {  // every thread of both CTAs
+    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// Arrive on the mbarrier at the same offset in CTA `cta` of the cluster.
+__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar, uint32_t cta) {
+    asm volatile(
+        "{\n\t.reg .b32 ra;\n\t"
+        "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
+        "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}"
+        ::"r"(bar), "r"(cta)
+        : "memory");
+}
+
 // ------------------------------------------------------------------ TMA
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* m) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(m)) : "memory");
 }
+// CTAS = 1: data and completion bytes go to this CTA. CTAS = 2 (CTA pair): data lands in the executing CTA's smem,
+// completion bytes go to the LEADER's mbarrier.
+template <int CTAS = 1>
 __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1)
-        : "memory");
+    if constexpr (CTAS == 1) {
+        asm volatile(
+            "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+            ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1)
+            : "memory");
+    } else {
+        asm volatile(
+            "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, "
+            "%4}], [%2];" ::"r"(dst),
+            "l"(reinterpret_cast<uint64_t>(m)), "r"(bar & PEER_BIT_MASK), "r"(c0), "r"(c1)
+            : "memory");
+    }
 }
+template <int CTAS = 1>
 __device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2,
                                             int c3) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], "
-        "[%2];" ::"r"(dst),
-        "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-        : "memory");
+    if constexpr (CTAS == 1) {
+        asm volatile(
+            "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], "
+            "[%2];" ::"r"(dst),
+            "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+            : "memory");
+    } else {
+        asm volatile(
+            "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, "
+            "%4, %5, %6}], [%2];" ::"r"(dst),
+            "l"(reinterpret_cast<uint64_t>(m)), "r"(bar & PEER_BIT_MASK), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+            : "memory");
+    }
 }
 // Pull a box into L2 only (no smem, no barrier): lets the real load of a later tile hit L2 instead of HBM.
 __device__ __forceinline__ void tma_prefetch_l2_4d(const CUtensorMap* m, int c0, int c1, int c2, int c3) {
@@ -172,14 +215,25 @@ __device__ __forceinline__ void tma_store_wait_read() {
 __device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
 // ------------------------------------------------------------------ TMEM
-// One full warp executes alloc / dealloc (.sync.aligned).
+// One full warp executes alloc / dealloc (.sync.aligned); in a CTA pair (CTAS = 2) the same warp of both CTAs.
+template <int CTAS = 1>
 __device__ __forceinline__ void tmem_alloc(uint32_t smem_dst, uint32_t ncols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(ncols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    if constexpr (CTAS == 1) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(ncols)
+                     : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    } else {
+        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(ncols)
+                     : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    }
 }
+template <int CTAS = 1>
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+    if constexpr (CTAS == 1)
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+    else
+        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
@@ -197,22 +251,41 @@ __device__ __forceinline__ void tmem_ld_32x32b_x32(uint32_t taddr, uint32_t (&r)
         : "memory");
 }
 
-// ------------------------------------------------------------------ tcgen05.mma (single CTA, bf16/f16 -> fp32)
-// D[tmem] (+)= A[smem desc] * B[smem desc]; issued by ONE thread.
+// ------------------------------------------------------------------ tcgen05.mma (bf16/f16 -> fp32)
+// D[tmem] (+)= A[smem desc] * B[smem desc]; issued by ONE thread. CTAS = 2: D[256 x N] (+)= A[256 x 16] * B[N x 16]^T
+// over the CTA pair, each CTA holding its own 128 rows of A and half of B; issued by one thread of the leader CTA.
+template <int CTAS = 1>
 __device__ __forceinline__ void umma_bf16_ss(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
                                              uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-        : "memory");
+    if constexpr (CTAS == 1) {
+        asm volatile(
+            "{\n\t.reg .pred p;\n\t"
+            "setp.ne.b32 p, %4, 0;\n\t"
+            "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+            ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+            : "memory");
+    } else {
+        asm volatile(
+            "{\n\t.reg .pred p;\n\t"
+            "setp.ne.b32 p, %4, 0;\n\t"
+            "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+            ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+            : "memory");
+    }
 }
 // Arrive on an mbarrier once every previously issued tcgen05.mma of this thread has completed
-// (implies tcgen05.fence::before_thread_sync).
+// (implies tcgen05.fence::before_thread_sync). CTAS = 2: on the mbarrier at this offset in BOTH CTAs.
+template <int CTAS = 1>
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar)
-                 : "memory");
+    if constexpr (CTAS == 1) {
+        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar)
+                     : "memory");
+    } else {
+        asm volatile(
+            "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+            ::"r"(bar), "h"(static_cast<uint16_t>(3))
+            : "memory");
+    }
 }
 
 // K-major, 128-byte-swizzled operand tile (rows of 128 B, 8-row atoms of 1024 B):
@@ -252,70 +325,6 @@ __device__ __forceinline__ uint32_t bf16x2_max(uint32_t a, uint32_t b) {
     uint32_t r;
     asm("max.bf16x2 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b));
     return r;
-}
-
-// ------------------------------------------------------------------ CTA pairs (cta_group::2, cluster of 2)
-// A shared::cta address carries the CTA's rank within the pair in bit 24 when used as a shared::cluster address;
-// clearing it addresses the same offset in CTA 0 (the MMA leader).
-constexpr uint32_t PEER_BIT_MASK = 0xFEFFFFFFu;
-
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {  // every thread of both CTAs
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// TMA loads of a CTA pair: data lands in the executing CTA's smem, completion bytes go to the LEADER's mbarrier.
-__device__ __forceinline__ void tma_load_2d_2sm(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], "
-        "[%2];" ::"r"(dst),
-        "l"(reinterpret_cast<uint64_t>(m)), "r"(bar & PEER_BIT_MASK), "r"(c0), "r"(c1)
-        : "memory");
-}
-__device__ __forceinline__ void tma_load_4d_2sm(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1,
-                                                int c2, int c3) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, "
-        "%5, %6}], [%2];" ::"r"(dst),
-        "l"(reinterpret_cast<uint64_t>(m)), "r"(bar & PEER_BIT_MASK), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_2sm(uint32_t smem_dst, uint32_t ncols) {  // same warp id in both CTAs
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(ncols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_2sm(uint32_t taddr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-// D[256 x N] (+)= A[256 x 16] * B[N x 16]^T over the CTA pair; issued by one thread of the leader CTA.
-__device__ __forceinline__ void umma_bf16_ss_2sm(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                                 uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// Arrive on the mbarrier at this offset in BOTH CTAs once the leader's previously issued MMAs have completed.
-__device__ __forceinline__ void umma_commit_2sm(uint32_t bar) {
-    asm volatile(
-        "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-        "h"(static_cast<uint16_t>(3))
-        : "memory");
-}
-// Arrive on the mbarrier at the same offset in CTA `cta` of the cluster.
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar, uint32_t cta) {
-    asm volatile(
-        "{\n\t.reg .b32 ra;\n\t"
-        "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-        "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}"
-        ::"r"(bar), "r"(cta)
-        : "memory");
 }
 
 // ------------------------------------------------------------------ precise mode helpers (value = bf16 hi + bf16 lo)

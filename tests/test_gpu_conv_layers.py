@@ -13,8 +13,9 @@ pytestmark = pytest.mark.gpu
 
 @pytest.fixture(params=["halo", "per-tap", "pair"], autouse=True)
 def kernel_variant(request, monkeypatch):
-    """Cout 64/128 layers have two kernels (conv_halo.cu / conv_gemm.cu) and Cout multiples of 256 have the single-CTA
-    and the CTA-pair kernel (conv_gemm.cu / conv_gemm2.cu); run every case through all selections."""
+    """Cout 64/128 layers have two kernel families (halo reuse in conv_halo.cu, per tap in conv_gemm.cu), and the halo
+    family and the Cout-multiple-of-256 per-tap kernels each run as one CTA or as a CTA pair; run every case through
+    all selections."""
     monkeypatch.setenv("FI_NO_HALO", "1" if request.param == "per-tap" else "0")
     monkeypatch.setenv("FI_CTA2", "1" if request.param == "pair" else "0")
     return request.param
