@@ -146,20 +146,18 @@ struct fiNet {
     bool profiling = false;
     std::vector<cudaEvent_t> prof_events;  // [call][step][2], resolved by fiNetGetProfile
     int prof_calls = 0;
-    // clip pipeline (fiNetInterpolateClipHostU8): double-buffered pinned + device staging, copy streams, events
+    // host-clip pipeline (fiNetInterpolateDyadicHostU8): double-buffered pinned + device staging, copy streams, events
     struct ClipSlot {
         void* pin_in = nullptr;
-        void* pin_out = nullptr;
         void* dev_in = nullptr;
-        void* dev_out = nullptr;
         cudaEvent_t in_ready = nullptr, done = nullptr, out_ready = nullptr;
-        uint64_t* pin_sad = nullptr;  // per-pair SAD of the batch (fiNetInterpolateClipHostU8Sad only)
+        uint64_t* pin_sad = nullptr;  // per-pair SAD of the group (when the caller asks for it)
         uint64_t* dev_sad = nullptr;
-        DevBuf pool;                  // fiNetInterpolateDyadicHostU8: every node of the group's bisection tree
+        DevBuf pool;                  // every node of the group's bisection tree
         void* pin_nodes = nullptr;    // ... and the requested nodes on their way to the host
         size_t pin_nodes_bytes = 0;
     } clip[2];
-    size_t clip_in_bytes = 0, clip_out_bytes = 0;
+    size_t clip_in_bytes = 0;
     int clip_sad_pairs = 0;  // capacity of pin_sad / dev_sad
     cudaStream_t clip_h2d = nullptr, clip_d2h = nullptr;
     DevBuf dyadic_gather;    // in0 | in1 of one bisection forward: the parents of up to pairs_per_batch nodes
@@ -677,10 +675,9 @@ struct DeviceGuard {
     DeviceGuard _device_guard(device); \
     if (_device_guard.rc) return _device_guard.rc
 
-// Copy streams, events and the double-buffered staging of the pipelined host-clip calls: per slot at least in_bytes of
-// pinned and device input, out_bytes of pinned and device output (0: none needed), and with `sad` B per-pair SAD values.
-// Buffers only grow: a reallocation keeps the larger of the held and the asked sizes.
-int clip_staging(fiNet* net, int B, size_t in_bytes, size_t out_bytes, bool sad) {
+// Copy streams, events and the double-buffered input staging of the pipelined host-clip call: per slot at least
+// in_bytes of pinned and device input, and with `sad` B per-pair SAD values. Buffers only grow.
+int clip_staging(fiNet* net, int B, size_t in_bytes, bool sad) {
     if (!net->clip_h2d) {
         CUDA_TRY(cudaStreamCreateWithFlags(&net->clip_h2d, cudaStreamNonBlocking));
         CUDA_TRY(cudaStreamCreateWithFlags(&net->clip_d2h, cudaStreamNonBlocking));
@@ -690,28 +687,19 @@ int clip_staging(fiNet* net, int B, size_t in_bytes, size_t out_bytes, bool sad)
             CUDA_TRY(cudaEventCreateWithFlags(&c.out_ready, cudaEventDisableTiming));
         }
     }
-    if (net->clip_in_bytes < in_bytes || net->clip_out_bytes < out_bytes) {
-        in_bytes = std::max(in_bytes, net->clip_in_bytes);
-        out_bytes = std::max(out_bytes, net->clip_out_bytes);
+    if (net->clip_in_bytes < in_bytes) {
         CUDA_TRY(cudaDeviceSynchronize());
         for (auto& c : net->clip) {
             if (c.pin_in) cudaFreeHost(c.pin_in);
-            if (c.pin_out) cudaFreeHost(c.pin_out);
             if (c.dev_in) cudaFree(c.dev_in);
-            if (c.dev_out) cudaFree(c.dev_out);
-            c.pin_in = c.pin_out = c.dev_in = c.dev_out = nullptr;
+            c.pin_in = c.dev_in = nullptr;
         }
-        net->clip_in_bytes = net->clip_out_bytes = 0;
+        net->clip_in_bytes = 0;
         for (auto& c : net->clip) {
             CUDA_TRY(cudaMallocHost(&c.pin_in, in_bytes));
             CUDA_TRY(cudaMalloc(&c.dev_in, in_bytes));
-            if (out_bytes) {
-                CUDA_TRY(cudaMallocHost(&c.pin_out, out_bytes));
-                CUDA_TRY(cudaMalloc(&c.dev_out, out_bytes));
-            }
         }
         net->clip_in_bytes = in_bytes;
-        net->clip_out_bytes = out_bytes;
     }
     if (sad && net->clip_sad_pairs < B) {
         CUDA_TRY(cudaDeviceSynchronize());
@@ -798,9 +786,7 @@ int fiNetDestroy(fiNet* net) {
     for (cudaEvent_t e : net->prof_events) cudaEventDestroy(e);
     for (auto& c : net->clip) {
         if (c.pin_in) cudaFreeHost(c.pin_in);
-        if (c.pin_out) cudaFreeHost(c.pin_out);
         if (c.dev_in) cudaFree(c.dev_in);
-        if (c.dev_out) cudaFree(c.dev_out);
         if (c.pin_sad) cudaFreeHost(c.pin_sad);
         if (c.dev_sad) cudaFree(c.dev_sad);
         if (c.pin_nodes) cudaFreeHost(c.pin_nodes);
@@ -1046,89 +1032,6 @@ int fiNetInterpolateHostU8(fiNet* net, const uint8_t* frame1_host, const uint8_t
     return FI_OK;
 }
 
-int fiNetInterpolateClipHostU8(fiNet* net, const uint8_t* frames_host, int n_frames, int channels_per_frame,
-                               uint8_t* out_host, int H, int W, int pairs_per_batch, void* stream) {
-    if (!net) return fail(FI_ERR_INVALID, "null argument");
-    return fiNetInterpolateClipHostU8Strided(net, frames_host, static_cast<int64_t>(channels_per_frame) * H * W, n_frames,
-                                             channels_per_frame, out_host, static_cast<int64_t>(net->n_classes) * H * W, H,
-                                             W, pairs_per_batch, stream);
-}
-
-int fiNetInterpolateClipHostU8Strided(fiNet* net, const uint8_t* frames_host, int64_t frame_stride, int n_frames,
-                                      int channels_per_frame, uint8_t* out_host, int64_t out_stride, int H, int W,
-                                      int pairs_per_batch, void* stream) {
-    return fiNetInterpolateClipHostU8Sad(net, frames_host, frame_stride, n_frames, channels_per_frame, out_host,
-                                         out_stride, H, W, pairs_per_batch, stream, nullptr);
-}
-
-int fiNetInterpolateClipHostU8Sad(fiNet* net, const uint8_t* frames_host, int64_t frame_stride, int n_frames,
-                                  int channels_per_frame, uint8_t* out_host, int64_t out_stride, int H, int W,
-                                  int pairs_per_batch, void* stream, uint64_t* pair_sad_host) {
-    if (!net || !frames_host || !out_host) return fail(FI_ERR_INVALID, "null argument");
-    if (2 * channels_per_frame != net->n_channels)
-        return fail(FI_ERR_INVALID, "2 x %d channels per frame != n_channels %d", channels_per_frame, net->n_channels);
-    if (n_frames < 2 || H <= 0 || W <= 0 || pairs_per_batch < 1) return fail(FI_ERR_INVALID, "empty clip or batch");
-    ON_DEVICE(net->device);
-    int rc = FI_OK;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const int B = pairs_per_batch;
-    const size_t frame_bytes = static_cast<size_t>(channels_per_frame) * H * W;
-    const size_t outf_bytes = static_cast<size_t>(net->n_classes) * H * W;
-    const size_t in_bytes = (B + 1) * frame_bytes, out_bytes = B * outf_bytes;
-    if (frame_stride < static_cast<int64_t>(frame_bytes) || out_stride < static_cast<int64_t>(outf_bytes))
-        return fail(FI_ERR_INVALID, "frame strides are smaller than a frame");
-    if ((rc = clip_staging(net, B, in_bytes, out_bytes, pair_sad_host != nullptr))) return rc;
-    const int n_pairs = n_frames - 1;
-    const int n_batches = (n_pairs + B - 1) / B;
-    auto collect = [&](int b) -> int {  // wait for batch b's D2H and hand its frames to the caller
-        fiNet::ClipSlot& c = net->clip[b & 1];
-        CUDA_TRY(cudaEventSynchronize(c.out_ready));
-        const int first = b * B;
-        const int cnt = n_pairs - first < B ? n_pairs - first : B;
-        if (out_stride == static_cast<int64_t>(outf_bytes)) {
-            memcpy(out_host + static_cast<size_t>(first) * outf_bytes, c.pin_out, cnt * outf_bytes);
-        } else {
-            for (int i = 0; i < cnt; ++i)
-                memcpy(out_host + static_cast<int64_t>(first + i) * out_stride,
-                       static_cast<const char*>(c.pin_out) + i * outf_bytes, outf_bytes);
-        }
-        if (pair_sad_host) memcpy(pair_sad_host + first, c.pin_sad, cnt * sizeof(uint64_t));
-        return FI_OK;
-    };
-    for (int b = 0; b < n_batches; ++b) {
-        fiNet::ClipSlot& c = net->clip[b & 1];
-        const int first = b * B;
-        const int cnt = n_pairs - first < B ? n_pairs - first : B;
-        // slot reuse is safe: batch b-2 was collected (host-synchronised) in iteration b-1
-        if (frame_stride == static_cast<int64_t>(frame_bytes)) {
-            memcpy(c.pin_in, frames_host + static_cast<size_t>(first) * frame_bytes, (cnt + 1) * frame_bytes);
-        } else {
-            for (int i = 0; i <= cnt; ++i)
-                memcpy(static_cast<char*>(c.pin_in) + i * frame_bytes, frames_host + static_cast<int64_t>(first + i) * frame_stride,
-                       frame_bytes);
-        }
-        CUDA_TRY(cudaMemcpyAsync(c.dev_in, c.pin_in, (cnt + 1) * frame_bytes, cudaMemcpyHostToDevice, net->clip_h2d));
-        CUDA_TRY(cudaEventRecord(c.in_ready, net->clip_h2d));
-        CUDA_TRY(cudaStreamWaitEvent(st, c.in_ready, 0));
-        if (pair_sad_host)  // the batch's cnt+1 frames were just uploaded: the SAD reads them from L2, not the host
-            KERNEL_TRY(fi::pair_sad_launch(static_cast<const uint8_t*>(c.dev_in), static_cast<int64_t>(frame_bytes),
-                                           static_cast<int64_t>(frame_bytes), cnt + 1, c.dev_sad, st));
-        const fiPlanes p0 = u8_planes(c.dev_in, channels_per_frame, H, W, frame_bytes);
-        const fiPlanes p1 = u8_planes(static_cast<const uint8_t*>(c.dev_in) + frame_bytes, channels_per_frame, H, W,
-                                      frame_bytes);
-        rc = fiNetForward(net, &p0, &p1, FI_IN_U8, nullptr, static_cast<uint8_t*>(c.dev_out), cnt, H, W, stream);
-        if (rc) return rc;
-        CUDA_TRY(cudaEventRecord(c.done, st));
-        CUDA_TRY(cudaStreamWaitEvent(net->clip_d2h, c.done, 0));
-        CUDA_TRY(cudaMemcpyAsync(c.pin_out, c.dev_out, cnt * outf_bytes, cudaMemcpyDeviceToHost, net->clip_d2h));
-        if (pair_sad_host)
-            CUDA_TRY(cudaMemcpyAsync(c.pin_sad, c.dev_sad, cnt * sizeof(uint64_t), cudaMemcpyDeviceToHost, net->clip_d2h));
-        CUDA_TRY(cudaEventRecord(c.out_ready, net->clip_d2h));
-        if (b > 0 && (rc = collect(b - 1))) return rc;
-    }
-    return collect(n_batches - 1);
-}
-
 int fiNetInterpolateDyadicHostU8(fiNet* net, const uint8_t* frames_host, int64_t frame_stride, int n_frames,
                                  int channels_per_frame, int H, int W, int depth, const int32_t* req_pair_host,
                                  const int32_t* req_num_host, int n_req, uint8_t* out_host, int64_t out_stride,
@@ -1140,16 +1043,19 @@ int fiNetInterpolateDyadicHostU8(fiNet* net, const uint8_t* frames_host, int64_t
         return fail(FI_ERR_INVALID, "req_pair_host, req_num_host and out_host are required when n_req > 0");
     if (2 * channels_per_frame != net->n_channels)
         return fail(FI_ERR_INVALID, "2 x %d channels per frame != n_channels %d", channels_per_frame, net->n_channels);
-    if (net->n_classes != channels_per_frame)
-        return fail(FI_ERR_INVALID, "n_classes %d != channels_per_frame %d: bisection feeds each node back into the network",
-                    net->n_classes, channels_per_frame);
     if (depth < 1 || depth > 6) return fail(FI_ERR_INVALID, "depth %d is outside 1..6", depth);
+    if (depth > 1 && net->n_classes != channels_per_frame)
+        return fail(FI_ERR_INVALID, "n_classes %d != channels_per_frame %d: below depth 1 bisection feeds nodes back "
+                    "into the network", net->n_classes, channels_per_frame);
     if (n_frames < 2) return fail(FI_ERR_INVALID, "n_frames %d: a clip needs at least two frames", n_frames);
     if (H < 16 || W < 16) return fail(FI_ERR_INVALID, "input %dx%d is smaller than 16x16 (4 poolings)", H, W);
     if (pairs_per_batch < 1) return fail(FI_ERR_INVALID, "pairs_per_batch %d < 1", pairs_per_batch);
-    const size_t fb = static_cast<size_t>(channels_per_frame) * H * W;  // a frame and a node have the same size
+    // bytes of a frame and of a node (an output of the network); the two are equal wherever a node is fed back
+    const size_t fb = static_cast<size_t>(channels_per_frame) * H * W;
+    const size_t nodeb = static_cast<size_t>(net->n_classes) * H * W;
     if (frame_stride < static_cast<int64_t>(fb)) return fail(FI_ERR_INVALID, "frame_stride is smaller than a frame");
-    if (n_req > 0 && out_stride < static_cast<int64_t>(fb)) return fail(FI_ERR_INVALID, "out_stride is smaller than a frame");
+    if (n_req > 0 && out_stride < static_cast<int64_t>(nodeb))
+        return fail(FI_ERR_INVALID, "out_stride is smaller than a node");
     const int n_pairs = n_frames - 1, full = 1 << depth;
     for (int j = 0; j < n_req; ++j) {
         const int p = req_pair_host[j], v = req_num_host[j];
@@ -1191,22 +1097,26 @@ int fiNetInterpolateDyadicHostU8(fiNet* net, const uint8_t* frames_host, int64_t
     };
     std::vector<Group> groups;  // groups of B pairs that have requests (all of them when the SAD is asked for)
     size_t max_nodes = 0, max_req = 0;
+    bool gather = false;  // a forward gathers its parents: a node below level 1, or midpoints of non-consecutive pairs
     for (int first = 0, r = 0; first < n_pairs; first += B) {
         Group g{first, std::min(B, n_pairs - first), r, r};
         while (r < n_req && req_pair_host[r] < first + g.cnt) ++r;
         g.r1 = r;
         if (g.r0 == g.r1 && !pair_sad_host) continue;
         groups.push_back(g);
-        max_nodes = std::max(max_nodes, static_cast<size_t>(closure(g.first, g.cnt, g.r0, g.r1)));
+        const int nodes = closure(g.first, g.cnt, g.r0, g.r1);
+        bool direct = nodes == 0 || req_pair_host[g.r1 - 1] - req_pair_host[g.r0] + 1 == nodes;
+        for (int j = g.r0; j < g.r1 && direct; ++j) direct = req_num_host[j] == full / 2;
+        gather = gather || !direct;
+        max_nodes = std::max(max_nodes, static_cast<size_t>(nodes));
         max_req = std::max(max_req, static_cast<size_t>(g.r1 - g.r0));
     }
     if (groups.empty()) {
         if (n_forwards_host) *n_forwards_host = 0;
         return FI_OK;
     }
-    // the clip call's input staging and SAD buffers; its output staging is not used (nodes go through pin_nodes)
-    if ((rc = clip_staging(net, B, (B + 1) * fb, 0, pair_sad_host != nullptr))) return rc;
-    const size_t gather_bytes = max_nodes > 0 ? 2 * B * fb : 0, pool_bytes = max_nodes * fb, nodes_bytes = max_req * fb;
+    if ((rc = clip_staging(net, B, (B + 1) * fb, pair_sad_host != nullptr))) return rc;
+    const size_t gather_bytes = gather ? 2 * B * fb : 0, pool_bytes = max_nodes * nodeb, nodes_bytes = max_req * nodeb;
     bool grow = net->dyadic_gather.bytes < gather_bytes;
     for (auto& c : net->clip) grow = grow || c.pool.bytes < pool_bytes || c.pin_nodes_bytes < nodes_bytes;
     if (grow) {
@@ -1230,16 +1140,17 @@ int fiNetInterpolateDyadicHostU8(fiNet* net, const uint8_t* frames_host, int64_t
             }
         }
     }
-    // one plan of the clip call's capacity serves every level's batches (<= B images each)
-    if (max_nodes > 0 && (rc = build_plan(net, B, H, W))) return rc;
+    // one plan serves every level's batches: none has more than B images or more than a group's nodes
+    if (max_nodes > 0 && (rc = build_plan(net, static_cast<int>(std::min(static_cast<size_t>(B), max_nodes)), H, W)))
+        return rc;
 
     auto collect = [&](size_t b) -> int {  // wait for group b's D2H and hand its requested nodes to the caller
         const Group& g = groups[b];
         fiNet::ClipSlot& c = net->clip[b & 1];
         CUDA_TRY(cudaEventSynchronize(c.out_ready));
         for (int r = g.r0; r < g.r1; ++r)
-            memcpy(out_host + static_cast<int64_t>(r) * out_stride, static_cast<const char*>(c.pin_nodes) + (r - g.r0) * fb,
-                   fb);
+            memcpy(out_host + static_cast<int64_t>(r) * out_stride,
+                   static_cast<const char*>(c.pin_nodes) + (r - g.r0) * nodeb, nodeb);
         if (pair_sad_host) memcpy(pair_sad_host + g.first, c.pin_sad, g.cnt * sizeof(uint64_t));
         return FI_OK;
     };
@@ -1273,7 +1184,7 @@ int fiNetInterpolateDyadicHostU8(fiNet* net, const uint8_t* frames_host, int64_t
         auto node = [&](int q, int v) -> const uint8_t* {
             if (v == 0) return frames_dev + q * fb;
             if (v == full) return frames_dev + (q + 1) * fb;
-            return pool + slot[(q << depth) | v] * fb;
+            return pool + slot[(q << depth) | v] * nodeb;
         };
         int next = 0;  // pool slots in evaluation order, so that each forward's outputs are contiguous
         for (int level = 1; level <= depth; ++level) {
@@ -1284,13 +1195,22 @@ int fiNetInterpolateDyadicHostU8(fiNet* net, const uint8_t* frames_host, int64_t
                     if (need[(q << depth) | v]) todo.push_back((q << depth) | v);
             for (size_t k0 = 0; k0 < todo.size(); k0 += B) {
                 const int nb = static_cast<int>(std::min(todo.size() - k0, static_cast<size_t>(B)));
+                // the midpoints of consecutive pairs q0 .. q0+nb-1 read their parents where they were uploaded; any
+                // other batch gathers them into in0 | in1
+                const int q0 = todo[k0] >> depth;
+                const bool direct = level == 1 && (todo[k0 + nb - 1] >> depth) - q0 == nb - 1;
                 for (int k = 0; k < nb; ++k) {
                     const int key = todo[k0 + k], q = key >> depth, v = key & (full - 1);
-                    CUDA_TRY(cudaMemcpyAsync(in0 + k * fb, node(q, v - half), fb, cudaMemcpyDeviceToDevice, st));
-                    CUDA_TRY(cudaMemcpyAsync(in1 + k * fb, node(q, v + half), fb, cudaMemcpyDeviceToDevice, st));
+                    if (!direct) {
+                        CUDA_TRY(cudaMemcpyAsync(in0 + k * fb, node(q, v - half), fb, cudaMemcpyDeviceToDevice, st));
+                        CUDA_TRY(cudaMemcpyAsync(in1 + k * fb, node(q, v + half), fb, cudaMemcpyDeviceToDevice, st));
+                    }
                     slot[key] = next + k;
                 }
-                rc = fiNetForward(net, &p0, &p1, FI_IN_U8, nullptr, pool + next * fb, nb, H, W, stream);
+                const fiPlanes d0 = u8_planes(frames_dev + q0 * fb, channels_per_frame, H, W, fb);
+                const fiPlanes d1 = u8_planes(frames_dev + (q0 + 1) * fb, channels_per_frame, H, W, fb);
+                rc = fiNetForward(net, direct ? &d0 : &p0, direct ? &d1 : &p1, FI_IN_U8, nullptr, pool + next * nodeb,
+                                  nb, H, W, stream);
                 if (rc) return rc;
                 next += nb;
             }
@@ -1302,8 +1222,8 @@ int fiNetInterpolateDyadicHostU8(fiNet* net, const uint8_t* frames_host, int64_t
             const int s = slot[((req_pair_host[r] - g.first) << depth) | req_num_host[r]];
             int e = r + 1;
             while (e < g.r1 && slot[((req_pair_host[e] - g.first) << depth) | req_num_host[e]] == s + (e - r)) ++e;
-            CUDA_TRY(cudaMemcpyAsync(static_cast<char*>(c.pin_nodes) + (r - g.r0) * fb, pool + s * fb, (e - r) * fb,
-                                     cudaMemcpyDeviceToHost, net->clip_d2h));
+            CUDA_TRY(cudaMemcpyAsync(static_cast<char*>(c.pin_nodes) + (r - g.r0) * nodeb, pool + s * nodeb,
+                                     (e - r) * nodeb, cudaMemcpyDeviceToHost, net->clip_d2h));
             r = e;
         }
         if (pair_sad_host)

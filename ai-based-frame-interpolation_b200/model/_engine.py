@@ -60,12 +60,6 @@ _SIGNATURES = {
                                C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "fiNetInterpolateHostU8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int,
                                          C.c_int, C.c_void_p]),
-    "fiNetInterpolateClipHostU8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
-                                             C.c_int, C.c_void_p]),
-    "fiNetInterpolateClipHostU8Strided": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p,
-                                                    C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p]),
-    "fiNetInterpolateClipHostU8Sad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p,
-                                                C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "fiNetInterpolateDyadicHostU8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int,
                                                C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_int,
                                                C.c_void_p, C.c_void_p, C.POINTER(C.c_int64)]),
@@ -282,30 +276,26 @@ class Net:
         return out
 
     def interpolate_clip_host_u8(self, frames, pairs_per_batch=4, out=None, sad_out=None):
-        """numpy uint8 [F,C,H,W] host clip in, numpy uint8 [F-1,n_classes,H,W] midpoints out; copies and compute are
-        pipelined inside the library. `out`: optional preallocated result array (e.g. this GPU's slice of a clip-wide
-        buffer when the pairs are sharded across GPUs). Both arrays may be strided along the frame axis (every frame
-        itself contiguous), e.g. `seq[0::2]` in and `seq[1::2]` out of one interleaved sequence. `sad_out`: optional
-        contiguous uint64 [F-1] array that receives the scene-cut statistic of every pair, sum |f[i+1] - f[i]| over
-        all C*H*W bytes, computed on the GPU from the uploaded frames (fiNetInterpolateClipHostU8Sad)."""
+        """numpy uint8 [F,C,H,W] host clip in, numpy uint8 [F-1,n_classes,H,W] midpoints out: the depth-1 bisection
+        node of every pair (interpolate_dyadic_host_u8), with copies and compute pipelined inside the library. `out`:
+        optional preallocated result array (e.g. this GPU's slice of a clip-wide buffer when the pairs are sharded
+        across GPUs). Both arrays may be strided along the frame axis (every frame itself contiguous), e.g. `seq[0::2]`
+        in and `seq[1::2]` out of one interleaved sequence. `sad_out`: optional contiguous uint64 [F-1] array that
+        receives the scene-cut statistic of every pair, sum |f[i+1] - f[i]| over all C*H*W bytes, computed on the GPU
+        from the uploaded frames."""
+        import numpy as np
         frames = _host_clip(frames)
-        f, c, h, w = frames.shape
-        out = _host_out(out, f - 1, self.n_classes, h, w)
-        _check_sad_out(sad_out, f)
-        with torch.cuda.device(self.device):
-            check(lib().fiNetInterpolateClipHostU8Sad(self._h, frames.ctypes.data, frames.strides[0], f, c,
-                                                      out.ctypes.data, out.strides[0] if f > 1 else 0, h, w,
-                                                      pairs_per_batch, current_stream(),
-                                                      sad_out.ctypes.data if sad_out is not None else None))
-        return out
+        pairs = np.arange(max(frames.shape[0] - 1, 0), dtype=np.int32)
+        return self.interpolate_dyadic_host_u8(frames, pairs, np.ones_like(pairs), 1, pairs_per_batch, out=out,
+                                               sad_out=sad_out)[0]
 
     def interpolate_dyadic_host_u8(self, frames, pairs, nums, depth, pairs_per_batch=4, out=None, sad_out=None):
         """Frames at dyadic times between the frames of a clip, by recursive bisection on the device
         (fiNetInterpolateDyadicHostU8). frames: numpy uint8 [F,C,H,W] host clip (strided along the frame axis like
-        interpolate_clip_host_u8) with C == n_classes. Request j is node (pairs[j], nums[j] / 2**depth): pairs sorted,
-        0 < nums[j] < 2**depth. Returns (out, n_forwards): out uint8 [len(pairs),C,H,W] (optional preallocated, frames
-        contiguous) and the number of images the network forwarded. sad_out: optional uint64 [F-1] that receives every
-        pair's SAD, as in interpolate_clip_host_u8."""
+        interpolate_clip_host_u8), with C == n_classes when depth > 1. Request j is node (pairs[j], nums[j] / 2**depth):
+        pairs sorted, 0 < nums[j] < 2**depth. Returns (out, n_forwards): out uint8 [len(pairs),n_classes,H,W] (optional
+        preallocated, frames contiguous) and the number of images the network forwarded. sad_out: optional uint64
+        [F-1] that receives every pair's SAD, as in interpolate_clip_host_u8."""
         import numpy as np
         frames = _host_clip(frames)
         f, c, h, w = frames.shape

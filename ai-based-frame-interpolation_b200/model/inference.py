@@ -241,15 +241,6 @@ class FrameInterpolator:
             out += self._forward_pairs(firsts[i:i + self.pairs_per_batch], seconds[i:i + self.pairs_per_batch])
         return out
 
-    def _clip_call(self, frames, out, sad=None):
-        """[F,C,H,W] u8 host clip -> out [F-1,n_classes,H,W]: one GPU = the library's pipelined clip call (pinned
-        double-buffered staging, copies overlapped with compute); several GPUs = contiguous pair ranges, one per GPU.
-        sad: optional uint64 [F-1] that receives each pair's sum of absolute differences, computed on the GPU."""
-        if self._single_device:
-            return self.model._engine(self.device).interpolate_clip_host_u8(frames, self.pairs_per_batch, out=out,
-                                                                            sad_out=sad)
-        return self._gpu_pool().clip_midpoints(frames, self.pairs_per_batch, out, sad_out=sad)
-
     def interpolate_clip(self, frames, out=None):
         """Midpoint of every consecutive pair of a clip held in ONE uint8 array: [F,H,W] grey or [F,H,W,3] BGR ->
         [F-1,H,W] / [F-1,H,W,3]. `out` may be a preallocated result array (re-used across calls by the video loop and by
@@ -273,7 +264,8 @@ class FrameInterpolator:
         elif out.shape != (arr.shape[0] - 1,) + arr.shape[1:] or out.dtype != np.uint8:
             raise ValueError("out must be a uint8 array with one frame less than the clip")
         sad = np.zeros(arr.shape[0] - 1, dtype=np.uint64) if detect else None
-        self._planar(self._clip_call, arr, out, sad)
+        pairs = np.arange(arr.shape[0] - 1, dtype=np.int32)            # the depth-1 node (i, 1/2) of every pair
+        self._planar(lambda fr, o, s: self._dyadic_call(fr, pairs, np.ones_like(pairs), 1, o, s), arr, out, sad)
         if not detect:
             return out, None, prev_mafd
         scores, last_mafd = scene_scores(sad, arr[0].size, prev_mafd)
@@ -360,8 +352,10 @@ class FrameInterpolator:
         return result, cuts, last_mafd
 
     def _dyadic_call(self, frames, pairs, nums, depth, out, sad):
-        """[F,C,H,W] u8 host clip -> the bisection nodes (pairs[j], nums[j] / 2^depth) in out[j]: one GPU = the library
-        call, several GPUs = contiguous pair ranges, one per GPU (as `_clip_call`)."""
+        """[F,C,H,W] u8 host clip -> the bisection nodes (pairs[j], nums[j] / 2^depth) in out[j]: one GPU = the library's
+        pipelined host-clip call (pinned double-buffered staging, copies overlapped with compute); several GPUs =
+        contiguous pair ranges, one per GPU. sad: optional uint64 [F-1] that receives each pair's sum of absolute
+        differences, computed on the GPU."""
         if self._single_device:
             return self.model._engine(self.device).interpolate_dyadic_host_u8(frames, pairs, nums, depth,
                                                                               self.pairs_per_batch, out=out, sad_out=sad)

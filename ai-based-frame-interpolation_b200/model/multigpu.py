@@ -3,9 +3,9 @@
 
 Every pair (frame i, frame i+1) is independent (reference model/inference.py:101-122 keeps no state), so a clip of F frames
 is cut into contiguous ranges of pairs (model/sharding.py: neighbouring ranges share one boundary frame) and each range goes
-through one GPU's pipelined clip call (fiNetInterpolateClipHostU8). There is no collective and no device-to-device traffic:
-each worker reads its frames from the caller's host array and writes its midpoints into its slice of the caller's result
-array, so the in-order gather for the video writer is free.
+through one GPU's pipelined host-clip call (fiNetInterpolateDyadicHostU8; the midpoint clip is its depth-1 case). There is
+no collective and no device-to-device traffic between GPUs: each worker reads its frames from the caller's host array and
+writes its frames into its slice of the caller's result array, so the in-order gather for the video writer is free.
 
 One host thread per GPU drives one fiNet handle (a handle must not be shared between threads); the C-ABI calls are made
 through ctypes, which releases the GIL, so the workers really run concurrently. A worker whose call raises is retired
@@ -26,9 +26,8 @@ except ImportError:  # model/ on sys.path, like the reference's scripts
 
 
 class GpuPool:
-    """`runners`: one object per GPU with `.interpolate_clip_host_u8(frames, pairs_per_batch, out=..., sad_out=...)`
-    and, for clip_dyadic, `.interpolate_dyadic_host_u8(frames, pairs, nums, depth, pairs_per_batch, out=...,
-    sad_out=...)` (an `_engine.Net`, or a stand-in in the CPU tests of the scheduling logic)."""
+    """`runners`: one object per GPU with `.interpolate_dyadic_host_u8(frames, pairs, nums, depth, pairs_per_batch,
+    out=..., sad_out=...)` (an `_engine.Net`, or a stand-in in the CPU tests of the scheduling logic)."""
 
     def __init__(self, runners):
         if not runners:
@@ -77,28 +76,12 @@ class GpuPool:
     def n_alive(self):
         return sum(self.alive)
 
-    def clip_midpoints(self, frames, pairs_per_batch, out, sad_out=None):
-        """frames: uint8 [F,C,H,W] C-contiguous host array; out: uint8 [F-1,n_classes,H,W] C-contiguous. Pair i of the
-        clip lands in out[i] whichever GPU computed it. sad_out: optional uint64 [F-1] array; the worker of pair i
-        writes its scene-cut statistic to sad_out[i] (a re-queued range rewrites the same slots)."""
-        n_frames = frames.shape[0]
-        if n_frames < 2:
-            return out
-
-        def job(runner, first, n):
-            extra = {} if sad_out is None else {"sad_out": sad_out[first:first + n]}
-            runner.interpolate_clip_host_u8(frames[first:first + n + 1], pairs_per_batch, out=out[first:first + n],
-                                            **extra)
-
-        self._run_ranges(n_frames - 1, job)
-        return out
-
     def clip_dyadic(self, frames, pairs, nums, depth, pairs_per_batch, out, sad_out=None):
-        """Bisection nodes (`_engine.Net.interpolate_dyadic_host_u8`) of a clip sharded like clip_midpoints: each worker
-        takes a contiguous range of pairs with the requests inside it. frames: uint8 [F,C,H,W] host array; pairs / nums:
-        the requests, sorted by pair; out: uint8 [len(pairs),C,H,W]. Request j lands in out[j] whichever GPU computed
-        it, and sad_out[i] (optional uint64 [F-1]) receives pair i's SAD. Returns (out, images forwarded by the ranges
-        that completed)."""
+        """Bisection nodes (`_engine.Net.interpolate_dyadic_host_u8`) of a clip: each worker takes a contiguous range of
+        pairs with the requests inside it. frames: uint8 [F,C,H,W] host array; pairs / nums: the requests, sorted by
+        pair; out: uint8 [len(pairs),n_classes,H,W]. Request j lands in out[j] whichever GPU computed it, and sad_out[i]
+        (optional uint64 [F-1]) receives pair i's SAD (a re-queued range rewrites the same slots). Returns (out, images
+        forwarded by the ranges that completed)."""
         pairs = np.ascontiguousarray(pairs, dtype=np.int32)
         nums = np.ascontiguousarray(nums, dtype=np.int32)
         n_frames = frames.shape[0]

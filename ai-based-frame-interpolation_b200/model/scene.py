@@ -3,7 +3,7 @@
 At a hard cut the two frames of a pair show unrelated shots, so the network can only write a ghosted blend of both.
 Like ffmpeg's scdet / minterpolate and RIFE's video script, the video path detects such pairs and repeats the pair's
 first frame instead. The statistic is the mean absolute frame difference of ffmpeg's scdet, computed from the exact
-per-pair sum of absolute differences (SAD) that the GPU forms inside the clip call (fiNetInterpolateClipHostU8Sad):
+per-pair sum of absolute differences (SAD) that the GPU forms inside the host-clip call (fiNetInterpolateDyadicHostU8):
 
     mafd_i  = 100 * SAD_i / (B * 256)                    B = bytes of one frame, all colour planes
     score_i = clamp(min(mafd_i, |mafd_i - mafd_{i-1}|), 0, 100),   mafd_{-1} = 0 at the first pair of a clip / video

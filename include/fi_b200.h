@@ -85,46 +85,29 @@ int fiNetForward(fiNet* net, const fiPlanes* in0, const fiPlanes* in1, int in_dt
 int fiNetInterpolateHostU8(fiNet* net, const uint8_t* frame1_host, const uint8_t* frame2_host, int channels_per_frame,
                            uint8_t* out_host, int N, int H, int W, void* stream);
 
-/* The video loop FrameInterpolator.interpolate_video needs (reference main.py:118-129; the reference never wrote it,
- * SURVEY.md D3): a clip of n_frames planar u8 frames [n_frames, C, H, W] on the host -> the n_frames-1 midpoint
- * frames [n_frames-1, n_classes, H, W] on the host. Frames are uploaded once per batch of `pairs_per_batch` pairs;
- * H2D of batch i+1, the forward of batch i and D2H of batch i-1 overlap (two copy streams + `stream`, double-buffered
- * pinned staging). Synchronous: returns when out_host is complete. */
-int fiNetInterpolateClipHostU8(fiNet* net, const uint8_t* frames_host, int n_frames, int channels_per_frame,
-                               uint8_t* out_host, int H, int W, int pairs_per_batch, void* stream);
-
-/* The same with the frames frame_stride bytes and the results out_stride bytes apart (each frame itself contiguous):
- * lets FrameInterpolator.interpolate_sequence (factor 2^k bisection, reference main.py:128 `--factor`) read every other
- * frame of an interleaved sequence and write the new midpoints straight between them, without gathering copies. */
-int fiNetInterpolateClipHostU8Strided(fiNet* net, const uint8_t* frames_host, int64_t frame_stride, int n_frames,
-                                      int channels_per_frame, uint8_t* out_host, int64_t out_stride, int H, int W,
-                                      int pairs_per_batch, void* stream);
-
-/* The same, plus the scene-cut statistic of every pair (the reference has no scene detection): when pair_sad_host is
- * not NULL it receives n_frames-1 uint64 values, pair_sad_host[i] = sum |f[i+1] - f[i]| over all C*H*W bytes (exact).
- * Each batch's SAD runs on the frames the call has just uploaded (fiPairSadU8 on `stream`, before the forward) and is
- * copied back with the batch's midpoints; the host frames are not read again. With NULL this is exactly the strided
- * call above (which wraps it). */
-int fiNetInterpolateClipHostU8Sad(fiNet* net, const uint8_t* frames_host, int64_t frame_stride, int n_frames,
-                                  int channels_per_frame, uint8_t* out_host, int64_t out_stride, int H, int W,
-                                  int pairs_per_batch, void* stream, uint64_t* pair_sad_host);
-
-/* Frame-rate conversion (main.py video --fps; the reference has none): frames at dyadic times between the frames of a
- * clip, by recursive bisection on the device. The network has no time input, so node (i, a/2^d) with a odd is the
- * network midpoint of (i, (a-1)/2^d) and (i, (a+1)/2^d), each in lowest terms; (i, 0) is frame i and (i, 1) frame i+1.
- * That is exactly the frame host-side recursive bisection produces (the forward gives the same bits at any batch size).
- *   frames_host: n_frames planar u8 frames [C, H, W], frame_stride bytes apart; n_classes must equal C
- *                (channels_per_frame), because every node is fed back into the network;
+/* Host clips (main.py video; the reference never wrote its video loop, SURVEY.md D3, and has no --fps): frames at
+ * dyadic times between the frames of a clip, by recursive bisection on the device. The network has no time input, so
+ * node (i, a/2^d) with a odd is the network midpoint of (i, (a-1)/2^d) and (i, (a+1)/2^d), each in lowest terms; (i, 0)
+ * is frame i and (i, 1) frame i+1. That is exactly the frame host-side recursive bisection produces (the forward gives
+ * the same bits at any batch size). depth = 1 with req_pair = i, req_num = 1 for every pair i (the nodes (i, 1/2)) is
+ * the midpoint clip that FrameInterpolator.interpolate_clip and the video loop run.
+ *   frames_host: n_frames planar u8 frames [C, H, W], frame_stride bytes apart (each frame contiguous; strides let
+ *                interpolate_sequence read every other frame of an interleaved sequence and write the new midpoints
+ *                straight between them); C = channels_per_frame, and n_classes must equal C when depth > 1, because
+ *                nodes below level 1 are computed from nodes fed back into the network;
  *   request j:   node (req_pair_host[j], req_num_host[j] / 2^depth), depth in 1..6, 0 <= pair < n_frames-1,
  *                0 < num < 2^depth, requests sorted by pair (any order of num, repeats allowed); it is written to
- *                out_host + j*out_stride as u8 [C, H, W].
+ *                out_host + j*out_stride as u8 [n_classes, H, W].
  * Pairs go in groups of pairs_per_batch; each group's frames are uploaded once, the closure of its requests is evaluated
- * level by level in batches of <= pairs_per_batch images with every node kept in a device pool (parents gathered with
- * device-to-device copies), and only the requested nodes are copied back. Upload of group g+1, the levels of group g and
- * the download of group g-1 overlap, as in the clip call. pair_sad_host (optional) receives every pair's SAD as in
- * fiNetInterpolateClipHostU8Sad; with NULL, groups without requests are never uploaded. n_forwards_host (optional)
- * receives the number of images forwarded. Any invalid argument returns FI_ERR_INVALID, naming it, before anything is
- * launched or written. Synchronous: returns when out_host is complete. */
+ * level by level in batches of <= pairs_per_batch images with every node kept in a device pool, and only the requested
+ * nodes are copied back. A level-1 batch of consecutive pairs reads its parents where they were uploaded; any other
+ * batch gathers them with device-to-device copies. Upload of group g+1 (copy stream), the levels of group g (`stream`)
+ * and the download of group g-1 (a second copy stream) overlap through double-buffered pinned staging.
+ * pair_sad_host (optional; the reference has no scene detection) receives n_frames-1 uint64 values, pair_sad_host[i] =
+ * sum |f[i+1] - f[i]| over all C*H*W bytes (exact), computed by fiPairSadU8 on `stream` from each group's uploaded
+ * frames, so the host frames are not read again; with NULL, groups without requests are never uploaded.
+ * n_forwards_host (optional) receives the number of images forwarded. Any invalid argument returns FI_ERR_INVALID,
+ * naming it, before anything is launched or written. Synchronous: returns when out_host is complete. */
 int fiNetInterpolateDyadicHostU8(fiNet* net, const uint8_t* frames_host, int64_t frame_stride, int n_frames,
                                  int channels_per_frame, int H, int W, int depth, const int32_t* req_pair_host,
                                  const int32_t* req_num_host, int n_req, uint8_t* out_host, int64_t out_stride,

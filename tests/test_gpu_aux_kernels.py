@@ -132,8 +132,8 @@ def test_host_buffer_entry_point(cuda_device):
 
 
 def test_clip_pipeline_matches_pairwise_calls(cuda_device):
-    """fiNetInterpolateClipHostU8 (pipelined video loop) == the synchronous per-batch entry point, bit for bit,
-    including a ragged last batch."""
+    """The midpoint clip (interpolate_clip_host_u8: the pipelined host-clip call at depth 1, as the video loop runs
+    it) == the synchronous per-batch entry point, bit for bit, including a ragged last batch."""
     sd = O.init_state_dict(0, 2, 1, False)
     net = E.Net(cuda_device, 2, 1, False)
     net.load_state_dict(sd)

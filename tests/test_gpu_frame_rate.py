@@ -1,6 +1,7 @@
 """GPU tier of frame-rate conversion: fiNetInterpolateDyadicHostU8 bit for bit against explicit recursive bisection
 through single-pair forwards, FrameInterpolator.interpolate_at at power-of-two rates against interpolate_sequence, the
-forward counts of the timing rule, the SAD, scene cuts, the `main.py video --fps` path and argument errors."""
+forward counts of the timing rule, level-1 batches read in place against gathered ones, the SAD, scene cuts, the
+`main.py video --fps` path and argument errors."""
 from fractions import Fraction
 
 import numpy as np
@@ -177,6 +178,38 @@ def test_forward_counts_follow_the_rule(nets, dst, per_pair):
     assert one == per_pair
 
 
+@pytest.mark.parametrize("name", ["grey_convt", "colour", "grey_to_rgb"])
+def test_level_one_reads_consecutive_pairs_in_place(nets, name):
+    """A level-1 batch of consecutive pairs reads its parents where they were uploaded; any other batch gathers them.
+    Calls that mix both give the midpoint clip's bytes and forward every node once. UNet(2, 3) has nodes of 3 planes
+    and frames of 1: at depth 1 no node is fed back, so its midpoints come through the same call."""
+    if name == "grey_to_rgb":
+        net = E.Net("cuda:0", 2, 3, False)
+        net.load_state_dict(O.init_state_dict(3, 2, 3, False))
+    else:
+        net = nets[name]
+    c = net.n_channels // 2
+    frames = smooth_clip(13, c, 40, 56, seed=7)
+    mids = net.interpolate_clip_host_u8(frames, 4)             # 12 pairs: groups [0, 4), [4, 8), [8, 12)
+    assert mids.shape == (12, net.n_classes, 40, 56)
+    assert np.array_equal(mids, net.interpolate_host_u8(frames[:-1], frames[1:]))
+    # group 0 whole (in place), group 1 pairs 5 and 7 (gathered), group 2 the run 9, 10 (in place from pair 9)
+    pairs = np.array([0, 1, 2, 3, 5, 7, 9, 10, 10], np.int32)
+    got, forwards = net.interpolate_dyadic_host_u8(frames, pairs, np.ones(len(pairs), np.int32), 1, 4)
+    assert forwards == 8 and np.array_equal(got, mids[pairs])
+    if name != "grey_to_rgb":
+        # depth 2: level 1 of the run 4 .. 7 in place, level 2 gathered from it in the same group
+        pairs = np.array([4, 4, 5, 6, 7, 7], np.int32)
+        nums = np.array([2, 1, 2, 2, 3, 2], np.int32)
+        got, forwards = net.interpolate_dyadic_host_u8(frames, pairs, nums, 2, 4)
+        assert forwards == len(needed(pairs, nums, 2)) == 6
+        assert np.array_equal(got[nums == 2], mids[pairs[nums == 2]])
+        ref = bisection_reference(net, frames[4:9], 2)
+        assert np.array_equal(got[1], ref[0][1]) and np.array_equal(got[4], ref[3][3])
+    else:
+        net.close()
+
+
 # ------------------------------------------------------------------------------------------- 4. SAD
 @pytest.mark.parametrize("ppb", [1, 3, 4])
 def test_sad_equals_the_clip_call(nets, ppb):
@@ -300,10 +333,10 @@ def test_bad_arguments_are_refused_before_any_work(nets):
     sad = np.full(4, 5, np.uint64)
     forwards = np.full(1, -3, np.int64)
 
-    def call(pairs, nums, depth=3, handle=net._h, channels=1):
+    def call(pairs, nums, depth=3, handle=net._h, channels=1, dst=out):
         p, n = np.array(pairs, np.int32), np.array(nums, np.int32)
         rc = lib.fiNetInterpolateDyadicHostU8(handle, frames.ctypes.data, frames.strides[0], 5, channels, 32, 48, depth,
-                                              p.ctypes.data, n.ctypes.data, len(p), out.ctypes.data, out.strides[0], 2,
+                                              p.ctypes.data, n.ctypes.data, len(p), dst.ctypes.data, dst.strides[0], 2,
                                               E.current_stream(), sad.ctypes.data,
                                               forwards.ctypes.data_as(E.C.POINTER(E.C.c_int64)))
         return rc, lib.fiLastError().decode()
@@ -319,8 +352,13 @@ def test_bad_arguments_are_refused_before_any_work(nets):
         rc, msg = call(pairs, nums, **kw)
         assert rc == -1 and word in msg, (pairs, nums, kw, msg)
     colour3 = E.Net("cuda:0", 2, 3, False)                        # UNet(2, 3): n_classes != channels per frame
-    rc, msg = call([0, 1, 2], [1, 2, 3], handle=colour3._h)
-    assert rc == -1 and "n_classes" in msg, msg
+    for depth in (2, 3):                                          # below depth 1 nodes are fed back: refused
+        rc, msg = call([0, 1, 2], [1, 2, 3], depth=depth, handle=colour3._h)
+        assert rc == -1 and "n_classes" in msg, (depth, msg)
+    nodes3 = np.full((3, 3, 32, 48), 77, np.uint8)                # output slots of UNet(2, 3)'s 3-plane nodes
+    rc, msg = call([0, 1, 2], [1, 1, 1], depth=1, handle=colour3._h, dst=nodes3)
+    assert rc == -3 and "fiNetLoadWeights" in msg, msg           # depth 1 is not refused: no weights are loaded
+    assert (nodes3 == 77).all()
     colour3.close()
     assert (out == 77).all() and (sad == 5).all() and forwards[0] == -3
     rc, _ = call([0, 1, 2], [1, 2, 3])

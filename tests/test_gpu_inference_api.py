@@ -291,7 +291,7 @@ def test_http_concurrent_requests_are_batched(cuda_device, checkpoints, tmp_path
 
 
 def test_strided_clip_and_in_place_bisection(cuda_device, checkpoints):
-    """fiNetInterpolateClipHostU8Strided: frames / results strided along the frame axis (seq[0::2] -> seq[1::2]) give the
+    """The midpoint clip with frames / results strided along the frame axis (seq[0::2] -> seq[1::2]) gives the
     bytes of the contiguous call, and interpolate_sequence(factor 4) built on it equals pair-by-pair bisection."""
     from model import _engine as E
     from model.inference import FrameInterpolator

@@ -1,5 +1,5 @@
-"""GPU tier of scene-cut detection: the exact pair-SAD kernel (fiPairSadU8), the SAD the pipelined clip call returns
-(fiNetInterpolateClipHostU8Sad), and FrameInterpolator(scene_threshold=...) on a clip with one hard cut — clip,
+"""GPU tier of scene-cut detection: the exact pair-SAD kernel (fiPairSadU8), the SAD the pipelined host-clip call
+returns (fiNetInterpolateDyadicHostU8), and FrameInterpolator(scene_threshold=...) on a clip with one hard cut — clip,
 sequence (factor 2, 3, 4), grey and colour models, the mp4 video loop across chunk edges and two GPUs."""
 import numpy as np
 import pytest

@@ -92,7 +92,8 @@ class _SadRunner:
     def __init__(self, fail=False):
         self.fail, self.calls = fail, 0
 
-    def interpolate_clip_host_u8(self, frames, pairs_per_batch, out=None, sad_out=None):
+    def interpolate_dyadic_host_u8(self, frames, pairs, nums, depth, pairs_per_batch, out=None, sad_out=None):
+        assert depth == 1 and list(pairs) == list(range(len(frames) - 1)) and (nums == 1).all()
         self.calls += 1
         if sad_out is not None:
             sad_out[...] = 12345                    # a failing worker may leave garbage behind
@@ -102,12 +103,18 @@ class _SadRunner:
         if sad_out is not None:
             d = np.abs(frames[1:].astype(np.int16) - frames[:-1]).reshape(len(out), -1)
             sad_out[...] = d.sum(axis=1, dtype=np.int64).astype(np.uint64)
-        return out
+        return out, len(pairs)
 
 
 def _clip(frames, seed):
     rs = np.random.RandomState(seed)
     return rs.randint(0, 256, size=(frames, 2, 5, 7)).astype(np.uint8)
+
+
+def _midpoints(pool, clip, out, sad):
+    """The midpoint clip: the depth-1 node of every pair."""
+    pairs = np.arange(len(clip) - 1, dtype=np.int32)
+    return pool.clip_dyadic(clip, pairs, np.ones_like(pairs), 1, 4, out, sad_out=sad)
 
 
 def _expected_sad(clip):
@@ -116,38 +123,24 @@ def _expected_sad(clip):
 
 @pytest.mark.parametrize("workers", [1, 2, 3])
 @pytest.mark.parametrize("frames", [2, 9, 14])
-def test_pool_sad_slices_land_in_their_slots(workers, frames):
+def test_pool_midpoint_clip_sad_slices_land_in_their_slots(workers, frames):
     from model.multigpu import GpuPool
     clip = _clip(frames, workers * 10 + frames)
     out = np.zeros((frames - 1, 2, 5, 7), np.uint8)
     sad = np.full(frames - 1, 7, np.uint64)
-    GpuPool([_SadRunner() for _ in range(workers)]).clip_midpoints(clip, 4, out, sad_out=sad)
+    _midpoints(GpuPool([_SadRunner() for _ in range(workers)]), clip, out, sad)
     assert np.array_equal(sad, _expected_sad(clip))
     assert np.array_equal(out, ((clip[:-1].astype(np.int32) + clip[1:]) // 2).astype(np.uint8))
 
 
-def test_pool_sad_after_failed_worker_requeue():
+def test_pool_midpoint_clip_sad_after_failed_worker_requeue():
     from model.multigpu import GpuPool
     clip = _clip(22, 5)
     out = np.zeros((21, 2, 5, 7), np.uint8)
     sad = np.zeros(21, np.uint64)
     runners = [_SadRunner(), _SadRunner(fail=True), _SadRunner()]
     pool = GpuPool(runners)
-    pool.clip_midpoints(clip, 4, out, sad_out=sad)
+    _midpoints(pool, clip, out, sad)
     assert pool.alive == [True, False, True]
     assert np.array_equal(sad, _expected_sad(clip))   # the re-queued range overwrote the failed worker's slots
 
-
-def test_pool_without_sad_keeps_the_old_runner_call():
-    """Runners that predate sad_out are still called exactly as before when no SAD is asked for."""
-    from model.multigpu import GpuPool
-
-    class Old:
-        def interpolate_clip_host_u8(self, frames, pairs_per_batch, out=None):
-            out[...] = frames[:-1]
-            return out
-
-    clip = _clip(6, 1)
-    out = np.zeros((5, 2, 5, 7), np.uint8)
-    GpuPool([Old(), Old()]).clip_midpoints(clip, 4, out)
-    assert np.array_equal(out, clip[:-1])

@@ -66,24 +66,32 @@ class _FakeRunner:
     def __init__(self, ident, fail_on=None):
         self.ident, self.fail_on, self.calls = ident, fail_on, []
 
-    def interpolate_clip_host_u8(self, frames, pairs_per_batch, out=None):
+    def interpolate_dyadic_host_u8(self, frames, pairs, nums, depth, pairs_per_batch, out=None, sad_out=None):
         import numpy as np
+        assert depth == 1 and list(pairs) == list(range(frames.shape[0] - 1)) and (nums == 1).all()
         self.calls.append(frames.shape[0] - 1)
         if self.fail_on is not None and self.fail_on(frames):
             raise RuntimeError(f"injected failure on worker {self.ident}")
         out[...] = ((frames[:-1].astype(np.int32) + frames[1:]) // 2).astype(np.uint8)
-        return out
+        return out, len(pairs)
+
+
+def _midpoints(pool, clip, out):
+    """The midpoint clip: the depth-1 node of every pair."""
+    import numpy as np
+    pairs = np.arange(len(clip) - 1, dtype=np.int32)
+    return pool.clip_dyadic(clip, pairs, np.ones_like(pairs), 1, 4, out)
 
 
 @pytest.mark.parametrize("workers,frames", [(1, 9), (2, 9), (4, 30), (8, 5), (3, 2)])
-def test_pool_covers_every_pair_in_order(workers, frames):
+def test_pool_midpoint_clip_covers_every_pair_in_order(workers, frames):
     import numpy as np
     from model.multigpu import GpuPool
     rs = np.random.RandomState(workers * 100 + frames)
     clip = rs.randint(0, 256, size=(frames, 1, 6, 7)).astype(np.uint8)
     out = np.full((frames - 1, 1, 6, 7), 255, np.uint8)
     runners = [_FakeRunner(i) for i in range(workers)]
-    GpuPool(runners).clip_midpoints(clip, 4, out)
+    _midpoints(GpuPool(runners), clip, out)
     assert np.array_equal(out, ((clip[:-1].astype(np.int32) + clip[1:]) // 2).astype(np.uint8))
     used = [r for r in runners if r.calls]
     assert len(used) == min(workers, frames - 1)
@@ -92,28 +100,28 @@ def test_pool_covers_every_pair_in_order(workers, frames):
     assert max(sizes) - min(sizes) <= 1
 
 
-def test_pool_requeues_the_range_of_a_failed_worker():
+def test_pool_midpoint_clip_requeues_the_range_of_a_failed_worker():
     import numpy as np
     from model.multigpu import GpuPool
     clip = np.arange(21 * 4 * 5, dtype=np.uint32).reshape(21, 1, 4, 5).astype(np.uint8)
     out = np.zeros((20, 1, 4, 5), np.uint8)
     runners = [_FakeRunner(0), _FakeRunner(1, fail_on=lambda fr: True), _FakeRunner(2)]
     pool = GpuPool(runners)
-    pool.clip_midpoints(clip, 4, out)
+    _midpoints(pool, clip, out)
     assert np.array_equal(out, ((clip[:-1].astype(np.int32) + clip[1:]) // 2).astype(np.uint8))
     assert pool.alive == [True, False, True] and pool.n_alive == 2
     assert len(pool.errors) == 1 and pool.errors[0][0] == 1 and "injected" in str(pool.errors[0][2])
     # the next clip is split over the two survivors only
     out2 = np.zeros_like(out)
-    pool.clip_midpoints(clip, 4, out2)
+    _midpoints(pool, clip, out2)
     assert np.array_equal(out2, out) and len(runners[1].calls) == 1
     # every worker failing is an error, not a silent partial result
     dead = GpuPool([_FakeRunner(0, fail_on=lambda fr: True), _FakeRunner(1, fail_on=lambda fr: True)])
     with pytest.raises(RuntimeError, match="all GPU workers failed"):
-        dead.clip_midpoints(clip, 4, np.zeros_like(out))
+        _midpoints(dead, clip, np.zeros_like(out))
 
 
-def test_pool_raises_invalid_requests_without_retiring_workers():
+def test_pool_midpoint_clip_raises_invalid_requests_without_retiring():
     import numpy as np
     from model.multigpu import GpuPool
 
@@ -125,5 +133,5 @@ def test_pool_raises_invalid_requests_without_retiring_workers():
 
     pool = GpuPool([_FakeRunner(0, fail_on=reject), _FakeRunner(1, fail_on=reject)])
     with pytest.raises(Invalid):
-        pool.clip_midpoints(np.zeros((9, 1, 8, 8), np.uint8), 4, np.zeros((8, 1, 8, 8), np.uint8))
+        _midpoints(pool, np.zeros((9, 1, 8, 8), np.uint8), np.zeros((8, 1, 8, 8), np.uint8))
     assert pool.alive == [True, True] and not pool.errors
