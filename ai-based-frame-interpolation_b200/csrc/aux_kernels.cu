@@ -496,6 +496,84 @@ gather_triplets_u8_kernel(const uint8_t* __restrict__ frames, long long n_frames
     }
 }
 
+// ------------------------------------------------------------------------------------------------ crop gather
+// Training batches of random windows from a cache of frames of different sizes (FrameTripletDataset(crop=S)):
+// out_k[b][c][y][x] = frames[off[f] + (c*H + y0 + y)*W + x0 + (mirror ? S-1-x : x)] / 255 with f = rows[b][k], k < 3.
+// One thread writes 4 consecutive output pixels of one output row with a 16-byte store; a warp covers 128 pixels of a
+// row, so a 256-wide row is two coalesced warps. Source rows start at any byte: the 4 source bytes are funnel-shifted
+// out of the (at most two) aligned 32-bit words that hold them, which never reads a word without a byte of the window;
+// mirroring reverses the bytes of the same 4-byte run read from the mirrored position. A row whose frame indices,
+// sizes or window are out of range is written as NaN (all three outputs) and none of its bytes are read.
+constexpr int GC_THREADS = 256;
+
+struct CropSrc {
+    const uint8_t* base;   // first byte of the window's top-left pixel in plane 0
+    long long plane;       // H*W
+    int w;                 // row stride
+};
+
+__device__ __forceinline__ bool crop_src(const uint8_t* frames, long long frames_bytes, const long long* offsets,
+                                         const int* sizes, long long n_frames, int C, int S, int f, int y0, int x0,
+                                         CropSrc* out) {
+    if (f < 0 || f >= n_frames) return false;
+    const long long off = __ldg(offsets + f);
+    const int h = __ldg(sizes + 2 * f), w = __ldg(sizes + 2 * f + 1);
+    if (h < 1 || w < 1 || y0 < 0 || x0 < 0 || y0 > h - S || x0 > w - S) return false;
+    const long long plane = static_cast<long long>(h) * w;
+    if (off < 0 || off > frames_bytes - C * plane) return false;
+    out->base = frames + off + static_cast<long long>(y0) * w + x0;
+    out->plane = plane;
+    out->w = w;
+    return true;
+}
+
+__device__ __forceinline__ uint32_t load4_unaligned(const uint8_t* p) {
+    // bytes p[0..3] as a little-endian word, from the aligned words that hold them
+    const uintptr_t a = reinterpret_cast<uintptr_t>(p);
+    const uint32_t* w = reinterpret_cast<const uint32_t*>(a & ~static_cast<uintptr_t>(3));
+    const uint32_t sh = static_cast<uint32_t>(a & 3) * 8;
+    const uint32_t lo = __ldg(w);
+    if (sh == 0) return lo;
+    return __funnelshift_r(lo, __ldg(w + 1), sh);
+}
+
+__global__ void __launch_bounds__(GC_THREADS)
+gather_crops_u8_kernel(const uint8_t* __restrict__ frames, long long frames_bytes, const long long* __restrict__ offsets,
+                       const int* __restrict__ sizes, long long n_frames, int C, const int* __restrict__ rows,
+                       int S, long long units, float* __restrict__ out0, float* __restrict__ out1,
+                       float* __restrict__ out2) {
+    const float nan = __int_as_float(0x7fc00000);
+    const int q = S / 4;                       // 4-pixel units per output row
+    for (long long u = static_cast<long long>(blockIdx.x) * GC_THREADS + threadIdx.x; u < units;
+         u += static_cast<long long>(gridDim.x) * GC_THREADS) {
+        const long long r = u / q;             // output row: ((b*3 + k)*C + c)*S + y
+        const int j = static_cast<int>(u - r * q);
+        const int y = static_cast<int>(r % S);
+        const long long bkc = r / S;
+        const int c = static_cast<int>(bkc % C);
+        const long long bk = bkc / C;
+        const long long b = bk / 3;
+        const int k = static_cast<int>(bk - 3 * b);
+        const int* row = rows + 6 * b;
+        const int y0 = __ldg(row + 3), x0 = __ldg(row + 4), mirror = __ldg(row + 5);
+        CropSrc s0, s1, s2;
+        const bool ok = crop_src(frames, frames_bytes, offsets, sizes, n_frames, C, S, __ldg(row), y0, x0, &s0) &&
+                        crop_src(frames, frames_bytes, offsets, sizes, n_frames, C, S, __ldg(row + 1), y0, x0, &s1) &&
+                        crop_src(frames, frames_bytes, offsets, sizes, n_frames, C, S, __ldg(row + 2), y0, x0, &s2);
+        float* out = (k == 0 ? out0 : k == 1 ? out1 : out2) + ((b * C + c) * S + y) * static_cast<long long>(S) + 4 * j;
+        float4 v = make_float4(nan, nan, nan, nan);
+        if (ok) {
+            const CropSrc& s = k == 0 ? s0 : k == 1 ? s1 : s2;
+            const uint8_t* src = s.base + c * s.plane + static_cast<long long>(y) * s.w;
+            uint32_t b4 = load4_unaligned(src + (mirror ? S - 4 - 4 * j : 4 * j));
+            if (mirror) b4 = __byte_perm(b4, 0, 0x0123);
+            v = make_float4(div255_u8(b4 & 0xff), div255_u8((b4 >> 8) & 0xff), div255_u8((b4 >> 16) & 0xff),
+                            div255_u8(b4 >> 24));
+        }
+        *reinterpret_cast<float4*>(out) = v;
+    }
+}
+
 int grid_for(size_t work_items, int threads) {
     size_t g = (work_items + threads - 1) / threads;
     const size_t cap = 148 * 16;  // grid-stride loops: a few waves of the 148 SMs is enough
@@ -624,6 +702,23 @@ const char* gather_triplets_u8_launch(const uint8_t* frames, int64_t n_frames, c
     const long long gy = rows < 65535 ? rows : 65535;
     gather_triplets_u8_kernel<<<dim3(static_cast<unsigned>(gx), static_cast<unsigned>(gy)), GT_THREADS, 0, stream>>>(
         frames, n_frames, triplets, n_triplets, reinterpret_cast<const long long*>(samples), rows, plane, vec, frame1,
+        frame2, target);
+    return last_launch_error();
+}
+
+const char* gather_crops_u8_launch(const uint8_t* frames, int64_t frames_bytes, const int64_t* offsets,
+                                   const int32_t* sizes, int64_t n_frames, int C, const int32_t* rows, int n, int S,
+                                   float* frame1, float* frame2, float* target, cudaStream_t stream) {
+    if (!frames || !offsets || !sizes || !rows || !frame1 || !frame2 || !target) return "gather_crops: null operand";
+    if (n < 1 || S < 4 || S % 4) return "gather_crops: needs n >= 1 and S a positive multiple of 4";
+    if (C != 1 && C != 3) return "gather_crops: C must be 1 or 3";
+    if (n_frames < 0 || frames_bytes < 0) return "gather_crops: negative frame count or size";
+    if ((reinterpret_cast<uintptr_t>(frame1) | reinterpret_cast<uintptr_t>(frame2) |
+         reinterpret_cast<uintptr_t>(target)) % 16)
+        return "gather_crops: outputs must be 16-byte aligned";
+    const long long units = 3LL * n * C * S * (S / 4);
+    gather_crops_u8_kernel<<<grid_for(static_cast<size_t>(units), GC_THREADS), GC_THREADS, 0, stream>>>(
+        frames, frames_bytes, reinterpret_cast<const long long*>(offsets), sizes, n_frames, C, rows, S, units, frame1,
         frame2, target);
     return last_launch_error();
 }

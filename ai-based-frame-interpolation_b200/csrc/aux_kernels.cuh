@@ -54,6 +54,11 @@ const char* pair_sad_launch(const uint8_t* frames, int64_t frame_stride, int64_t
 
 // Training batch from the device frame cache: frame1/frame2/target[b] = frames[triplets[samples[b]][0|1|2]] / 255 as
 // fp32 [n][H*W]; out-of-range samples or frame indices give NaN rows (fiGatherTripletsU8).
+// S x S windows (rows[b] = f1, f2, gt, y0, x0, mirror) of C-plane u8 frames of any size in one flat buffer ->
+// three fp32 [n][C][S][S]; bad indices or windows give NaN rows (fiGatherCropsU8).
+const char* gather_crops_u8_launch(const uint8_t* frames, int64_t frames_bytes, const int64_t* offsets,
+                                   const int32_t* sizes, int64_t n_frames, int C, const int32_t* rows, int n, int S,
+                                   float* frame1, float* frame2, float* target, cudaStream_t stream);
 const char* gather_triplets_u8_launch(const uint8_t* frames, int64_t n_frames, const int32_t* triplets,
                                       int64_t n_triplets, const int64_t* samples, int n, int H, int W, float* frame1,
                                       float* frame2, float* target, cudaStream_t stream);

@@ -1480,6 +1480,22 @@ int fiGatherTripletsU8(const uint8_t* frames, int64_t n_frames, const int32_t* t
     return FI_OK;
 }
 
+int fiGatherCropsU8(const uint8_t* frames, int64_t frames_bytes, const int64_t* offsets, const int32_t* sizes,
+                    int64_t n_frames, int C, const int32_t* rows, int n, int S, float* frame1, float* frame2,
+                    float* target, void* stream) {
+    if (!frames || !offsets || !sizes || !rows || !frame1 || !frame2 || !target)
+        return fail(FI_ERR_INVALID, "null argument");
+    if (n < 1 || S < 4 || S % 4) return fail(FI_ERR_INVALID, "needs n >= 1 and S a positive multiple of 4 (got %d, %d)", n, S);
+    if (C != 1 && C != 3) return fail(FI_ERR_INVALID, "C must be 1 or 3 (got %d)", C);
+    if (n_frames < 0 || frames_bytes < 0) return fail(FI_ERR_INVALID, "negative frame count or buffer size");
+    if ((reinterpret_cast<uintptr_t>(frame1) | reinterpret_cast<uintptr_t>(frame2) | reinterpret_cast<uintptr_t>(target)) % 16)
+        return fail(FI_ERR_INVALID, "outputs must be 16-byte aligned");
+    const char* e = fi::gather_crops_u8_launch(frames, frames_bytes, offsets, sizes, n_frames, C, rows, n, S, frame1,
+                                               frame2, target, static_cast<cudaStream_t>(stream));
+    if (e) return fail(FI_ERR_CUDA, "%s", e);
+    return FI_OK;
+}
+
 
 // ---------------------------------------------------------------------------------------------- training-step kernels
 #define TRAIN_CALL(expr)                                        \

@@ -17,6 +17,11 @@ def _scene_threshold(text):
         raise argparse.ArgumentTypeError(str(e)) from None
 
 
+def _crop_size(text):
+    from model.train import crop_size
+    return crop_size(text)
+
+
 def _frame_rate(text):
     from model.timing import parse_rate
     try:
@@ -36,8 +41,8 @@ class _TypedFactor(argparse.Action):
 def build_parser():
     p = argparse.ArgumentParser(description="AI-Based Frame Interpolation (B200-native path)")
     sub = p.add_subparsers(dest="command", help="Available commands")
-    # flags, defaults and required-ness as reference main.py:40-72; --frame-cache, --gpus, --scene-threshold and --fps
-    # are the only additions
+    # flags, defaults and required-ness as reference main.py:40-72; --frame-cache, --color, --crop, --gpus,
+    # --scene-threshold and --fps are the only additions
     t = sub.add_parser("train", help="Train the frame interpolation model")
     t.add_argument("--data-dir", required=True, help="Directory containing training data")
     t.add_argument("--epochs", type=int, default=100, help="Number of training epochs")
@@ -46,6 +51,11 @@ def build_parser():
     t.add_argument("--device", default="auto", help="Device to use (cuda/auto)")
     t.add_argument("--frame-cache", action="store_true",
                    help="Decode every frame once into GPU memory and build the batches there (default: off)")
+    t.add_argument("--color", action="store_true",
+                   help="Train the colour model UNet(6, 3) on BGR frames instead of the grey one (default: off)")
+    t.add_argument("--crop", type=_crop_size, default=None, metavar="S",
+                   help="Train on random S x S windows (S a multiple of 16) of frames at their native size, mirrored "
+                        "and with the input pair swapped at random, instead of resizing to 256x256 (default: off)")
     i = sub.add_parser("infer", help="Run inference on two frames")
     i.add_argument("--frame1", required=True, help="Path to first frame")
     i.add_argument("--frame2", required=True, help="Path to second frame")
@@ -98,6 +108,10 @@ def main(argv=None):
                 fwd += ["--batch-size", str(args.batch_size)]
             if args.frame_cache:
                 fwd.append("--frame-cache")
+            if args.color:
+                fwd.append("--color")
+            if args.crop is not None:
+                fwd += ["--crop", str(args.crop)]
             train_main(fwd)
             return 0
         if args.command == "infer":
@@ -143,13 +157,11 @@ def main(argv=None):
             print(f"Epoch: {meta.get('epoch', 'Unknown')}")
             print(f"Training Loss: {fmt(meta.get('train_loss', 'Unknown'))}")
             print(f"Validation Loss: {fmt(meta.get('val_loss', 'Unknown'))}")
-            from model.unet import FrameInterpolationUNet
-            state = meta.get("model_state_dict", checkpoint)
-            bilinear = not any(k.endswith("up1.up.weight") for k in state)
-            model = FrameInterpolationUNet(bilinear=bilinear)
+            from model.unet import architecture_name, model_from_state_dict
+            model, _ = model_from_state_dict(meta.get("model_state_dict", checkpoint))
             total = sum(p.numel() for p in model.parameters())
             trainable = sum(p.numel() for p in model.parameters() if p.requires_grad)
-            print(f"Architecture: FrameInterpolationUNet(bilinear={bilinear})")
+            print(f"Architecture: {architecture_name(model)}")
             print(f"Total Parameters: {total:,}")
             print(f"Trainable Parameters: {trainable:,}")
     except ImportError as e:

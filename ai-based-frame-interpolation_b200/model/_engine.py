@@ -86,6 +86,8 @@ _SIGNATURES = {
     "fiPairSadU8": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_void_p]),
     "fiGatherTripletsU8": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int, C.c_int,
                                      C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fiGatherCropsU8": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_int,
+                                  C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     # training-step kernels
     "fiBnStats": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "fiBnStatsShifted": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -420,6 +422,33 @@ def gather_triplets_u8(frames: torch.Tensor, triplets: torch.Tensor, samples: to
         check(lib().fiGatherTripletsU8(frames.data_ptr(), f, triplets.data_ptr(), triplets.shape[0], samples.data_ptr(),
                                        n, h, w, out[0].data_ptr(), out[1].data_ptr(), out[2].data_ptr(),
                                        current_stream()))
+    return out[0], out[1], out[2]
+
+
+def gather_crops_u8(frames: torch.Tensor, offsets: torch.Tensor, sizes: torch.Tensor, channels: int,
+                    rows: torch.Tensor, size: int):
+    """frames: uint8 CUDA [B] flat buffer of planar [C,H,W] frames; offsets: int64 CUDA [F] byte offset of each frame;
+    sizes: int32 CUDA [F,2] (H, W) of each; rows: int32 CUDA [n,6] (f1, f2, gt, y0, x0, mirror). Returns three fresh fp32
+    tensors [n,C,size,size] (frame1, frame2, target) = the windows / 255, mirrored left-right where asked, written by one
+    fiGatherCropsU8 launch on the current stream (no host synchronisation). A row naming a frame out of range, or a
+    window outside its frame, comes back as NaN."""
+    require_cuda(frames.device)
+    if frames.dtype != torch.uint8 or frames.dim() != 1 or not frames.is_contiguous():
+        raise FiError("frames must be a contiguous flat uint8 tensor")
+    if offsets.dtype != torch.int64 or offsets.dim() != 1 or not offsets.is_contiguous():
+        raise FiError("offsets must be a contiguous int64 tensor [F]")
+    if (sizes.dtype != torch.int32 or sizes.shape != (offsets.shape[0], 2) or not sizes.is_contiguous()):
+        raise FiError("sizes must be a contiguous int32 tensor [F,2]")
+    if rows.dtype != torch.int32 or rows.dim() != 2 or rows.shape[1] != 6 or not rows.is_contiguous() or rows.shape[0] < 1:
+        raise FiError("rows must be a non-empty contiguous int32 tensor [n,6]")
+    if not (offsets.device == sizes.device == rows.device == frames.device):
+        raise FiError("frames, offsets, sizes and rows must be on the same device")
+    n = rows.shape[0]
+    out = torch.empty((3, n, channels, size, size), dtype=torch.float32, device=frames.device)
+    with torch.cuda.device(frames.device):
+        check(lib().fiGatherCropsU8(frames.data_ptr(), frames.numel(), offsets.data_ptr(), sizes.data_ptr(),
+                                    offsets.shape[0], channels, rows.data_ptr(), n, size, out[0].data_ptr(),
+                                    out[1].data_ptr(), out[2].data_ptr(), current_stream()))
     return out[0], out[1], out[2]
 
 

@@ -20,13 +20,13 @@ try:
     from .multigpu import GpuPool
     from .scene import check_threshold, scene_cuts, scene_scores
     from .timing import MAX_DEPTH, depth_for, output_window, parse_rate, position, snap, video_rate
-    from .unet import FrameInterpolationUNet, UNet
+    from .unet import FrameInterpolationUNet, model_from_state_dict
 except ImportError:  # `python model/inference.py` / model/ on sys.path, like the reference's scripts
     import _engine as _E
     from multigpu import GpuPool
     from scene import check_threshold, scene_cuts, scene_scores
     from timing import MAX_DEPTH, depth_for, output_window, parse_rate, position, snap, video_rate
-    from unet import FrameInterpolationUNet, UNet
+    from unet import FrameInterpolationUNet, model_from_state_dict
 
 
 # ------------------------------------------------------------------------------------------- pre / post processing
@@ -165,19 +165,10 @@ class FrameInterpolator:
         self.last_scene_cuts = None
         self.device = _resolve_device(device)
         state, _ = _read_checkpoint(model_path, self.device)
-        keys = list(state.keys())
-        prefix = "unet." if any(k.startswith("unet.") for k in keys) else ""
-        bilinear = (prefix + "up1.up.weight") not in state
-        n_channels = state[prefix + "inc.double_conv.0.weight"].shape[1]
-        n_classes = state[prefix + "outc.conv.weight"].shape[0]
-        if prefix and (n_channels, n_classes) == (2, 1):
-            self.model = FrameInterpolationUNet(bilinear=bilinear)
-        else:
-            self.model = UNet(n_channels, n_classes, bilinear)
-            state = {k[len(prefix):]: v for k, v in state.items()} if prefix else state
+        self.model, state = model_from_state_dict(state)
         self.model.load_state_dict(state)
         self.model = self.model.to(self.device).eval()
-        self.n_channels, self.n_classes, self.bilinear = n_channels, n_classes, bilinear
+        self.n_channels, self.n_classes, self.bilinear = self.model._engine_spec()
         self.pairs_per_batch = max(1, int(pairs_per_batch))
         if gpus is None:
             gpus = int(os.environ.get("FI_GPUS", "1"))

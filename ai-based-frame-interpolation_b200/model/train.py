@@ -25,6 +25,7 @@ keys, ReduceLROnPlateau(factor 0.5, patience 10) schedule) and main().
 from __future__ import annotations
 
 import argparse
+import copy
 import ctypes as C
 import math
 import os
@@ -36,9 +37,11 @@ import torch.nn.functional as F
 
 try:
     from . import _engine as E
+    from . import crops
     from .unet import FrameInterpolationUNet, UNet
 except ImportError:  # model/ on sys.path, like the reference's scripts
     import _engine as E
+    import crops
     from unet import FrameInterpolationUNet, UNet
 
 BN_MOMENTUM = 0.1
@@ -542,12 +545,19 @@ class CombinedLoss(nn.Module):
 
 class FrameTripletDataset(torch.utils.data.Dataset):
     """(frame_t0, frame_t1, ground_truth_mid) from <data_dir>/<video>/<sorted frames>: frames i and i+2 are the inputs,
-    i+1 the target; grayscale, resized to 256x256, [0,1] fp32 [1,H,W] (reference model/train.py:89-151)."""
+    i+1 the target; grayscale, resized to 256x256, [0,1] fp32 [1,H,W] (reference model/train.py:89-151).
+
+    color=True: BGR frames as planes [3,H,W] in cv2's B, G, R order (what FrameInterpolator feeds a colour model),
+    for UNet(6, 3). crop=S: S x S windows of the frames at their native size instead of the resize; training samples
+    take the random window, left-right mirror and frame1/frame2 swap of model/crops.py for (seed, epoch, triplet),
+    the copy returned by `for_validation()` the centre window without either. `set_epoch(e)` selects the draws."""
 
     EXTENSIONS = (".jpg", ".png", ".bmp")
 
-    def __init__(self, data_dir, sequence_length=3):
+    def __init__(self, data_dir, sequence_length=3, color=False, crop=None, seed=0):
         self.data_dir, self.sequence_length = data_dir, sequence_length
+        self.color, self.crop = bool(color), None if crop is None else crops.check_size(crop)
+        self.seed, self.epoch, self.augment = int(seed), 0, True
         self.triplets = []
         for video in os.listdir(data_dir):
             path = os.path.join(data_dir, video)
@@ -561,16 +571,55 @@ class FrameTripletDataset(torch.utils.data.Dataset):
     def __len__(self):
         return len(self.triplets)
 
+    def set_epoch(self, epoch):
+        """The epoch of the crop draws (train_model calls it at the start of every epoch)."""
+        self.epoch = int(epoch)
+
+    def for_validation(self):
+        """The same triplets with centre windows and no mirror or swap (a shallow copy; only matters with crop)."""
+        v = copy.copy(self)
+        v.augment = False
+        return v
+
     def __getitem__(self, idx):
         import cv2
         import numpy as np
         t = self.triplets[idx]
-        out = []
+        if not self.color and self.crop is None:
+            out = []
+            for key in ("frame_t0", "frame_t1", "ground_truth"):
+                img = cv2.imread(os.path.join(t["video_dir"], t[key]), cv2.IMREAD_GRAYSCALE)
+                img = cv2.resize(img, (256, 256)).astype(np.float32) / 255.0
+                out.append(torch.from_numpy(img).unsqueeze(0))
+            return tuple(out)
+        planes = []
         for key in ("frame_t0", "frame_t1", "ground_truth"):
-            img = cv2.imread(os.path.join(t["video_dir"], t[key]), cv2.IMREAD_GRAYSCALE)
-            img = cv2.resize(img, (256, 256)).astype(np.float32) / 255.0
-            out.append(torch.from_numpy(img).unsqueeze(0))
-        return tuple(out)
+            path = os.path.join(t["video_dir"], t[key])
+            img = cv2.imread(path, cv2.IMREAD_COLOR if self.color else cv2.IMREAD_GRAYSCALE)
+            if img is None:
+                raise ValueError(f"cannot read frame {path!r}")
+            if self.crop is None:
+                img = cv2.resize(img, (256, 256))
+            elif img.shape[0] < self.crop or img.shape[1] < self.crop:
+                raise ValueError(f"frame {path!r} is {img.shape[1]}x{img.shape[0]}, smaller than the "
+                                 f"{self.crop}x{self.crop} crop")
+            planes.append((path, img.transpose(2, 0, 1) if self.color else img[None]))
+        if self.crop is not None:
+            s = self.crop
+            for path, p in planes[1:]:
+                if p.shape != planes[0][1].shape:
+                    raise ValueError(f"frame {path!r} differs in size from {planes[0][0]!r} of the same triplet")
+            h, w = planes[0][1].shape[1:]
+            if self.augment:
+                y0, x0, mirror, swap = (v[0] for v in crops.draw(self.seed, self.epoch, [idx], h, w, s))
+            else:
+                (y0, x0), mirror, swap = crops.centre(h, w, s), False, False
+            y0, x0 = int(y0), int(x0)
+            planes = [(path, p[:, y0:y0 + s, x0:x0 + s][:, :, ::-1] if mirror else p[:, y0:y0 + s, x0:x0 + s])
+                      for path, p in planes]
+            if swap:                     # the midpoint of (t1, t0) is the same target
+                planes[0], planes[1] = planes[1], planes[0]
+        return tuple(torch.from_numpy(p.astype(np.float32) / 255.0) for _, p in planes)
 
 
 class _PlateauSchedule:
@@ -622,6 +671,11 @@ def train_model(model, train_loader, val_loader, num_epochs=100, device="cuda", 
         sampler = getattr(train_loader, "sampler", None)
         if hasattr(sampler, "set_epoch"):
             sampler.set_epoch(epoch)
+        data = getattr(train_loader, "dataset", None)
+        while isinstance(data, torch.utils.data.Subset):
+            data = data.dataset
+        if hasattr(data, "set_epoch"):    # the crop draws of FrameTripletDataset (DataLoader and frame cache alike)
+            data.set_epoch(epoch)
         model.train()
         total = torch.zeros((), dtype=torch.float32, device=device)   # summed on the device: no sync per step
         for f0, f1, gt in train_loader:
@@ -633,8 +687,9 @@ def train_model(model, train_loader, val_loader, num_epochs=100, device="cuda", 
         total = torch.zeros(1, dtype=torch.float32, device=device)
         with torch.no_grad():
             for f0, f1, gt in val_loader:
-                total += step.loss_value(model(f0.to(device, non_blocking=True), f1.to(device, non_blocking=True)),
-                                         gt.to(device, non_blocking=True))
+                f0, f1 = f0.to(device, non_blocking=True), f1.to(device, non_blocking=True)
+                y = model(torch.cat([f0, f1], 1)) if isinstance(model, UNet) else model(f0, f1)   # UNet takes one tensor
+                total += step.loss_value(y, gt.to(device, non_blocking=True))
         val_losses.append(mean_over_ranks(total.item(), len(val_loader)))
         sched.step(val_losses[-1])
         say(f"Epoch {epoch + 1}/{num_epochs}:\n  Train Loss: {train_losses[-1]:.6f}\n  Val Loss: {val_losses[-1]:.6f}\n"
@@ -652,9 +707,18 @@ def train_model(model, train_loader, val_loader, num_epochs=100, device="cuda", 
     return train_losses, val_losses
 
 
+def crop_size(text):
+    """argparse type of --crop: a multiple of 16, at least 16."""
+    try:
+        return crops.check_size(int(text))
+    except ValueError:
+        raise argparse.ArgumentTypeError(f"crop size must be a multiple of 16 and at least 16, got {text!r}") from None
+
+
 def main(argv=None):
     """python model/train.py --data-dir D [--epochs 100 --batch-size 8 --device auto --val-split 0.2]
-    (reference model/train.py:251-313). Data parallel over the GPUs of a box:
+    (reference model/train.py:251-313); --frame-cache, --color and --crop S are opt-in additions (see
+    FrameTripletDataset and model/framecache.py). Data parallel over the GPUs of a box:
 
         torchrun --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 model/train.py --data-dir D ...
 
@@ -670,6 +734,11 @@ def main(argv=None):
     ap.add_argument("--frame-cache", action="store_true",
                     help="decode every frame once into GPU memory (64 KB a frame) and build batches there instead of "
                          "decoding three files per sample in DataLoader workers")
+    ap.add_argument("--color", action="store_true",
+                    help="train UNet(6, 3) on BGR frames, the colour model FrameInterpolator runs once per frame pair")
+    ap.add_argument("--crop", type=crop_size, default=None, metavar="S",
+                    help="train on random S x S windows of frames at their native size (S a multiple of 16), mirrored "
+                         "and with the input pair swapped at random, instead of resizing every frame to 256x256")
     args = ap.parse_args(argv)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if world > 1:
@@ -681,10 +750,12 @@ def main(argv=None):
         device = torch.device("cuda" if args.device == "auto" else args.device)
     E.require_cuda(device)
     rank0 = world == 1 or dist.get_rank() == 0
-    data = FrameTripletDataset(args.data_dir)
+    data = FrameTripletDataset(args.data_dir, color=args.color, crop=args.crop)
     n_val = int(len(data) * args.val_split)
     split_gen = torch.Generator().manual_seed(0) if world > 1 else None     # every rank must draw the same split
     train_set, val_set = torch.utils.data.random_split(data, [len(data) - n_val, n_val], generator=split_gen)
+    if args.crop is not None:      # validation: centre windows, no mirror or swap
+        val_set = torch.utils.data.Subset(data.for_validation(), val_set.indices)
     if rank0:
         print(f"Dataset split: {len(train_set)} train, {len(val_set)} validation")
     cache = None
@@ -706,7 +777,7 @@ def main(argv=None):
         return torch.utils.data.DataLoader(d, batch_size=args.batch_size, shuffle=shuffle and sampler is None,
                                            sampler=sampler, num_workers=4, pin_memory=True)
 
-    model = FrameInterpolationUNet(bilinear=True).to(device)
+    model = (UNet(6, 3, bilinear=True) if args.color else FrameInterpolationUNet(bilinear=True)).to(device)
     if rank0:
         print(f"Model parameters: {sum(p.numel() for p in model.parameters()):,} total")
     try:

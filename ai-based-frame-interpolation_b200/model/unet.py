@@ -309,6 +309,28 @@ class FrameInterpolationUNet(_EngineBacked):
         return out
 
 
+def model_from_state_dict(state):
+    """The architecture a checkpoint's state dict was saved from, read off its keys and shapes: bilinear vs
+    ConvTranspose2d decoder, input channels (2 grey, 6 colour) and classes. Returns (model, state) with a fresh module
+    of that architecture, FrameInterpolationUNet for a wrapped 2->1 model, else UNet, and the state dict keyed for it
+    (the `unet.` prefix of a wrapped colour model stripped); the weights are not loaded."""
+    prefix = "unet." if any(k.startswith("unet.") for k in state) else ""
+    bilinear = (prefix + "up1.up.weight") not in state
+    n_channels = state[prefix + "inc.double_conv.0.weight"].shape[1]
+    n_classes = state[prefix + "outc.conv.weight"].shape[0]
+    if prefix and (n_channels, n_classes) == (2, 1):
+        return FrameInterpolationUNet(bilinear=bilinear), state
+    state = {k[len(prefix):]: v for k, v in state.items()} if prefix else state
+    return UNet(n_channels, n_classes, bilinear), state
+
+
+def architecture_name(model):
+    """How `main.py info` names a model: FrameInterpolationUNet(bilinear=...) or UNet(n_channels, n_classes, ...)."""
+    if isinstance(model, FrameInterpolationUNet):
+        return f"FrameInterpolationUNet(bilinear={model.unet.bilinear})"
+    return f"UNet(n_channels={model.n_channels}, n_classes={model.n_classes}, bilinear={model.bilinear})"
+
+
 def count_parameters(model):
     """Number of trainable parameters — reference model/unet.py:114-116."""
     return sum(p.numel() for p in model.parameters() if p.requires_grad)

@@ -231,6 +231,18 @@ int fiPairSadU8(const uint8_t* frames, int64_t frame_stride, int64_t frame_bytes
 int fiGatherTripletsU8(const uint8_t* frames, int64_t n_frames, const int32_t* triplets, int64_t n_triplets,
                        const int64_t* samples, int n, int H, int W, float* frame1, float* frame2, float* target,
                        void* stream);
+/* FrameTripletDataset(crop=S).__getitem__ + the DataLoader collate (model/train.py:89-151) for frames of any size
+ * already on the device (model/framecache.py, --crop): frames is one flat u8 buffer of frames_bytes bytes holding frame
+ * f as planar [C][H_f][W_f] at byte offsets[f] (int64), sizes int32 [n_frames][2] = (H_f, W_f), C 1 (grey) or 3 (BGR).
+ * rows int32 [n][6] = (f1, f2, gt, y0, x0, mirror): frame1[b][c][y][x] = frame f1 at (c, y0 + y, x0 + x'), x' = S-1-x
+ * when mirror != 0 else x, and likewise frame2 from f2 and target from gt, each fp32 [n][C][S][S] and bit-identical to
+ * crop.astype(float32) / 255.0. The random draw (model/crops.py, including the swap of f1 and f2) is made on the host.
+ * A row naming a frame outside [0, n_frames), or a window or frame outside its bounds, is never dereferenced: its three
+ * outputs are NaN. FI_ERR_INVALID on NULL pointers, n < 1, S not a positive multiple of 4, C not 1 or 3, negative
+ * counts, or outputs not 16-byte aligned. No host synchronisation. */
+int fiGatherCropsU8(const uint8_t* frames, int64_t frames_bytes, const int64_t* offsets, const int32_t* sizes,
+                    int64_t n_frames, int C, const int32_t* rows, int n, int S, float* frame1, float* frame2,
+                    float* target, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------
  * Training step (model/train.py:153-249; SURVEY.md §8f row 2): the kernels around the tensor-core convolutions.
