@@ -214,34 +214,60 @@ head_post_kernel(const float* __restrict__ y, uint8_t* __restrict__ out, size_t 
 // ------------------------------------------------------------------------------------------------ SSIM + PSNR
 // compute_ssim / compute_psnr of the reference (model/evaluation.py:194-218) call scikit-image with data_range=255:
 // 7x7 uniform window, sample covariance (x49/48), K1=.01, K2=.03, mean over the image cropped by 3; PSNR from the MSE.
+// Colour images are scored as structural_similarity(..., channel_axis=-1): the mean over channels of each channel's
+// grey SSIM (each with its own 3-pixel crop), and PSNR over all C*H*W samples.
 // All 49-pixel window sums of u8 data are exact in int32, so the per-pixel ratio is formed from exact integers:
 //   S = (2 Sx Sy + C1 49^2)(2(49 Sxy - Sx Sy) + C2 48 49) / ((Sx^2 + Sy^2 + C1 49^2)(49 Sqq - Sx^2 - Sy^2 + C2 48 49))
 // with Sx = sum x, Sy = sum y, Sqq = sum (x^2 + y^2), Sxy = sum x y over the window.
-// Thread = 4 adjacent columns, sliding down SS_ROWS rows: horizontal window sums slide along x, vertical along y.
+// Block = one channel of one image (blockIdx.z = n*C + c) x SS_COLS columns x SS_ROWS rows. Thread = 4 adjacent
+// columns, sliding down SS_ROWS rows: horizontal window sums slide along x, vertical along y.
 constexpr int SS_THREADS = 128;
 constexpr int SS_COLS = 4 * SS_THREADS;  // columns per block
 constexpr int SS_ROWS = 36;              // owned rows per block (+6 halo rows streamed)
 
-__device__ __forceinline__ uint32_t load_word_guarded(const uint8_t* rowp, int c0, int W, bool aligned) {
-    if (c0 >= 0 && c0 + 3 < W && aligned) return __ldg(reinterpret_cast<const uint32_t*>(rowp + c0));
+// Pixels c0 .. c0+3 of one channel of a row, packed little-endian into a word (0 outside [0, W)). PS is the pixel
+// stride: 1 = planar (one word load when aligned), 3 = interleaved BGR, where rowp points at pixel 0 of channel 0 and
+// the 12 bytes of pixels c0 .. c0+3 are three aligned words; __byte_perm picks channel `ch`'s bytes 3k + ch out of
+// them (sel1 from words 0-1, sel2 adds word 2), so the window arithmetic below sees the same word either way.
+template <int PS>
+__device__ __forceinline__ uint32_t load_word_guarded(const uint8_t* rowp, int c0, int W, bool aligned, int ch,
+                                                      uint32_t sel1, uint32_t sel2) {
+    if (c0 >= 0 && c0 + 3 < W && aligned) {
+        if (PS == 1) return __ldg(reinterpret_cast<const uint32_t*>(rowp + c0));
+        const uint32_t* p = reinterpret_cast<const uint32_t*>(rowp + 3 * c0);
+        return __byte_perm(__byte_perm(__ldg(p), __ldg(p + 1), sel1), __ldg(p + 2), sel2);
+    }
     uint32_t v = 0;
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
         const int c = c0 + k;
-        if (c >= 0 && c < W) v |= static_cast<uint32_t>(__ldg(rowp + c)) << (8 * k);
+        if (c >= 0 && c < W) v |= static_cast<uint32_t>(__ldg(rowp + PS * c + (PS == 1 ? 0 : ch))) << (8 * k);
     }
     return v;
 }
 
+// One operand: channel plane (n, c) starts at ptr + n*batch + c*chan, rows are `row` bytes apart. Interleaved
+// operands (PS = 3) keep chan = 1 and are addressed from channel 0 (the loader adds the channel).
+struct SsimOperand {
+    const uint8_t* ptr;
+    long long batch, chan, row;
+    int aligned;  // every word the loader reads is 4-byte aligned
+};
+
+template <int PA, int PB>
 __global__ void __launch_bounds__(SS_THREADS, 4)
-ssim_psnr_kernel(const uint8_t* __restrict__ a, const uint8_t* __restrict__ b, int H, int W, int aligned,
-                 double* __restrict__ part_ssim, unsigned long long* __restrict__ part_ssd) {
+ssim_psnr_kernel(SsimOperand a, SsimOperand b, int C, int H, int W, double* __restrict__ part_ssim,
+                 unsigned long long* __restrict__ part_ssd) {
     const int tid = threadIdx.x;
-    const int n = blockIdx.z;
+    const int n = blockIdx.z / C, ch = blockIdx.z - n * C;
     const int xb = blockIdx.x * SS_COLS + 4 * tid;  // first owned column
     const int ty0 = blockIdx.y * SS_ROWS;
-    const uint8_t* ia = a + static_cast<size_t>(n) * H * W;
-    const uint8_t* ib = b + static_cast<size_t>(n) * H * W;
+    const uint8_t* ia = a.ptr + n * a.batch + (PA == 1 ? ch * a.chan : 0);
+    const uint8_t* ib = b.ptr + n * b.batch + (PB == 1 ? ch * b.chan : 0);
+    // __byte_perm selectors of channel ch in an interleaved span: bytes ch, ch+3 from words 0-1 (+ ch+6 when < 8),
+    // then the rest from word 2
+    const uint32_t sel1 = ch | (ch + 3) << 4 | (ch + 6 < 8 ? (ch + 6) << 8 : 0u);
+    const uint32_t sel2 = 0x10u | (ch + 6 < 8 ? 2u : static_cast<uint32_t>(ch + 2)) << 8 | static_cast<uint32_t>(ch + 5) << 12;
 
     uint32_t ring1[7][4], ringq[7][4], ringp[7][4];
     uint32_t v1[4] = {0, 0, 0, 0}, vq[4] = {0, 0, 0, 0}, vp[4] = {0, 0, 0, 0};
@@ -256,19 +282,24 @@ ssim_psnr_kernel(const uint8_t* __restrict__ a, const uint8_t* __restrict__ b, i
     const float K2 = 58.5225f * 2352.0f;  // C2 * 48 * 49
 
     // The six words of row i+1 are requested before row i is reduced, so their latency overlaps the arithmetic.
+    // Rows are fetched in order, so the two row pointers advance by their strides (32-bit: a row is < 2 GB).
     uint32_t na[3], nb[3];
+    const int row_a = static_cast<int>(a.row), row_b = static_cast<int>(b.row);
+    const bool aligned = a.aligned && b.aligned;
+    ia += static_cast<long long>(ty0 - 3) * a.row;
+    ib += static_cast<long long>(ty0 - 3) * b.row;
     auto fetch_row = [&](int yin) {
 #pragma unroll
         for (int k = 0; k < 3; ++k) na[k] = nb[k] = 0;
         if (yin >= 0 && yin < H && xb - 4 < W) {
-            const uint8_t* ra = ia + static_cast<size_t>(yin) * W;
-            const uint8_t* rbp = ib + static_cast<size_t>(yin) * W;
 #pragma unroll
             for (int k = 0; k < 3; ++k) {
-                na[k] = load_word_guarded(ra, xb - 4 + 4 * k, W, aligned);
-                nb[k] = load_word_guarded(rbp, xb - 4 + 4 * k, W, aligned);
+                na[k] = load_word_guarded<PA>(ia, xb - 4 + 4 * k, W, aligned, ch, sel1, sel2);
+                nb[k] = load_word_guarded<PB>(ib, xb - 4 + 4 * k, W, aligned, ch, sel1, sel2);
             }
         }
+        ia += row_a;
+        ib += row_b;
     };
     fetch_row(ty0 - 3);
     for (int rb = 0; rb < SS_ROWS + 6; rb += 7) {
@@ -352,39 +383,49 @@ ssim_psnr_kernel(const uint8_t* __restrict__ a, const uint8_t* __restrict__ b, i
             ts += sh_s[k];
             tu += sh_u[k];
         }
-        const size_t slot = (static_cast<size_t>(n) * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x;
+        const size_t slot = (static_cast<size_t>(blockIdx.z) * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x;
         part_ssim[slot] = ts;
         part_ssd[slot] = tu;
     }
 }
 
+// One block per image: each channel's partials are summed in a fixed order (so C = 1 is the grey result bit for bit),
+// the channel SSIMs are averaged in channel order and the squared errors of all channels are summed in 64 bit.
 __global__ void __launch_bounds__(256)
 ssim_psnr_finalize_kernel(const double* __restrict__ part_ssim, const unsigned long long* __restrict__ part_ssd,
-                          int nblk, int H, int W, double* __restrict__ out) {
+                          int nblk, int C, int H, int W, double* __restrict__ out) {
     const int n = blockIdx.x;
     __shared__ double sh_s[256];
     __shared__ unsigned long long sh_u[256];
-    double s = 0.0;
-    unsigned long long u = 0;
-    for (int i = threadIdx.x; i < nblk; i += 256) {
-        s += part_ssim[static_cast<size_t>(n) * nblk + i];
-        u += part_ssd[static_cast<size_t>(n) * nblk + i];
-    }
-    sh_s[threadIdx.x] = s;
-    sh_u[threadIdx.x] = u;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) {
-            sh_s[threadIdx.x] += sh_s[threadIdx.x + o];
-            sh_u[threadIdx.x] += sh_u[threadIdx.x + o];
+    double ssim_sum = 0.0;
+    unsigned long long sse = 0;
+    for (int ch = 0; ch < C; ++ch) {
+        const size_t base = (static_cast<size_t>(n) * C + ch) * nblk;
+        double s = 0.0;
+        unsigned long long u = 0;
+        for (int i = threadIdx.x; i < nblk; i += 256) {
+            s += part_ssim[base + i];
+            u += part_ssd[base + i];
         }
+        sh_s[threadIdx.x] = s;
+        sh_u[threadIdx.x] = u;
         __syncthreads();
+        for (int o = 128; o > 0; o >>= 1) {
+            if (threadIdx.x < o) {
+                sh_s[threadIdx.x] += sh_s[threadIdx.x + o];
+                sh_u[threadIdx.x] += sh_u[threadIdx.x + o];
+            }
+            __syncthreads();
+        }
+        ssim_sum += sh_s[0] / (static_cast<double>(H - 6) * (W - 6));
+        sse += sh_u[0];
+        __syncthreads();  // sh_s / sh_u are rewritten by the next channel
     }
     if (threadIdx.x == 0) {
-        const double mse = static_cast<double>(sh_u[0]) / (static_cast<double>(H) * W);
+        const double mse = static_cast<double>(sse) / (static_cast<double>(H) * W * C);
         // skimage peak_signal_noise_ratio: 10*log10(data_range^2 / mse); identical images -> inf
-        out[2 * n + 0] = sh_u[0] == 0 ? __longlong_as_double(0x7ff0000000000000LL) : 10.0 * log10(65025.0 / mse);
-        out[2 * n + 1] = sh_s[0] / (static_cast<double>(H - 6) * (W - 6));
+        out[2 * n + 0] = sse == 0 ? __longlong_as_double(0x7ff0000000000000LL) : 10.0 * log10(65025.0 / mse);
+        out[2 * n + 1] = ssim_sum / C;
     }
 }
 
@@ -635,28 +676,55 @@ static void ssim_grid(int H, int W, int* gx, int* gy) {
     *gy = (H + SS_ROWS - 1) / SS_ROWS;
 }
 
-size_t ssim_psnr_workspace_bytes(int N, int H, int W) {
+size_t ssim_psnr_workspace_bytes(int N, int C, int H, int W) {
     int gx, gy;
     ssim_grid(H, W, &gx, &gy);
-    return static_cast<size_t>(N) * gx * gy * 16;
+    return static_cast<size_t>(N) * C * gx * gy * 16;
 }
 
-const char* ssim_psnr_launch(const uint8_t* a, const uint8_t* b, int N, int H, int W, double* out, void* workspace,
-                             cudaStream_t stream) {
-    if (N <= 0) return "ssim: empty batch";
-    if (H < 7 || W < 7) return "ssim: win_size 7 exceeds image extent (skimage raises ValueError here too)";
-    if (N > 65535) return "ssim: at most 65535 image pairs per call";
-    if (!a || !b || !out || !workspace) return "ssim: null operand";
+// Pixel stride of a supported layout (1 planar, 3 interleaved BGR), or 0.
+static int ssim_layout(const PlaneSrc& p) {
+    if (p.batch_stride < 0 || p.chan_stride < 0 || p.row_stride < 0 || p.row_stride > 0x7fffffff) return 0;
+    if (p.px_stride == 1) return 1;
+    if (p.px_stride == 3 && p.chan_stride == 1 && p.channels == 3) return 3;
+    return 0;
+}
+
+static SsimOperand ssim_operand(const PlaneSrc& p, int ps, int N) {
+    const uint8_t* ptr = static_cast<const uint8_t*>(p.ptr);
+    long long bits = static_cast<long long>(reinterpret_cast<uintptr_t>(ptr)) | p.row_stride;
+    if (N > 1) bits |= p.batch_stride;
+    if (ps == 1 && p.channels > 1) bits |= p.chan_stride;
+    return SsimOperand{ptr, p.batch_stride, p.chan_stride, p.row_stride, static_cast<int>(bits % 4 == 0)};
+}
+
+const char* ssim_psnr_launch(const PlaneSrc& pred, const PlaneSrc& target, int N, int H, int W, double* out,
+                             void* workspace, cudaStream_t stream) {
+    if (N <= 0) return "ssim: empty batch (N < 1)";
+    if (H < 7 || W < 7) return "ssim: win_size 7 exceeds image extent: H and W must be >= 7 (skimage raises ValueError here too)";
+    if (!pred.ptr || !target.ptr) return "ssim: null pred or target pointer";
+    if (!out || !workspace) return "ssim: null out or workspace";
+    if (pred.channels != target.channels) return "ssim: pred and target channel counts differ";
+    const int C = pred.channels;
+    if (C != 1 && C != 3) return "ssim: channels must be 1 or 3";
+    const int pa = ssim_layout(pred), pb = ssim_layout(target);
+    if (!pa) return "ssim: pred layout is neither planar (px_stride 1) nor interleaved (px_stride 3, chan_stride 1, 3 channels)";
+    if (!pb) return "ssim: target layout is neither planar (px_stride 1) nor interleaved (px_stride 3, chan_stride 1, 3 channels)";
+    if (static_cast<long long>(N) * C > 65535) return "ssim: too many planes: N * channels must be <= 65535";
     int gx, gy;
     ssim_grid(H, W, &gx, &gy);
     const int nblk = gx * gy;
     double* part_ssim = static_cast<double*>(workspace);
-    unsigned long long* part_ssd = reinterpret_cast<unsigned long long*>(part_ssim + static_cast<size_t>(N) * nblk);
-    const int aligned = (W % 4 == 0) && ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b)) % 4 == 0);
-    ssim_psnr_kernel<<<dim3(gx, gy, N), SS_THREADS, 0, stream>>>(a, b, H, W, aligned, part_ssim, part_ssd);
+    unsigned long long* part_ssd = reinterpret_cast<unsigned long long*>(part_ssim + static_cast<size_t>(N) * C * nblk);
+    const SsimOperand a = ssim_operand(pred, pa, N), b = ssim_operand(target, pb, N);
+    const dim3 grid(gx, gy, N * C);
+    if (pa == 1 && pb == 1) ssim_psnr_kernel<1, 1><<<grid, SS_THREADS, 0, stream>>>(a, b, C, H, W, part_ssim, part_ssd);
+    if (pa == 1 && pb == 3) ssim_psnr_kernel<1, 3><<<grid, SS_THREADS, 0, stream>>>(a, b, C, H, W, part_ssim, part_ssd);
+    if (pa == 3 && pb == 1) ssim_psnr_kernel<3, 1><<<grid, SS_THREADS, 0, stream>>>(a, b, C, H, W, part_ssim, part_ssd);
+    if (pa == 3 && pb == 3) ssim_psnr_kernel<3, 3><<<grid, SS_THREADS, 0, stream>>>(a, b, C, H, W, part_ssim, part_ssd);
     const char* e = last_launch_error();
     if (e) return e;
-    ssim_psnr_finalize_kernel<<<N, 256, 0, stream>>>(part_ssim, part_ssd, nblk, H, W, out);
+    ssim_psnr_finalize_kernel<<<N, 256, 0, stream>>>(part_ssim, part_ssd, nblk, C, H, W, out);
     return last_launch_error();
 }
 

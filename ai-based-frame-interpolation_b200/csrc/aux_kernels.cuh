@@ -42,9 +42,11 @@ const char* pack_pair_launch(const uint8_t* f0, const uint8_t* f1, float* out, i
 // postprocess_image (reference inference.py:54-61) on n fp32 values.
 const char* head_post_launch(const float* y, uint8_t* out, size_t n, cudaStream_t stream);
 
-// skimage-equivalent SSIM (7x7 uniform window, sample covariance, data_range 255) and PSNR of N u8 image pairs.
-size_t ssim_psnr_workspace_bytes(int N, int H, int W);
-const char* ssim_psnr_launch(const uint8_t* a, const uint8_t* b, int N, int H, int W, double* out /*[N][2]*/,
+// skimage-equivalent SSIM (7x7 uniform window, sample covariance, data_range 255, channel_axis=-1: mean of the channel
+// SSIMs) and PSNR (over all C*H*W samples) of N u8 image pairs of C = 1 or 3 channels. Each operand is planar
+// (px_stride 1) or interleaved BGR (px_stride 3, chan_stride 1); N*C <= 65535. Returns a message naming the bad argument.
+size_t ssim_psnr_workspace_bytes(int N, int C, int H, int W);
+const char* ssim_psnr_launch(const PlaneSrc& pred, const PlaneSrc& target, int N, int H, int W, double* out /*[N][2]*/,
                              void* workspace, cudaStream_t stream);
 
 // Scene-cut statistic: sad[p] = sum |f[p+1] - f[p]| over the frame_bytes bytes of each of the n_frames-1 consecutive

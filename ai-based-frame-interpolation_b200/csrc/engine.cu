@@ -1446,14 +1446,25 @@ int fiHeadPostU8(const float* logits, uint8_t* out, size_t n, void* stream) {
     return FI_OK;
 }
 
-size_t fiSsimPsnrWorkspaceBytes(int N, int H, int W) {
-    if (N <= 0 || H <= 0 || W <= 0) return 0;
-    return fi::ssim_psnr_workspace_bytes(N, H, W);
+size_t fiSsimPsnrWorkspaceBytes(int N, int H, int W) { return fiSsimPsnrPlanesWorkspaceBytes(N, 1, H, W); }
+
+size_t fiSsimPsnrPlanesWorkspaceBytes(int N, int C, int H, int W) {
+    if (N <= 0 || C <= 0 || H <= 0 || W <= 0) return 0;
+    return fi::ssim_psnr_workspace_bytes(N, C, H, W);
 }
 
 int fiSsimPsnrU8(const uint8_t* pred, const uint8_t* target, int N, int H, int W, double* out, void* workspace,
                  void* stream) {
-    const char* e = fi::ssim_psnr_launch(pred, target, N, H, W, out, workspace, static_cast<cudaStream_t>(stream));
+    const int64_t plane = static_cast<int64_t>(H) * W;
+    const fiPlanes p = {pred, plane, plane, W, 1, 1}, t = {target, plane, plane, W, 1, 1};
+    return fiSsimPsnrPlanesU8(&p, &t, N, H, W, out, workspace, stream);
+}
+
+int fiSsimPsnrPlanesU8(const fiPlanes* pred, const fiPlanes* target, int N, int H, int W, double* out, void* workspace,
+                       void* stream) {
+    if (!pred || !target) return fail(FI_ERR_INVALID, "ssim: null pred or target descriptor");
+    const char* e = fi::ssim_psnr_launch(to_src(pred), to_src(target), N, H, W, out, workspace,
+                                         static_cast<cudaStream_t>(stream));
     if (e) return fail(FI_ERR_INVALID, "%s", e);
     return FI_OK;
 }

@@ -83,6 +83,9 @@ _SIGNATURES = {
     "fiSsimPsnrWorkspaceBytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "fiSsimPsnrU8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                C.c_void_p]),
+    "fiSsimPsnrPlanesWorkspaceBytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int]),
+    "fiSsimPsnrPlanesU8": (C.c_int, [C.POINTER(Planes), C.POINTER(Planes), C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                     C.c_void_p, C.c_void_p]),
     "fiPairSadU8": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_void_p]),
     "fiGatherTripletsU8": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int, C.c_int,
                                      C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -382,6 +385,29 @@ def ssim_psnr_u8(pred: torch.Tensor, target: torch.Tensor) -> torch.Tensor:
     with torch.cuda.device(pred.device):
         check(lib().fiSsimPsnrU8(pred.data_ptr(), target.data_ptr(), n, h, w, out.data_ptr(), ws.data_ptr(),
                                  current_stream()))
+    return out
+
+
+def ssim_psnr_planes_u8(pred: torch.Tensor, target: torch.Tensor) -> torch.Tensor:
+    """pred/target: uint8 CUDA tensors [N,C,H,W], C = 1 or 3, read in place when planar (unit pixel stride, e.g. what
+    the forward writes) or interleaved (a channels-last [N,H,W,3] tensor's .permute(0, 3, 1, 2), e.g. cv2 BGR frames);
+    any other strides are copied to planar first. Returns a float64 CUDA tensor [N,2] = (PSNR, SSIM) with
+    scikit-image's channel_axis=-1 semantics (fiSsimPsnrPlanesU8)."""
+    require_cuda(pred.device)
+    if pred.dim() != 4 or pred.shape != target.shape or pred.dtype != torch.uint8 or target.dtype != torch.uint8:
+        raise FiError("pred and target must be uint8 tensors [N,C,H,W] of the same shape")
+
+    def layout(t):
+        s = t.stride()
+        return t if s[3] == 1 or (s[3] == 3 and s[1] == 1 and t.shape[1] == 3) else t.contiguous()
+    pred, target = layout(pred), layout(target.to(pred.device))
+    n, c, h, w = pred.shape
+    ws = torch.empty(max(16, lib().fiSsimPsnrPlanesWorkspaceBytes(n, c, h, w)), dtype=torch.uint8, device=pred.device)
+    out = torch.empty((n, 2), dtype=torch.float64, device=pred.device)
+    p, t = planes_of(pred), planes_of(target)
+    with torch.cuda.device(pred.device):
+        check(lib().fiSsimPsnrPlanesU8(C.byref(p), C.byref(t), n, h, w, out.data_ptr(), ws.data_ptr(),
+                                       current_stream()))
     return out
 
 

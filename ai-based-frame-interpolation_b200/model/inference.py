@@ -69,13 +69,7 @@ def load_model(model_path, device):
     model = FrameInterpolationUNet(bilinear=True)
     state, meta = _read_checkpoint(model_path, device)
     model.load_state_dict(state)
-    if meta is not None:
-        print(f"Model loaded from {model_path}")
-        print(f"Trained for {meta.get('epoch', 'Unknown')} epochs")
-        val = meta.get("val_loss", "Unknown")
-        print(f"Best validation loss: {val:.6f}" if isinstance(val, float) else f"Best validation loss: {val}")
-    else:
-        print(f"Model state dict loaded from {model_path}")
+    _print_checkpoint(model_path, meta)
     model = model.to(device)
     model.eval()
     return model
@@ -131,6 +125,52 @@ def save_frames_as_video(frames, output_path, fps=30):
         wr.release()
     print(f"Video saved successfully to {output_path}")
     print(f"Video contains {len(video_frames)} frames at {fps} FPS")
+
+
+def load_checkpoint_model(model_path, device):
+    """load_model for any architecture training makes: the network is built from the checkpoint's own keys and
+    shapes (model_from_state_dict: bilinear or ConvTranspose2d decoder, grey FrameInterpolationUNet or colour
+    UNet(6, 3)), loaded strictly, moved to `device`, eval mode; prints load_model's lines."""
+    state, meta = _read_checkpoint(model_path, device)
+    model, state = model_from_state_dict(state)
+    model.load_state_dict(state)
+    _print_checkpoint(model_path, meta)
+    return model.to(device).eval()
+
+
+def _print_checkpoint(model_path, meta):
+    if meta is not None:
+        print(f"Model loaded from {model_path}")
+        print(f"Trained for {meta.get('epoch', 'Unknown')} epochs")
+        val = meta.get("val_loss", "Unknown")
+        print(f"Best validation loss: {val:.6f}" if isinstance(val, float) else f"Best validation loss: {val}")
+    else:
+        print(f"Model state dict loaded from {model_path}")
+
+
+def check_model_frames(model, c):
+    """The model's input channels, or FiError when frames of c channels cannot reach it (forward_frames_u8's rules)."""
+    n_channels = model._engine_spec()[0]
+    if n_channels != 2 and n_channels != 2 * c:
+        raise _E.FiError(f"model expects {n_channels} input channels, frames have {c} per frame")
+    return n_channels
+
+
+def forward_frames_u8(model, a, b):
+    """The network's midpoint of frame pairs held on the device: a, b uint8 CUDA tensors [n,H,W] (grey) or [n,H,W,C]
+    (interleaved, e.g. BGR). Returns planar uint8 [n, C_out, H, W] on the device. The one place that maps frames to
+    the model: a grey model (2 input channels) runs once per plane of colour frames (a batch of n*C grey pairs read as
+    strided views, no copy); a colour model runs on the planar view of the pair; a model whose input does not match the
+    frames (a colour model on grey frames) raises before any work."""
+    n_channels = check_model_frames(model, 1 if a.dim() == 3 else a.shape[3])
+    if a.dim() == 3:
+        a, b = a[..., None], b[..., None]
+    n, h, w, c = a.shape
+    if n_channels == 2:  # grey model: every colour channel is its own pair
+        a4 = a.permute(0, 3, 1, 2).reshape(n * c, 1, h, w)  # strided views, no copy: the stem reads HWC directly
+        b4 = b.permute(0, 3, 1, 2).reshape(n * c, 1, h, w)
+        return model.forward_u8(a4, b4).view(n, c, h, w)
+    return model.forward_u8(a.permute(0, 3, 1, 2), b.permute(0, 3, 1, 2))
 
 
 # ------------------------------------------------------------------------------------------- FrameInterpolator
@@ -204,18 +244,7 @@ class FrameInterpolator:
         a = torch.from_numpy(np.ascontiguousarray(np.stack(firsts))).to(self.device, non_blocking=True)
         b = torch.from_numpy(np.ascontiguousarray(np.stack(seconds))).to(self.device, non_blocking=True)
         grey_in = a.dim() == 3
-        if grey_in:
-            a, b = a[..., None], b[..., None]
-        n, h, w, c = a.shape
-        if self.n_channels == 2:  # grey model: every colour channel is its own pair
-            a4 = a.permute(0, 3, 1, 2).reshape(n * c, 1, h, w)  # strided views, no copy: the stem reads HWC directly
-            b4 = b.permute(0, 3, 1, 2).reshape(n * c, 1, h, w)
-            out = self.model.forward_u8(a4, b4).view(n, c, h, w)
-        elif self.n_channels == 2 * c:
-            out = self.model.forward_u8(a.permute(0, 3, 1, 2), b.permute(0, 3, 1, 2))
-        else:
-            raise _E.FiError(f"model expects {self.n_channels} input channels, frames have {c} per frame")
-        out = out.permute(0, 2, 3, 1).contiguous().cpu().numpy()
+        out = forward_frames_u8(self.model, a, b).permute(0, 2, 3, 1).contiguous().cpu().numpy()
         return [o[..., 0] if grey_in and o.shape[-1] == 1 else o for o in out]
 
     def interpolate_frames(self, frame1, frame2):

@@ -211,10 +211,27 @@ int fiPackPairU8(const uint8_t* frame1, const uint8_t* frame2, float* out, int N
 /* postprocess_image (model/inference.py:43-63) on n fp32 values: trunc(clamp((t+1)/2,0,1)*255). */
 int fiHeadPostU8(const float* logits, uint8_t* out, size_t n, void* stream);
 /* compute_psnr / compute_ssim (model/evaluation.py:194-218 = evaluation_simple.py:103-109; scikit-image semantics,
- * data_range=255) for N u8 image pairs [N,H,W]: out[2n] = PSNR (dB, +inf when identical), out[2n+1] = SSIM. */
+ * data_range=255) for N u8 image pairs [N,H,W]: out[2n] = PSNR (dB, +inf when identical), out[2n+1] = SSIM.
+ * The C = 1 planar case of fiSsimPsnrPlanesU8 (same results, bit for bit). */
 size_t fiSsimPsnrWorkspaceBytes(int N, int H, int W);
 int fiSsimPsnrU8(const uint8_t* pred, const uint8_t* target, int N, int H, int W, double* out, void* workspace,
                  void* stream);
+/* The same metric for N image pairs of C = pred->channels = target->channels channels (1 or 3), each operand in its
+ * own layout, read in place:
+ *   planar      px_stride 1, any non-negative batch / chan / row strides (what fiNetForward writes, [N,C,H,W]);
+ *   interleaved px_stride 3, chan_stride 1, 3 channels (cv2's BGR HxWx3 frames, a channels-last tensor).
+ * For C = 3 this is scikit-image's structural_similarity(target, pred, channel_axis=-1, data_range=255): the mean over
+ * the channels of each channel's grey SSIM (its own 7x7 windows and 3-pixel crop), and
+ * peak_signal_noise_ratio(target, pred, data_range=255) over all C*H*W samples, 10*log10(255^2 / (SSE / (C*H*W))) with
+ * SSE exact in 64 bit (+inf when SSE = 0). All four layout combinations give the same bits. out[2n] = PSNR,
+ * out[2n+1] = SSIM. workspace: fiSsimPsnrPlanesWorkspaceBytes(N, C, H, W) bytes. Limits: H, W >= 7 (skimage raises
+ * there too) and N*C <= 65535 (one block column per plane in grid z). A null pointer, differing or unsupported channel
+ * counts, a layout outside the two above, H or W < 7 or too many planes return FI_ERR_INVALID naming it, before
+ * anything is launched or written; so does a row stride of 2^31 bytes or more. Stream-ordered; deterministic
+ * (fixed-order reduction, no atomics). */
+size_t fiSsimPsnrPlanesWorkspaceBytes(int N, int C, int H, int W);
+int fiSsimPsnrPlanesU8(const fiPlanes* pred, const fiPlanes* target, int N, int H, int W, double* out,
+                       void* workspace, void* stream);
 /* Scene-cut statistic (what ffmpeg's scdet and RIFE's video script compute on the host; the reference has none):
  * sad[i] = sum over k < frame_bytes of |frames[(i+1)*frame_stride + k] - frames[i*frame_stride + k]| for the n_frames-1
  * consecutive pairs of u8 frames, exact in 64 bit. sad is zeroed on `stream` first. Any alignment and stride work;
